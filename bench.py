@@ -16,6 +16,9 @@ One "step" = one whole-stream compression of the workload:
            block chain handed over through host memory, no NCCL / barrier / Python inside the step); the other ranks'
            processes idle on a host (gloo) barrier meanwhile.
 Prints ONE JSON line on rank 0.
+
+--dump-outputs DIR writes the .bz2 stream of the last timed step to DIR as .npy files (see dump_stream), so that two
+builds can be compared output for output: the inputs are seeded, identical from run to run.
 """
 import argparse
 import ctypes as C
@@ -30,9 +33,12 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark writes nothing into the source tree, which may be read-only
 
 METRIC = "compress_MBps_level9_byte_identical"
 UNIT = "MB/s"
+DUMP_WINDOW = 64 << 10                  # --dump-outputs: bytes per sampled window of the stream
+DUMP_WINDOWS = 128                      # 8 MiB of stream bytes, 32 MiB as float32
 
 
 def parse():
@@ -45,7 +51,33 @@ def parse():
     ap.add_argument("--level", type=int, default=9)
     ap.add_argument("--no-verify", action="store_true")
     ap.add_argument("--cpu-sample-mb", type=int, default=0, help="cpu_baseline sample size (0 = auto)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the stream of the last timed step to DIR (.npy)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+def dump_stream(out_dir, stream):
+    """Writes a compressed stream (uint8 array) for output-to-output comparison of two builds:
+        stream_length.npy   float64 [1]     its length in bytes
+        stream_offsets.npy  float64 [k]     where each row of stream_bytes starts in the stream
+        stream_bytes.npy    float32 [k, w]  byte values
+    A stream of at most DUMP_WINDOWS * DUMP_WINDOW bytes is written whole, as one row.  A longer one is sampled as
+    DUMP_WINDOWS windows of DUMP_WINDOW bytes: its first (stream header, first block) and its last (footer with the
+    combined CRC), and the others at offsets drawn from a fixed seed."""
+    os.makedirs(out_dir, exist_ok=True)
+    n = int(stream.size)
+    if n <= DUMP_WINDOWS * DUMP_WINDOW:
+        offs = np.zeros(1, dtype=np.int64)
+        rows = stream[None, :]
+    else:
+        mid = np.sort(np.random.default_rng(0).integers(0, n - DUMP_WINDOW + 1, size=DUMP_WINDOWS - 2))
+        offs = np.concatenate([[0], mid, [n - DUMP_WINDOW]]).astype(np.int64)
+        rows = stream[offs[:, None] + np.arange(DUMP_WINDOW)]
+    np.save(os.path.join(out_dir, "stream_length.npy"), np.array([n], dtype=np.float64))
+    np.save(os.path.join(out_dir, "stream_offsets.npy"), offs.astype(np.float64))
+    np.save(os.path.join(out_dir, "stream_bytes.npy"), rows.astype(np.float32))
 
 
 def measured_peak():
@@ -208,8 +240,10 @@ def run_reference(args):
     times = []
     for _ in range(steps):
         t0 = time.perf_counter()
-        pyref.compress_stream(raw, args.level, pyref.SPEC, threads=threads)
+        out = pyref.compress_stream(raw, args.level, pyref.SPEC, threads=threads)
         times.append(time.perf_counter() - t0)
+    if args.dump_outputs:
+        dump_stream(args.dump_outputs, np.frombuffer(out, dtype=np.uint8))
     dt = float(np.mean(times))
     value = len(raw) / 1e6 / dt
     sample = ("the whole workload (%d bytes)" % len(raw)) if len(raw) == total else "first %d bytes of the workload" % len(raw)
@@ -439,6 +473,14 @@ def _main(args, real_stdout):
         return 0
     e2e_value = total / 1e6 * args.steps / e2e_dt
     h2d_total, d2h_total = int(h2d), int(d2h)
+
+    if args.dump_outputs:
+        # N = 1: the stream of the last HBM-resident step (the one `value` times).  N > 1: those steps leave each rank's
+        # blocks on its own GPU, so the whole stream rank 0 holds is the one of the last multi-GPU call.
+        if world == 1:
+            dump_stream(args.dump_outputs, d_out[:state["dev_len"]].cpu().numpy())
+        else:
+            dump_stream(args.dump_outputs, h_out[:state["merged_len"]].numpy())
 
     # ---- verification outside the timed region ----
     verified = None
