@@ -38,7 +38,7 @@ EXPORTS = [
     "bz2b200_reset_kernel_stats", "bz2b200_stream_plan_dev", "bz2b200_compress_range_dev",
     "bz2b200_shard_plan_dev", "bz2b200_shard_compress_dev", "bz2b200_shift_bits_dev", "bz2b200_shard_scan_dev",
     "bz2b200_create_multi", "bz2b200_destroy_multi", "bz2b200_last_error_multi", "bz2b200_multi_devices",
-    "bz2b200_multi_context", "bz2b200_compress_stream_multi", "bz2b200_multi_stats",
+    "bz2b200_multi_context", "bz2b200_compress_stream_multi", "bz2b200_decompress_stream_multi", "bz2b200_multi_stats",
     "bz2b200_zstream_open", "bz2b200_zstream_write", "bz2b200_zstream_close",
 ]
 
@@ -116,6 +116,7 @@ def load_library():
     L.bz2b200_multi_context.argtypes = [vp, C.c_int]
     L.bz2b200_multi_context.restype = vp
     L.bz2b200_compress_stream_multi.argtypes = [vp, u8p, C.c_size_t, C.c_int, u8p, C.c_size_t, szp]
+    L.bz2b200_decompress_stream_multi.argtypes = [vp, u8p, C.c_size_t, u8p, C.c_size_t, szp]
     L.bz2b200_multi_stats.argtypes = [vp, C.POINTER(C.c_uint64 * 8)]
     L.bz2b200_zstream_open.argtypes = [vp, C.c_int, SINK, vp, C.POINTER(vp)]
     L.bz2b200_zstream_write.argtypes = [vp, u8p, C.c_size_t]
@@ -484,6 +485,31 @@ class MultiEngine:
         out = np.empty(cap, dtype=np.uint8)
         n = self.compress_into(a.ctypes.data, a.size, level, out.ctypes.data, cap)
         return out[:n].tobytes()
+
+    def decompress_into(self, in_ptr, n, out_ptr, out_cap):
+        """decompress (decompress.rs:38) on the ranks: raw host pointers (page-locked for full overlap) -> length."""
+        ln = C.c_size_t()
+        rc = self._L.bz2b200_decompress_stream_multi(self._h, in_ptr, n, out_ptr, out_cap, C.byref(ln))
+        if rc != OK:
+            raise Bz2B200Error(rc, self._L.bz2b200_last_error_multi(self._h).decode())
+        return ln.value
+
+    def decompress(self, data, max_out=None):
+        """The decompressed bytes of `data`; without `max_out`, a too-small first guess is retried once at the exact size
+        the failed call reports."""
+        a = _np_u8(data)
+        cap = max_out if max_out is not None else max(a.size * 8, 1 << 20)
+        out = np.empty(cap, dtype=np.uint8)
+        ln = C.c_size_t()
+        rc = self._L.bz2b200_decompress_stream_multi(self._h, a.ctypes.data, a.size, out.ctypes.data, cap, C.byref(ln))
+        if rc == E_CAP and max_out is None:
+            cap = ln.value
+            out = np.empty(max(cap, 1), dtype=np.uint8)
+            rc = self._L.bz2b200_decompress_stream_multi(self._h, a.ctypes.data, a.size, out.ctypes.data, cap,
+                                                         C.byref(ln))
+        if rc != OK:
+            raise Bz2B200Error(rc, self._L.bz2b200_last_error_multi(self._h).decode())
+        return out[:ln.value].tobytes()
 
     def stats(self):
         st = (C.c_uint64 * 8)()

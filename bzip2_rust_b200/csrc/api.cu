@@ -1,5 +1,6 @@
 // api.cu -- C ABI of libbz2b200 (include/bz2b200.h): context, staging, stage seams.
 #include "common.cuh"
+#include <atomic>
 #include <string.h>
 #include <new>
 
@@ -13,7 +14,16 @@ static void release_device_buffers(bz2b200_ctx *c) {
     for (DevBuf *b : all) b->release();
 }
 
+namespace {
+constexpr int DEV_SLOTS = 64;                // devices beyond share a slot: the lock is then merely taken more often
+std::atomic<int> g_ctx_on_dev[DEV_SLOTS];
+std::mutex g_dev_lock[DEV_SLOTS];
+}  // namespace
+int bz_contexts_on_device(int device) { return g_ctx_on_dev[device % DEV_SLOTS].load(); }
+std::mutex &bz_device_lock(int device) { return g_dev_lock[device % DEV_SLOTS]; }
+
 bz2b200_ctx::~bz2b200_ctx() {
+    g_ctx_on_dev[device % DEV_SLOTS]--;
     cudaSetDevice(device);
     release_device_buffers(this);
     h_stage.release(); h_small.release(); h_out.release();
@@ -42,6 +52,7 @@ int bz2b200_create(int device, bz2b200_ctx **out) {
     bz2b200_ctx *ctx = new (std::nothrow) bz2b200_ctx();
     if (!ctx) return BZ2B200_E_NOMEM;
     ctx->device = device;
+    g_ctx_on_dev[device % DEV_SLOTS]++;      // the destructor counts it down
     if (cudaSetDevice(device) != cudaSuccess ||
         cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking) != cudaSuccess) {
         delete ctx;

@@ -280,3 +280,43 @@ int bz_rle1_window(bz2b200_ctx *ctx, const u8 *d_x, u32 W, int level, bool is_eo
 int bz_crc_dev(bz2b200_ctx *ctx, const u8 *d_x, u32 n, u32 *d_crc_out);
 // api.cu
 int bz_compress_batch(bz2b200_ctx *ctx, const Batch &B, const u32 *d_crc, HufOut &H);
+// Contexts of this process on one device, and a lock per device.  The decoder's walkers spin on flags their producer
+// kernel sets (decode_bounds.cuh); with several contexts on one device it runs that phase under the lock.
+int bz_contexts_on_device(int device);
+std::mutex &bz_device_lock(int device);
+
+// ---- decode.cu: the decode core shared by bz2b200_decompress_stream and bz2b200_decompress_stream_multi ----
+// It decodes the chain of blocks and footers that starts in bits [8*lo, hi_bit) of the input; the device holds bytes
+// [lo, lo + len) of it, followed by 64 zero bytes.  Bit positions it reports are absolute (from the input's start).
+enum { DEC_BLOCK = 0, DEC_FOOTER = 1, DEC_STREAM = 2 };
+struct DecEvent {                  // in chain order
+    u64 bit;                       // where the element starts
+    u32 val;                       // block: stored CRC; footer: stored combined CRC; stream: level of its header
+    u32 nblock;                    // block: RLE1 length
+    int kind;
+};
+constexpr long long DEC_ENDED = 1ll << 62;   // chain end after the footer of the input's last stream
+constexpr int DEC_ABORTED = 1;               // DecSink::chain_start gave up (another window failed)
+struct DecSink {
+    // absolute bit where the window's chain begins (DEC_ENDED: before the window), < 0 = abort; called once, after
+    // the first batch's entropy decode, when the window did not know its start
+    virtual long long chain_start() { return -1; }
+    // the chain leaves the window at this absolute bit (or DEC_ENDED); may be called more than once with one value
+    virtual void chain_end(long long) {}
+    // a batch decodes to `nbytes`; `last` = no element of the window follows.  Sets the device buffer the bytes are
+    // written to (>= nbytes + 64) and optionally a host destination the core copies them to before its CRC check.
+    virtual int counted(u64 nbytes, bool last, u8 **d_out, u8 **h_out) = 0;
+    // the batch's bytes in d_out passed their block CRCs
+    virtual int ready(const u8 *, u64) { return BZ2B200_OK; }
+    virtual ~DecSink() {}
+};
+struct DecWindow {
+    const u8 *in; size_t n;        // the whole input, host
+    const u8 *d_win; size_t lo, len;
+    u64 hi_bit;                    // elements from here on belong to the next window (~0: none)
+    long long expect;              // absolute bit of the first element, -1 = ask DecSink::chain_start
+    u32 max_block;                 // buffers and bounds of every block
+    const std::vector<u64> *cand;  // candidate bits relative to d_win, sorted by position, bit 63 = footer magic
+};
+int bz_dec_candidates(bz2b200_ctx *ctx, const u8 *d_win, size_t len, u32 cap, std::vector<u64> &cand);
+int bz_decode_core(bz2b200_ctx *ctx, const DecWindow &w, DecSink &sink, std::vector<DecEvent> &ev);

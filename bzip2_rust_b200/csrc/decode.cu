@@ -70,6 +70,7 @@ __device__ __forceinline__ u32 split_index(u32 row, u32 key, u32 nreg) { return 
 __global__ void __launch_bounds__(256) k_ibwt_chase(const u32 *P, const u32 *len, const u32 *keys, u32 stride,
                                                     u32 *seglen, u32 *segnext, u32 sstride) {
     u32 b = blockIdx.y, n = len[b], key = keys[b];
+    if (n == 0) return;                                     // off-chain candidate of the batch: nothing to rank
     u32 nreg = (n + SPLIT - 1) / SPLIT;
     u32 j = blockIdx.x * 256 + threadIdx.x;
     if (j > nreg) return;
@@ -106,6 +107,7 @@ struct CoarseGeom {                      // jk = the origin's splitter: regular 
 __global__ void __launch_bounds__(128) k_ibwt_coarse(const u32 *len, const u32 *keys, const u32 *seglen, const u32 *segnext,
                                                      u32 sstride, u32 *clen, u32 *chops, u32 *cnext, u32 cstride) {
     u32 b = blockIdx.y;
+    if (len[b] == 0) return;                                // k_ibwt_chase wrote no segnext for it
     const CoarseGeom g(len[b], keys[b]);
     u32 c = blockIdx.x * 128 + threadIdx.x;
     if (c > g.ncr) return;
@@ -153,7 +155,7 @@ __global__ void __launch_bounds__(128) k_ibwt_fill(const u32 *len, const u32 *ke
                                                    u32 *visit_off, u32 vstride) {
     u32 b = blockIdx.y;
     u32 u = blockIdx.x * 128 + threadIdx.x;
-    if (u >= ncvisit[b]) return;
+    if (len[b] == 0 || u >= ncvisit[b]) return;
     const CoarseGeom g(len[b], keys[b]);
     u32 c = cv_split[(size_t)b * cstride + u];
     u32 j = g.splitter_of(c);
@@ -342,44 +344,39 @@ constexpr u64 FOOT = 1ull << 63;
 constexpr u32 DEC_BATCH = 128;           // candidate blocks decoded per pass (one pass for 100 MB at level 9)
 }  // namespace
 
-extern "C" int bz2b200_decompress_stream(bz2b200_ctx *ctx, const uint8_t *in, size_t n, uint8_t *out, size_t out_cap,
-                                         size_t *out_len) {
-    BZ_API_TRY
-    if (!ctx || !in || !out_len || (!out && out_cap) || n < 14 || n > 0xFFFFFF00ull * 4ull) return BZ2B200_E_ARG;
-    if (in[0] != 'B' || in[1] != 'Z' || in[2] != 'h' || in[3] < '1' || in[3] > '9') return BZ2B200_E_FORMAT;   // decompress.rs:46-62
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    if (cudaSetDevice(ctx->device) != cudaSuccess) return BZ2B200_E_CUDA;
+// every bit offset of d_win[0, len) that looks like a block or footer magic, sorted; BZ2B200_E_FORMAT past `cap`
+int bz_dec_candidates(bz2b200_ctx *ctx, const u8 *d_win, size_t len, u32 cap, std::vector<u64> &cand) {
     cudaStream_t st = ctx->stream;
-    *out_len = 0;
-    BZ_CHECK(ctx->d_in.ensure(n + 64));
-    BZ_CHECK(cudaMemcpyAsync(ctx->d_in.p, in, n, cudaMemcpyHostToDevice, st));
-    BZ_CHECK(cudaMemsetAsync(ctx->d_in.as<u8>() + n, 0, 64, st));       // word loads of the entropy stage read past the last byte
-    // ---- 1. every bit offset that looks like a block or footer magic ----
-    u32 cap = (u32)std::min<size_t>(n / 32 + 64, 0x7fffff00u);
     BZ_CHECK(ctx->d_dec1.ensure((size_t)cap * 8 + 64));
     u64 *d_cand = ctx->d_dec1.as<u64>();
     u32 *d_ncand = (u32 *)(d_cand + cap);
     BZ_CHECK(cudaMemsetAsync(d_ncand, 0, 4, st));
-    ctx->prof_begin(K_DEC_MAGIC, n); k_dec_find_magic<<<(u32)((n + 255) / 256), 256, 0, st>>>(ctx->d_in.as<u8>(), n, d_cand, d_ncand, cap); LAUNCH_OK();
+    ctx->prof_begin(K_DEC_MAGIC, len); k_dec_find_magic<<<(u32)((len + 255) / 256), 256, 0, st>>>(d_win, len, d_cand, d_ncand, cap); LAUNCH_OK();
     u32 ncand = 0;
     BZ_CHECK(cudaMemcpyAsync(&ncand, d_ncand, 4, cudaMemcpyDeviceToHost, st));
     BZ_CHECK(cudaStreamSynchronize(st));
-    if (ncand == 0 || ncand > cap) return BZ2B200_E_FORMAT;
-    std::vector<u64> cand(ncand);
-    BZ_CHECK(cudaMemcpy(cand.data(), d_cand, (size_t)ncand * 8, cudaMemcpyDeviceToHost));
+    cand.clear();
+    if (ncand > cap) { ctx->err = "decode: more magic candidates than the candidate buffer holds"; return BZ2B200_E_FORMAT; }
+    cand.resize(ncand);
+    if (ncand) BZ_CHECK(cudaMemcpy(cand.data(), d_cand, (size_t)ncand * 8, cudaMemcpyDeviceToHost));
     std::sort(cand.begin(), cand.end(), [](u64 a, u64 b) { return (a & ~FOOT) < (b & ~FOOT); });
-    // A magic can also occur by chance inside entropy-coded data, and a file may hold several streams one after the
-    // other (decompress.rs handles neither; libbz2 walks the blocks serially and accepts both).  So the candidates are
-    // only where blocks MAY start: the chain is walked from every decoded block's end, candidates off the chain are
-    // dropped, and a footer that is not the end of the input must be followed by the next stream's "BZh<level>".
-    int level = in[3] - '0';
-    for (u64 c : cand) {                                        // geometry: the largest block size any stream header announces
-        if (!(c & FOOT)) continue;
-        size_t hb = (size_t)(((c & ~FOOT) + 80 + 7) / 8);
-        if (hb + 4 <= n && in[hb] == 'B' && in[hb + 1] == 'Z' && in[hb + 2] == 'h' && in[hb + 3] >= '1' && in[hb + 3] <= '9')
-            level = std::max(level, in[hb + 3] - '0');
-    }
-    const u32 max_block = (u32)level * 100000u;
+    return BZ2B200_OK;
+}
+
+// A magic can also occur by chance inside entropy-coded data, and a file may hold several streams one after the other
+// (decompress.rs handles neither; libbz2 walks the blocks serially and accepts both).  So the candidates are only where
+// blocks MAY start: the chain is walked from every decoded block's end, candidates off the chain are dropped, and a
+// footer that is not the end of the input must be followed by the next stream's "BZh<level>".
+// A window that does not know where its chain enters entropy-decodes the first batch of its candidates first: the true
+// start is the first element at or after the window's first bit, so it is among them.
+int bz_decode_core(bz2b200_ctx *ctx, const DecWindow &w, DecSink &sink, std::vector<DecEvent> &ev) {
+    cudaStream_t st = ctx->stream;
+    const std::vector<u64> &cand = *w.cand;
+    const size_t ncand = cand.size();
+    const size_t n = w.len;                                     // bytes on the device
+    const u64 lo8 = (u64)w.lo * 8;
+    const u64 hi = w.hi_bit == ~0ull ? ~0ull : w.hi_bit - lo8;  // window-relative, like every bit below
+    const u32 max_block = w.max_block;
     const u32 stride = ((max_block + 64 + BZ_TILE - 1) / BZ_TILE) * BZ_TILE;
     const u32 sel_stride = max_block / 50 + 8;
     const u32 max_sym = max_block + 2;                           // every symbol but EOB yields at least one byte
@@ -412,115 +409,156 @@ extern "C" int bz2b200_decompress_stream(bz2b200_ctx *ctx, const uint8_t *in, si
     u32 *d_rand = d_keys + NB;
     u32 *d_se = d_rand + NB;
     u64 *d_rend = (u64 *)(d_se + 2 * (size_t)NB);                // after the spans; 8-byte aligned (all counts are multiples of NB * 4, NB even)
-    const u8 *d_bits = ctx->d_in.as<u8>();
+    const u8 *d_bits = w.d_win;
     if (!ctx->dec_attr_done) { BZ_CHECK(cudaFuncSetAttribute(k_dec_bounds, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)JRING_BYTES)); ctx->dec_attr_done = true; }
 
-    auto read32 = [&](u64 bit) {                                // 32 bits at an arbitrary bit offset of the input
+    auto read32 = [&](u64 bit) {                                // 32 bits at an absolute bit offset of the host input
         size_t byte = (size_t)(bit >> 3); int sh = (int)(bit & 7);
-        u64 w = 0;
-        for (int k = 0; k < 5; k++) w = (w << 8) | (byte + k < n ? in[byte + k] : 0);
-        return (u32)((w >> (8 - sh)) & 0xffffffffull);
+        u64 v = 0;
+        for (int k = 0; k < 5; k++) v = (v << 8) | (byte + k < w.n ? w.in[byte + k] : 0);
+        return (u32)((v >> (8 - sh)) & 0xffffffffull);
     };
     size_t ci = 0;                                              // next candidate to look at
-    u64 expect = 32;                                            // bit offset where the next block / footer must start
+    bool known = w.expect >= 0;                                 // the chain start is known
+    u64 expect = known ? (u64)w.expect - lo8 : 0;               // bit offset where the next block / footer must start
+    bool comb_known = known;                                    // the window has seen the start of the current stream
     u32 combined = 0;                                           // running combined CRC of the current stream
-    size_t total_out = 0;
+    bool have_batch = false;                                    // `starts` were decoded before the chain start was known
     std::vector<u64> starts, rends;
     const u64 range_limit = [] { const char *e = getenv("BZ2B200_DEC_RANGE_LIMIT"); return e ? (u64)strtoull(e, nullptr, 10) : 0ull; }();
     std::vector<DecTail> db;
     std::vector<u32> hlen(NB), hkey(NB), hrand(NB), se(2 * (size_t)NB), crcs(NB);
     std::vector<u64> olen(NB), ooff(NB);
     for (;;) {
-        while (ci < ncand && (cand[ci] & ~FOOT) < expect) ci++;
-        if (ci == ncand || (cand[ci] & ~FOOT) != expect) { ctx->err = "decode: no block or footer magic at bit " + std::to_string(expect); return BZ2B200_E_FORMAT; }
-        if (cand[ci] & FOOT) {                                  // end of a stream: combined CRC, then end of input or another stream
-            if (read32(expect + 48) != combined) return BZ2B200_E_CRC;                        // enforced, unlike decompress.rs:394-402
-            size_t hb = (size_t)((expect + 80 + 7) / 8);
-            if (hb == n) break;
-            if (hb + 4 > n || in[hb] != 'B' || in[hb + 1] != 'Z' || in[hb + 2] != 'h' || in[hb + 3] < '1' || in[hb + 3] > '9') {
-                ctx->err = "decode: trailing bytes after the stream footer"; return BZ2B200_E_FORMAT;
+        if (known) {
+            if (expect >= hi) { sink.chain_end((long long)(expect + lo8)); return BZ2B200_OK; }
+            while (ci < ncand && (cand[ci] & ~FOOT) < expect) ci++;
+            if (ci == ncand || (cand[ci] & ~FOOT) != expect) { ctx->err = "decode: no block or footer magic at bit " + std::to_string(expect + lo8); return BZ2B200_E_FORMAT; }
+            if (cand[ci] & FOOT) {                              // end of a stream: combined CRC, then end of input or another stream
+                const u32 stored = read32(expect + lo8 + 48);
+                ev.push_back(DecEvent{expect + lo8, stored, 0, DEC_FOOTER});
+                if (comb_known && stored != combined) return BZ2B200_E_CRC;                    // enforced, unlike decompress.rs:394-402
+                size_t hb = (size_t)((expect + lo8 + 80 + 7) / 8);
+                if (hb == w.n) { sink.chain_end(DEC_ENDED); return BZ2B200_OK; }
+                const u8 *in = w.in;
+                if (hb + 4 > w.n || in[hb] != 'B' || in[hb + 1] != 'Z' || in[hb + 2] != 'h' || in[hb + 3] < '1' || in[hb + 3] > '9') {
+                    ctx->err = "decode: trailing bytes after the stream footer"; return BZ2B200_E_FORMAT;
+                }
+                ev.push_back(DecEvent{(u64)hb * 8, (u32)(in[hb + 3] - '0'), 0, DEC_STREAM});
+                combined = 0; comb_known = true;
+                expect = (u64)hb * 8 + 32 - lo8;
+                continue;
             }
-            combined = 0;
-            expect = (u64)hb * 8 + 32;
+        }
+        bool reuse = false;
+        if (have_batch) for (u64 s : starts) reuse |= s == expect;
+        have_batch = false;
+        u32 nb = (u32)starts.size();
+        if (!reuse) {
+            // ---- 2. entropy decode of the next candidate blocks (decode4.cuh) ----
+            // A block's data cannot reach past the next candidate -- unless that one is a chance magic inside it: the walk
+            // then leaves the range its jump tables cover and finishes code by code.
+            starts.clear(); rends.clear();
+            u64 max_range = 0;
+            for (size_t k = ci; k < ncand && starts.size() < NB; k++) {
+                if (cand[k] & FOOT) continue;
+                if ((cand[k] & ~FOOT) >= hi) break;             // the next window's
+                u64 re = k + 1 < ncand ? (cand[k + 1] & ~FOOT) : (u64)n * 8;
+                // no valid block is longer than 20 bits per symbol plus its header (symbol map, selectors, six tables): a
+                // damaged stream whose next magic is far away must not size the jump tables
+                re = std::min<u64>(re, cand[k] + (u64)20 * (max_block + 64) + ((u64)1 << 19));
+                if (range_limit) re = std::min(re, cand[k] + range_limit);     // test knob: as if a chance magic cut the range
+                starts.push_back(cand[k]); rends.push_back(re);
+                max_range = std::max(max_range, re - cand[k]);
+            }
+            nb = (u32)starts.size();
+            if (nb) {
+                BZ_CHECK(cudaMemcpyAsync(d_starts, starts.data(), (size_t)nb * 8, cudaMemcpyHostToDevice, st));
+                BZ_CHECK(cudaMemcpyAsync(d_rend, rends.data(), (size_t)nb * 8, cudaMemcpyHostToDevice, st));
+                ctx->prof_begin(K_DEC_HEADER, 0); k_dec_header<<<nb, 32, 0, st>>>(d_bits, n, d_starts, ctx->d_sel.as<u8>(), sel_stride, d_tabs); LAUNCH_OK();
+                {   // group boundaries: jump tables (2 bytes per bit offset and table), and the walkers of the same blocks following
+                    // them window by window from a second, high-priority stream (their few CTAs are placed as soon as the producer's
+                    // first ones retire); in slices of the batch when the tables of all its blocks would not fit the budget
+                    // (incompressible data: 88 MB per block).  The producer is launched first: a tool that serialises kernels in
+                    // launch order (ncu, compute-sanitizer) then still terminates.
+                    // The walkers spin until their producer's CTAs have run.  One context's walkers (at most DEC_BATCH CTAs, two per
+                    // SM by shared memory) leave most SMs to its producer; the walkers of several contexts on one device could take
+                    // every SM while their producers wait for one.  So when this process holds more than one context on the device,
+                    // the phase runs under a per-device lock until its walkers are done: then the walkers on the device are those of
+                    // one batch, and every other kernel of the process on it finishes without waiting for anything.  (The count is
+                    // read without the lock: a context created while the device's only other context runs this phase unlocked
+                    // overlaps it once -- two batches, at most 128 of the 148 SMs, still leave SMs to both producers.)
+                    std::unique_lock<std::mutex> dev_lk;
+                    if (bz_contexts_on_device(ctx->device) > 1) dev_lk = std::unique_lock<std::mutex>(bz_device_lock(ctx->device));
+                    const u32 nwin_max = jump_windows(max_range);
+                    const size_t jstride = (size_t)nwin_max * 6 * 2 * JW;
+                    const size_t budget = (size_t)6 << 30;
+                    const u32 slice = (u32)std::max<size_t>(1, std::min<size_t>(nb, budget / jstride));
+                    BZ_CHECK(ctx->d_VALA.ensure((size_t)slice * jstride));
+                    BZ_CHECK(ctx->d_VALB.ensure((size_t)slice * nwin_max * 4));
+                    u32 *d_flags = ctx->d_VALB.as<u32>();
+                    if (!ctx->s_hi) {
+                        int lo = 0, hi_p = 0;
+                        BZ_CHECK(cudaDeviceGetStreamPriorityRange(&lo, &hi_p));
+                        BZ_CHECK(cudaStreamCreateWithPriority(&ctx->s_hi, cudaStreamNonBlocking, hi_p));
+                        for (int q = 0; q < 2; q++) BZ_CHECK(cudaEventCreateWithFlags(&ctx->ev_dec[q], cudaEventDisableTiming));
+                    }
+                    for (u32 b0 = 0; b0 < nb; b0 += slice) {
+                        const u32 cnt = std::min(slice, nb - b0);
+                        BZ_CHECK(cudaMemsetAsync(d_flags, 0, (size_t)cnt * nwin_max * 4, st));
+                        BZ_CHECK(cudaEventRecord(ctx->ev_dec[0], st));                   // headers parsed, flags clear, the previous slice done
+                        ctx->prof_begin(K_DEC_JUMPS, (u64)cnt * jstride);
+                        k_dec_jumps<<<dim3(cnt, nwin_max), 256, 0, st>>>(d_bits, n, d_tabs, d_rend, ctx->d_VALA.as<u8>(), jstride, d_flags, nwin_max, b0); LAUNCH_OK();
+                        BZ_CHECK(cudaStreamWaitEvent(ctx->s_hi, ctx->ev_dec[0], 0));
+                        k_dec_bounds<<<cnt, 32, JRING_BYTES, ctx->s_hi>>>(d_bits, n, ctx->d_sel.as<u8>(), sel_stride, d_tabs, d_rend, ctx->d_VALA.as<u8>(), jstride, d_flags, nwin_max, d_gbit, max_sym, b0);
+                        ctx->launches++;
+                        if (cudaGetLastError() != cudaSuccess) { ctx->err = "decode: k_dec_bounds launch"; cudaStreamSynchronize(st); return BZ2B200_E_CUDA; }
+                        BZ_CHECK(cudaEventRecord(ctx->ev_dec[1], ctx->s_hi));
+                        ctx->prof_begin(K_DEC_BOUNDS, n);                                // as timed on the main stream: what the walk adds after the producer
+                        BZ_CHECK(cudaStreamWaitEvent(st, ctx->ev_dec[1], 0));
+                        ctx->prof_end(); ctx->launches--;
+                    }
+                    if (dev_lk.owns_lock()) BZ_CHECK(cudaStreamSynchronize(ctx->s_hi));
+                }
+                dim3 gs((sel_stride + 127) / 128, nb);
+                ctx->prof_begin(K_DEC_SYMS, n); k_dec_syms<<<gs, 128, 0, st>>>(d_bits, n, ctx->d_sel.as<u8>(), sel_stride, d_tabs, d_gbit, d_sym, sym_stride); LAUNCH_OK();
+                dim3 gch((ch_stride + 7) / 8, nb);
+                ctx->prof_begin(K_DEC_CHUNKS, 0); k_dec_chunks<<<gch, 256, 0, st>>>(d_tabs, d_sym, sym_stride, d_lists, d_ccount, ch_stride, d_vid, max_block); LAUNCH_OK();
+                ctx->prof_begin(K_DEC_CHUNK_SCAN, 0); k_dec_chunk_scan<<<nb, 256, 0, st>>>(d_tabs, d_lists, d_ccount, d_coff, ch_stride, max_block); LAUNCH_OK();
+                ctx->prof_begin(K_DEC_EXPAND, 0); k_dec_expand<<<gch, 256, 0, st>>>(d_tabs, d_sym, sym_stride, d_lists, d_coff, ch_stride, d_vid, ctx->d_T.as<u8>(), stride); LAUNCH_OK();
+                db.resize(nb);
+                BZ_CHECK(cudaMemcpy2DAsync(db.data(), sizeof(DecTail), (const u8 *)d_tabs + offsetof(DecTables, T), sizeof(DecTables),
+                                           sizeof(DecTail), nb, cudaMemcpyDeviceToHost, st));
+                BZ_CHECK(cudaStreamSynchronize(st));
+            }
+        }
+        if (!known) {                                           // the hand-off from the window before
+            long long s = sink.chain_start();
+            if (s < 0) return DEC_ABORTED;
+            if (s == DEC_ENDED) { sink.chain_end(DEC_ENDED); return BZ2B200_OK; }
+            if ((u64)s < lo8) { ctx->err = "decode: chain enters the window before its first bit"; return BZ2B200_E_FORMAT; }
+            known = true;
+            expect = (u64)s - lo8;
+            have_batch = nb != 0;
             continue;
         }
-        // ---- 2. entropy decode of the next candidate blocks (decode4.cuh) ----
-        // A block's data cannot reach past the next candidate -- unless that one is a chance magic inside it: the walk
-        // then leaves the range its jump tables cover and finishes code by code.
-        starts.clear(); rends.clear();
-        u64 max_range = 0;
-        for (size_t k = ci; k < ncand && starts.size() < NB; k++) {
-            if (cand[k] & FOOT) continue;
-            u64 re = k + 1 < ncand ? (cand[k + 1] & ~FOOT) : (u64)n * 8;
-            // no valid block is longer than 20 bits per symbol plus its header (symbol map, selectors, six tables): a
-            // damaged stream whose next magic is far away must not size the jump tables
-            re = std::min<u64>(re, cand[k] + (u64)20 * (max_block + 64) + ((u64)1 << 19));
-            if (range_limit) re = std::min(re, cand[k] + range_limit);     // test knob: as if a chance magic cut the range
-            starts.push_back(cand[k]); rends.push_back(re);
-            max_range = std::max(max_range, re - cand[k]);
-        }
-        const u32 nb = (u32)starts.size();
-        BZ_CHECK(cudaMemcpyAsync(d_starts, starts.data(), (size_t)nb * 8, cudaMemcpyHostToDevice, st));
-        BZ_CHECK(cudaMemcpyAsync(d_rend, rends.data(), (size_t)nb * 8, cudaMemcpyHostToDevice, st));
-        ctx->prof_begin(K_DEC_HEADER, 0); k_dec_header<<<nb, 32, 0, st>>>(d_bits, n, d_starts, ctx->d_sel.as<u8>(), sel_stride, d_tabs); LAUNCH_OK();
-        {   // group boundaries: jump tables (2 bytes per bit offset and table), and the walkers of the same blocks following
-            // them window by window from a second, high-priority stream (their few CTAs are placed as soon as the producer's
-            // first ones retire); in slices of the batch when the tables of all its blocks would not fit the budget
-            // (incompressible data: 88 MB per block).  The producer is launched first: a tool that serialises kernels in
-            // launch order (ncu, compute-sanitizer) then still terminates.
-            const u32 nwin_max = jump_windows(max_range);
-            const size_t jstride = (size_t)nwin_max * 6 * 2 * JW;
-            const size_t budget = (size_t)6 << 30;
-            const u32 slice = (u32)std::max<size_t>(1, std::min<size_t>(nb, budget / jstride));
-            BZ_CHECK(ctx->d_VALA.ensure((size_t)slice * jstride));
-            BZ_CHECK(ctx->d_VALB.ensure((size_t)slice * nwin_max * 4));
-            u32 *d_flags = ctx->d_VALB.as<u32>();
-            if (!ctx->s_hi) {
-                int lo = 0, hi = 0;
-                BZ_CHECK(cudaDeviceGetStreamPriorityRange(&lo, &hi));
-                BZ_CHECK(cudaStreamCreateWithPriority(&ctx->s_hi, cudaStreamNonBlocking, hi));
-                for (int q = 0; q < 2; q++) BZ_CHECK(cudaEventCreateWithFlags(&ctx->ev_dec[q], cudaEventDisableTiming));
-            }
-            for (u32 b0 = 0; b0 < nb; b0 += slice) {
-                const u32 cnt = std::min(slice, nb - b0);
-                BZ_CHECK(cudaMemsetAsync(d_flags, 0, (size_t)cnt * nwin_max * 4, st));
-                BZ_CHECK(cudaEventRecord(ctx->ev_dec[0], st));                   // headers parsed, flags clear, the previous slice done
-                ctx->prof_begin(K_DEC_JUMPS, (u64)cnt * jstride);
-                k_dec_jumps<<<dim3(cnt, nwin_max), 256, 0, st>>>(d_bits, n, d_tabs, d_rend, ctx->d_VALA.as<u8>(), jstride, d_flags, nwin_max, b0); LAUNCH_OK();
-                BZ_CHECK(cudaStreamWaitEvent(ctx->s_hi, ctx->ev_dec[0], 0));
-                k_dec_bounds<<<cnt, 32, JRING_BYTES, ctx->s_hi>>>(d_bits, n, ctx->d_sel.as<u8>(), sel_stride, d_tabs, d_rend, ctx->d_VALA.as<u8>(), jstride, d_flags, nwin_max, d_gbit, max_sym, b0);
-                ctx->launches++;
-                if (cudaGetLastError() != cudaSuccess) { ctx->err = "decode: k_dec_bounds launch"; cudaStreamSynchronize(st); return BZ2B200_E_CUDA; }
-                BZ_CHECK(cudaEventRecord(ctx->ev_dec[1], ctx->s_hi));
-                ctx->prof_begin(K_DEC_BOUNDS, n);                                // as timed on the main stream: what the walk adds after the producer
-                BZ_CHECK(cudaStreamWaitEvent(st, ctx->ev_dec[1], 0));
-                ctx->prof_end(); ctx->launches--;
-            }
-        }
-        dim3 gs((sel_stride + 127) / 128, nb);
-        ctx->prof_begin(K_DEC_SYMS, n); k_dec_syms<<<gs, 128, 0, st>>>(d_bits, n, ctx->d_sel.as<u8>(), sel_stride, d_tabs, d_gbit, d_sym, sym_stride); LAUNCH_OK();
-        dim3 gch((ch_stride + 7) / 8, nb);
-        ctx->prof_begin(K_DEC_CHUNKS, 0); k_dec_chunks<<<gch, 256, 0, st>>>(d_tabs, d_sym, sym_stride, d_lists, d_ccount, ch_stride, d_vid, max_block); LAUNCH_OK();
-        ctx->prof_begin(K_DEC_CHUNK_SCAN, 0); k_dec_chunk_scan<<<nb, 256, 0, st>>>(d_tabs, d_lists, d_ccount, d_coff, ch_stride, max_block); LAUNCH_OK();
-        ctx->prof_begin(K_DEC_EXPAND, 0); k_dec_expand<<<gch, 256, 0, st>>>(d_tabs, d_sym, sym_stride, d_lists, d_coff, ch_stride, d_vid, ctx->d_T.as<u8>(), stride); LAUNCH_OK();
-        db.resize(nb);
-        BZ_CHECK(cudaMemcpy2DAsync(db.data(), sizeof(DecTail), (const u8 *)d_tabs + offsetof(DecTables, T), sizeof(DecTables),
-                                   sizeof(DecTail), nb, cudaMemcpyDeviceToHost, st));
-        BZ_CHECK(cudaStreamSynchronize(st));
         // ---- the chain inside this batch: candidate k is a block iff the block before it ends exactly there ----
         u32 max_n = 0, used = 0; u64 total_n = 0;
         for (u32 k = 0; k < nb; k++) {
             hlen[k] = 0; hkey[k] = 0; hrand[k] = 0;
             if (starts[k] != expect) continue;                  // inside another block's data: not a block
-            if (db[k].status != 0) { ctx->err = "decode: block at bit " + std::to_string(starts[k]) + " status " + std::to_string(db[k].status); return BZ2B200_E_FORMAT; }
+            if (db[k].status != 0) { ctx->err = "decode: block at bit " + std::to_string(starts[k] + lo8) + " status " + std::to_string(db[k].status); return BZ2B200_E_FORMAT; }
             if (db[k].key >= db[k].nblock) { ctx->err = "decode: origin pointer outside the block"; return BZ2B200_E_FORMAT; }
             hlen[k] = db[k].nblock; hkey[k] = db[k].key; hrand[k] = db[k].pad;
             max_n = std::max(max_n, hlen[k]); total_n += hlen[k];
             combined = ((combined << 1) | (combined >> 31)) ^ db[k].crc;                       // crc.rs:25-27
+            ev.push_back(DecEvent{starts[k] + lo8, db[k].crc, db[k].nblock, DEC_BLOCK});
             expect = db[k].end_bit;
             used = k + 1;
         }
         if (used == 0) { ctx->err = "decode: lost the block chain"; return BZ2B200_E_FORMAT; }
+        const bool last = expect >= hi;                         // the chain left the window: the next one may go on
+        if (last) sink.chain_end((long long)(expect + lo8));
         // candidates up to the last block of the chain are consumed (the next loop skips what lies below `expect`)
         while (ci < ncand && (cand[ci] & ~FOOT) <= starts[used - 1]) ci++;
         BZ_CHECK(cudaMemcpyAsync(d_len, hlen.data(), (size_t)nb * 4, cudaMemcpyHostToDevice, st));
@@ -535,17 +573,17 @@ extern "C" int bz2b200_decompress_stream(bz2b200_ctx *ctx, const uint8_t *in, si
         bool any_rand = false;
         for (u32 k = 0; k < used; k++) any_rand |= hrand[k] != 0;
         if (any_rand) { ctx->prof_begin(K_DEC_MISC, total_n); k_derandomize<<<used, 512, 0, st>>>(ctx->d_bwt.as<u8>(), d_len, d_rand, stride); LAUNCH_OK(); }
-        // ---- 4. inverse RLE1 + CRC; the batch's bytes go to out + total_out ----
+        // ---- 4. inverse RLE1 + CRC; the batch's bytes go where the sink says ----
         ctx->prof_begin(K_DEC_RLE1_COUNT, total_n); k_rle1_inv<0><<<used, 256, 0, st>>>(ctx->d_bwt.as<u8>(), d_len, stride, d_olen, nullptr, nullptr); LAUNCH_OK();
         BZ_CHECK(cudaMemcpyAsync(olen.data(), d_olen, (size_t)used * 8, cudaMemcpyDeviceToHost, st));
         BZ_CHECK(cudaStreamSynchronize(st));
         u64 btotal = 0;
         for (u32 k = 0; k < used; k++) { ooff[k] = btotal; btotal += olen[k]; }
-        *out_len = total_out + (size_t)btotal;
-        if (total_out + btotal > out_cap) return BZ2B200_E_CAP;
-        BZ_CHECK(ctx->d_stream.ensure((size_t)btotal + 64));
+        u8 *d_out = nullptr, *h_out = nullptr;
+        rc = sink.counted(btotal, last, &d_out, &h_out);
+        if (rc) return rc;
         BZ_CHECK(cudaMemcpyAsync(d_ooff, ooff.data(), (size_t)used * 8, cudaMemcpyHostToDevice, st));
-        ctx->prof_begin(K_DEC_RLE1_WRITE, btotal); k_rle1_inv<1><<<used, 256, 0, st>>>(ctx->d_bwt.as<u8>(), d_len, stride, nullptr, d_ooff, ctx->d_stream.as<u8>()); LAUNCH_OK();
+        ctx->prof_begin(K_DEC_RLE1_WRITE, btotal); k_rle1_inv<1><<<used, 256, 0, st>>>(ctx->d_bwt.as<u8>(), d_len, stride, nullptr, d_ooff, d_out); LAUNCH_OK();
         // block CRCs in sub-ranges of at most 2 GiB of output (a block decodes to at most ~46 MB; spans are 32-bit)
         for (u32 k0 = 0; k0 < used;) {
             u32 k1 = k0; u64 sub = 0, max_span = 0;
@@ -554,19 +592,68 @@ extern "C" int bz2b200_decompress_stream(bz2b200_ctx *ctx, const uint8_t *in, si
                 sub += olen[k1]; max_span = std::max(max_span, olen[k1]); k1++;
             }
             BZ_CHECK(cudaMemcpyAsync(d_se + 2 * k0, se.data() + 2 * k0, (size_t)(k1 - k0) * 8, cudaMemcpyHostToDevice, st));
-            rc = bz_crc_spans_dev(ctx, ctx->d_stream.as<u8>() + ooff[k0], d_se + 2 * k0, k1 - k0, (u32)max_span, ctx->d_crc.as<u32>() + k0);
+            rc = bz_crc_spans_dev(ctx, d_out + ooff[k0], d_se + 2 * k0, k1 - k0, (u32)max_span, ctx->d_crc.as<u32>() + k0);
             if (rc) return rc;
             BZ_CHECK(cudaStreamSynchronize(st));                // se is reused by the next sub-range
             k0 = k1;
         }
         BZ_CHECK(cudaMemcpyAsync(crcs.data(), ctx->d_crc.p, (size_t)used * 4, cudaMemcpyDeviceToHost, st));
-        if (btotal) BZ_CHECK(cudaMemcpyAsync(out + total_out, ctx->d_stream.p, (size_t)btotal, cudaMemcpyDeviceToHost, st));
+        if (btotal && h_out) BZ_CHECK(cudaMemcpyAsync(h_out, d_out, (size_t)btotal, cudaMemcpyDeviceToHost, st));
         BZ_CHECK(cudaStreamSynchronize(st));
         for (u32 k = 0; k < used; k++)
-            if (hlen[k] && crcs[k] != db[k].crc) { ctx->err = "decode: CRC mismatch in the block at bit " + std::to_string(starts[k]); return BZ2B200_E_CRC; }   // enforced, unlike decompress.rs:379-386
-        total_out += (size_t)btotal;
+            if (hlen[k] && crcs[k] != db[k].crc) { ctx->err = "decode: CRC mismatch in the block at bit " + std::to_string(starts[k] + lo8); return BZ2B200_E_CRC; }   // enforced, unlike decompress.rs:379-386
+        rc = sink.ready(d_out, btotal);
+        if (rc) return rc;
     }
-    *out_len = total_out;
+}
+
+namespace {
+// the whole input is one window; bytes go straight to the caller's buffer
+struct WholeSink : DecSink {
+    bz2b200_ctx *ctx; u8 *out; size_t out_cap; size_t *out_len; size_t total = 0;
+    int counted(u64 nbytes, bool, u8 **d_out, u8 **h_out) override {
+        *out_len = total + (size_t)nbytes;
+        if (total + nbytes > out_cap) return BZ2B200_E_CAP;
+        BZ_CHECK(ctx->d_stream.ensure((size_t)nbytes + 64));
+        *d_out = ctx->d_stream.as<u8>();
+        *h_out = out + total;
+        total += (size_t)nbytes;
+        return BZ2B200_OK;
+    }
+};
+}  // namespace
+
+extern "C" int bz2b200_decompress_stream(bz2b200_ctx *ctx, const uint8_t *in, size_t n, uint8_t *out, size_t out_cap,
+                                         size_t *out_len) {
+    BZ_API_TRY
+    if (!ctx || !in || !out_len || (!out && out_cap) || n < 14 || n > 0xFFFFFF00ull * 4ull) return BZ2B200_E_ARG;
+    if (in[0] != 'B' || in[1] != 'Z' || in[2] != 'h' || in[3] < '1' || in[3] > '9') return BZ2B200_E_FORMAT;   // decompress.rs:46-62
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    if (cudaSetDevice(ctx->device) != cudaSuccess) return BZ2B200_E_CUDA;
+    cudaStream_t st = ctx->stream;
+    *out_len = 0;
+    BZ_CHECK(ctx->d_in.ensure(n + 64));
+    BZ_CHECK(cudaMemcpyAsync(ctx->d_in.p, in, n, cudaMemcpyHostToDevice, st));
+    BZ_CHECK(cudaMemsetAsync(ctx->d_in.as<u8>() + n, 0, 64, st));       // word loads of the entropy stage read past the last byte
+    // ---- 1. every bit offset that looks like a block or footer magic ----
+    std::vector<u64> cand;
+    int rc = bz_dec_candidates(ctx, ctx->d_in.as<u8>(), n, (u32)std::min<size_t>(n / 32 + 64, 0x7fffff00u), cand);
+    if (rc) return rc;
+    if (cand.empty()) return BZ2B200_E_FORMAT;
+    int level = in[3] - '0';
+    for (u64 c : cand) {                                        // geometry: the largest block size any stream header announces
+        if (!(c & FOOT)) continue;
+        size_t hb = (size_t)(((c & ~FOOT) + 80 + 7) / 8);
+        if (hb + 4 <= n && in[hb] == 'B' && in[hb + 1] == 'Z' && in[hb + 2] == 'h' && in[hb + 3] >= '1' && in[hb + 3] <= '9')
+            level = std::max(level, in[hb + 3] - '0');
+    }
+    DecWindow w{in, n, ctx->d_in.as<u8>(), 0, n, ~0ull, 32, (u32)level * 100000u, &cand};
+    WholeSink sink;
+    sink.ctx = ctx; sink.out = out; sink.out_cap = out_cap; sink.out_len = out_len;
+    std::vector<DecEvent> ev;
+    rc = bz_decode_core(ctx, w, sink, ev);
+    if (rc) return rc;
+    *out_len = sink.total;
     return BZ2B200_OK;
     BZ_API_CATCH
 }

@@ -18,6 +18,7 @@
 //   "BZh<level>" and the footer (bitwriter.rs:67-72, :103-114).
 // The output is the byte string a single bz2b200_compress_stream call produces, for any N.
 #include "common.cuh"
+#include <algorithm>
 #include <atomic>
 #include <chrono>
 #include <condition_variable>
@@ -45,11 +46,20 @@ struct MWin {                                // one input window
     std::atomic<long long> bits_pub{-1};     // bit count, published when the window's blocks are compressed
     cudaEvent_t ev_up = nullptr;             // fires when the window's upload has landed (recorded on its rank's upload stream)
     std::atomic<int> up_rec{0};              // ev_up has been recorded (an event that was never recorded cannot be waited for)
+    // decompression
+    std::vector<DecEvent> events;            // the window's chain, in order
+    std::atomic<long long> len_pub{-1};      // decoded length, published after the count pass of the window's last batch
+    u64 out_len = 0, copied = 0;             // bytes decoded / already handed to the download stream
+    long long chain_out = -1;                // where the chain leaves the window (DEC_ENDED after the input's last footer)
+    int rc = 0;                              // BZ2B200_E_*, DEC_ABORTED when it stopped because another window failed
+    std::string err;
 };
 struct MRank {
     bz2b200_ctx *ctx = nullptr;
     std::thread th;
     DevBuf d_win[2], d_out, d_shift[2];      // two windows in flight: one being compressed, the next one arriving
+    DevBuf d_dec[2];                         // decompression: decoded batches, one being written while the other downloads
+    u64 ndec = 0;                            // batches decoded in the current call
     std::vector<cudaEvent_t> up_ev[2];       // upload progress of each window buffer
     cudaEvent_t ev_shift = nullptr;
     std::vector<cudaEvent_t> win_ev;         // one per window of this rank in the current call (MWin::ev_up)
@@ -67,7 +77,8 @@ struct bz2b200_mctx {
     int n = 0;
     std::vector<std::unique_ptr<MRank>> rk;
     std::vector<std::unique_ptr<MWin>> win;  // windows of the current call
-    std::mutex call_mu;                      // one compress call at a time
+    std::mutex call_mu;                      // one call at a time
+    bool decode = false;                     // the job: decompression (else compression)
     std::mutex mu;
     std::condition_variable cv_job, cv_done;
     u64 seq = 0;
@@ -106,6 +117,7 @@ int rank_fail(bz2b200_mctx *m, MRank &R, int rc, const char *what) {
 #define MCHECK(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { R.rc = BZ2B200_E_CUDA; R.err = std::string(#call) + ": " + cudaGetErrorString(e_); m->abort.store(1); return R.rc; } } while (0)
 
 const size_t LOOK0 = 4u << 20;               // look-ahead for the last block of a window, grown on demand
+constexpr u64 FOOT_BIT = 1ull << 63;          // a decoder candidate that is a footer magic
 inline size_t chunk_bytes() {
     static const size_t c = [] { const char *e = getenv("BZ2B200_E2E_CHUNK_MB"); int v = e ? atoi(e) : 8; return (size_t)(v < 1 ? 1 : v) << 20; }();
     return c;
@@ -268,6 +280,152 @@ int run_rank(bz2b200_mctx *m, int r) {
     return BZ2B200_OK;
 }
 
+// ---- decompression ---------------------------------------------------------------------------------------------
+// The compressed input is cut into byte windows dealt round robin like the compressor's.  Rank r, for each window:
+//   1. waits for its upload (window + 4 MiB look-ahead: the longest block that can start in it), finds the magic
+//      candidates and entropy-decodes the first batch of those in its range -- work needed wherever the chain enters
+//   2. waits for the chain from window - 1, walks it (decode.cu) and hands where it leaves to window + 1 before the
+//      inverse BWT; a footer belongs to the window it starts in, which also checks the next "BZh<level>" header
+//   3. publishes its decoded length after the count pass of its last batch; once the lengths of the windows before it
+//      are known, every batch is copied from the device straight to its final place in `out` (download stream)
+// the calling thread then walks the windows' events in order: combined CRCs, the block size the headers allow.
+// 24 MiB of -9 text (3.8-4.0:1 on the decode benchmark's text) hold some 105 blocks: one decoder batch of 128.  Less
+// compressible data gives fewer blocks per window; -1 streams and very compressible data give several batches per
+// window, which then copies batch by batch (a rank still holds at most two decoded batches while it waits for its offset).
+const size_t DEC_WIN_MAX = 24u << 20, DEC_WIN_MIN = 4u << 20;
+
+struct WinSink : DecSink {
+    bz2b200_mctx *m; MRank *R; MWin *W; size_t k;
+    bz2b200_ctx *ctx;
+    double t_wait = 0, t_out = 0;
+    long long chain_start() override {
+        auto t0 = clk::now();
+        long long v = wait_value(m, W->chain_in);
+        t_wait += ms_since(t0);
+        return v;
+    }
+    void chain_end(long long bit) override {
+        W->chain_out = bit;
+        if (k + 1 < m->win.size()) m->win[k + 1]->chain_in.store(bit, std::memory_order_release);
+    }
+    int counted(u64 nbytes, bool last, u8 **d_out, u8 **h_out) override {
+        W->out_len += nbytes;                                   // counted even when `out` cannot take it (E_CAP reports the size)
+        if (last) W->len_pub.store((long long)W->out_len, std::memory_order_release);
+        DevBuf &b = R->d_dec[R->ndec & 1];
+        if (R->ndec >= 2) BZ_CHECK(cudaStreamSynchronize(ctx->s_down));   // the download that last read this buffer
+        R->ndec++;
+        BZ_CHECK(b.ensure((size_t)nbytes + 64));
+        *d_out = b.as<u8>();
+        *h_out = nullptr;
+        return BZ2B200_OK;
+    }
+    int ready(const u8 *d_out, u64 nbytes) override {
+        auto t0 = clk::now();
+        u64 off = W->copied;
+        for (size_t q = 0; q < k; q++) {
+            long long v = wait_value(m, m->win[q]->len_pub);
+            if (v < 0) return DEC_ABORTED;
+            off += (u64)v;
+        }
+        W->copied += nbytes;
+        if (nbytes && off + nbytes <= m->out_cap) {
+            BZ_CHECK(cudaEventRecord(R->ev_shift, ctx->stream));
+            BZ_CHECK(cudaStreamWaitEvent(ctx->s_down, R->ev_shift, 0));
+            BZ_CHECK(cudaMemcpyAsync(m->out + off, d_out, (size_t)nbytes, cudaMemcpyDeviceToHost, ctx->s_down));
+            R->d2h += nbytes;
+        }
+        t_out += ms_since(t0);
+        return BZ2B200_OK;
+    }
+};
+
+// test knob: a spurious block candidate at the first bit of the window and between any two candidates, as chance magics
+// inside compressed data would be
+void add_chance_candidates(std::vector<u64> &cand) {
+    std::vector<u64> add;
+    if (cand.empty() || (cand[0] & ~FOOT_BIT) != 0) add.push_back(0);
+    for (size_t i = 0; i + 1 < cand.size(); i++) {
+        u64 a = cand[i] & ~FOOT_BIT, b = cand[i + 1] & ~FOOT_BIT;
+        if (b - a >= 2) add.push_back((a + b) / 2);
+    }
+    cand.insert(cand.end(), add.begin(), add.end());
+    std::sort(cand.begin(), cand.end(), [](u64 x, u64 y) { return (x & ~FOOT_BIT) < (y & ~FOOT_BIT); });
+}
+
+int run_dec_window(bz2b200_mctx *m, int r, size_t k, int slot) {
+    MRank &R = *m->rk[r];
+    MWin &W = *m->win[k];
+    bz2b200_ctx *ctx = R.ctx;
+    const size_t nwin = m->win.size();
+    const size_t len = R.posted_len[slot];
+    u8 *d = R.d_win[slot].as<u8>();
+    const bool chance = getenv("BZ2B200_MULTI_DEC_CHANCE") != nullptr;
+    auto t0 = clk::now();
+    WinSink sink;
+    sink.m = m; sink.R = &R; sink.W = &W; sink.k = k; sink.ctx = ctx;
+    int rc;
+    double t_scan;
+    {
+        std::lock_guard<std::mutex> lk(ctx->mu);
+        ctx->err.clear();
+        MCHECK(cudaStreamWaitEvent(ctx->stream, W.ev_up, 0));
+        MCHECK(cudaMemsetAsync(d + len, 0, 64, ctx->stream));  // word loads of the entropy stage read past the last byte
+        std::vector<u64> cand;
+        // at most one magic per 32 bits whatever the data: a window is never refused where the whole input is accepted
+        rc = bz_dec_candidates(ctx, d, len, (u32)std::min<size_t>(len / 4 + 64, 0x7fffff00u), cand);
+        t_scan = ms_since(t0);
+        if (!rc) {
+            if (chance) add_chance_candidates(cand);
+            // level-9 geometry: the headers of later windows are not known yet; the calling thread applies the block
+            // size they allow
+            DecWindow w{m->in, m->nbytes, d, W.lo, len, k + 1 == nwin ? ~0ull : (u64)W.hi * 8, k == 0 ? 32ll : -1ll,
+                        BZ2B200_MAX_BLOCK, &cand};
+            rc = bz_decode_core(ctx, w, sink, W.events);
+        }
+    }
+    R.t_scan += t_scan; R.t_wait += sink.t_wait; R.t_d2h += sink.t_out;
+    R.t_comp += ms_since(t0) - t_scan - sink.t_wait - sink.t_out;
+    if (rc) {
+        W.rc = rc;
+        if (rc != DEC_ABORTED) W.err = ctx->err;
+        m->abort.store(1);
+        return rc;
+    }
+    W.len_pub.store((long long)W.out_len, std::memory_order_release);
+    return BZ2B200_OK;
+}
+
+int run_dec_windows(bz2b200_mctx *m, int r) {
+    MRank &R = *m->rk[r];
+    MCHECK(cudaSetDevice(R.ctx->device));
+    if (!R.ev_shift) MCHECK(cudaEventCreateWithFlags(&R.ev_shift, cudaEventDisableTiming));
+    const size_t N = (size_t)m->n, nwin = m->win.size();
+    if ((size_t)r < nwin) { int rc = post_window(m, r, (size_t)r, 0, 0); if (rc) return rc; }
+    size_t i = 0;
+    for (size_t k = (size_t)r; k < nwin; k += N, i++) {
+        if (k + N < nwin) { int rc = post_window(m, r, k + N, (int)((i + 1) & 1), i + 1); if (rc) return rc; }   // arrives under this window's kernels
+        int rc = run_dec_window(m, r, k, (int)(i & 1));
+        if (rc) return rc;
+    }
+    return BZ2B200_OK;
+}
+
+int run_dec_rank(bz2b200_mctx *m, int r) {
+    MRank &R = *m->rk[r];
+    R.rc = 0; R.err.clear(); R.h2d = R.d2h = 0; R.nblk = 0; R.ndec = 0;
+    R.t_scan = R.t_chain = R.t_comp = R.t_wait = R.t_d2h = 0;
+    int rc;
+    try { rc = run_dec_windows(m, r); } catch (...) { rc = BZ2B200_E_NOMEM; R.rc = rc; R.err = "out of memory"; m->abort.store(1); }
+    // whatever failed: no copy from `in` or into `out` may still run when the call returns
+    bz2b200_ctx *ctx = R.ctx;
+    cudaSetDevice(ctx->device);
+    if (ctx->s_up) cudaStreamSynchronize(ctx->s_up);
+    if (ctx->s_hi) cudaStreamSynchronize(ctx->s_hi);
+    cudaStreamSynchronize(ctx->stream);
+    if (ctx->s_down) cudaStreamSynchronize(ctx->s_down);
+    return rc;
+}
+
 void worker(bz2b200_mctx *m, int r) {
     u64 seen = 0;
     for (;;) {
@@ -278,7 +436,7 @@ void worker(bz2b200_mctx *m, int r) {
             seen = m->seq;
         }
         int rc;
-        try { rc = run_rank(m, r); } catch (...) { rc = BZ2B200_E_NOMEM; m->rk[r]->rc = rc; m->rk[r]->err = "out of memory"; m->abort.store(1); }
+        try { rc = m->decode ? run_dec_rank(m, r) : run_rank(m, r); } catch (...) { rc = BZ2B200_E_NOMEM; m->rk[r]->rc = rc; m->rk[r]->err = "out of memory"; m->abort.store(1); }
         (void)rc;                                               // a failed rank has raised the abort flag: nobody waits for it
         {
             std::lock_guard<std::mutex> lk(m->mu);
@@ -357,6 +515,7 @@ int bz2b200_compress_stream_multi(bz2b200_mctx *m, const uint8_t *in, size_t n, 
     if (out_cap < 64) return BZ2B200_E_CAP;
     auto t0 = clk::now();
     m->in = in; m->nbytes = n; m->level = level; m->out = out; m->out_cap = out_cap;
+    m->decode = false;
     m->abort.store(0);
     {   // windows: a multiple of n_devices, at most 256 MiB each, whole 4 KiB pages
         // Two windows per rank when a window still holds 32 MiB: nothing can be compressed before a rank's first window is on
@@ -435,6 +594,100 @@ int bz2b200_compress_stream_multi(bz2b200_mctx *m, const uint8_t *in, size_t n, 
                     R.t_scan, R.t_wait, R.t_chain, R.t_comp, R.t_d2h, (unsigned)R.nblk);
         }
     }
+    return BZ2B200_OK;
+    BZ_API_CATCH
+}
+
+int bz2b200_decompress_stream_multi(bz2b200_mctx *m, const uint8_t *in, size_t n, uint8_t *out, size_t out_cap,
+                                    size_t *out_len) {
+    BZ_API_TRY
+    if (!m || !in || !out_len || (!out && out_cap) || n < 14 || n > 0xFFFFFF00ull * 4ull) return BZ2B200_E_ARG;
+    if (in[0] != 'B' || in[1] != 'Z' || in[2] != 'h' || in[3] < '1' || in[3] > '9') return BZ2B200_E_FORMAT;
+    std::lock_guard<std::mutex> call(m->call_mu);
+    *out_len = 0;
+    size_t win = std::min(DEC_WIN_MAX, std::max(DEC_WIN_MIN, ((n + 2 * (size_t)m->n - 1) / (2 * (size_t)m->n) + 4095) & ~(size_t)4095));
+    if (const char *e = getenv("BZ2B200_MULTI_DEC_WINDOW")) { long long v = atoll(e); if (v >= 1024) win = (size_t)v; }
+    // small inputs (or one device): the single-GPU path
+    if (m->n == 1 || n < 2 * win) {
+        int rc = bz2b200_decompress_stream(m->rk[0]->ctx, in, n, out, out_cap, out_len);
+        // That call stops at the first batch that does not fit; the caller is owed the exact size, so the input is decoded
+        // again into scratch memory (growing twofold while it does not fit) to learn it.  A defect behind the point where
+        // the first call stopped does not change the code: it stays E_CAP, with the size the first call reported.
+        const size_t first_len = *out_len;
+        for (std::vector<u8> tmp; rc == BZ2B200_E_CAP;) {
+            tmp.resize(std::max<size_t>(2 * *out_len, 1 << 20));
+            rc = bz2b200_decompress_stream(m->rk[0]->ctx, in, n, tmp.data(), tmp.size(), out_len);
+            if (rc == BZ2B200_OK) { rc = BZ2B200_E_CAP; break; }
+            if (rc != BZ2B200_E_CAP) { rc = BZ2B200_E_CAP; *out_len = first_len; break; }
+        }
+        if (rc) m->err = bz2b200_last_error(m->rk[0]->ctx);
+        m->stat[0] = n; m->stat[1] = rc ? 0 : *out_len;
+        return rc;
+    }
+    auto t0 = clk::now();
+    m->in = in; m->nbytes = n; m->out = out; m->out_cap = out_cap;
+    m->decode = true;
+    m->abort.store(0);
+    m->win.clear();
+    for (size_t lo = 0; lo < n; lo += win) {
+        m->win.emplace_back(new MWin());
+        m->win.back()->lo = lo;
+        m->win.back()->hi = std::min(n, lo + win);
+    }
+    {
+        std::lock_guard<std::mutex> lk(m->mu);
+        m->done = 0;
+        m->seq++;
+    }
+    m->cv_job.notify_all();
+    {
+        std::unique_lock<std::mutex> lk(m->mu);
+        m->cv_done.wait(lk, [&] { return m->done == m->n; });
+    }
+    u64 h2d = 0, d2h = 0;
+    for (auto &R : m->rk) { h2d += R->h2d; d2h += R->d2h; }
+    m->stat[0] = h2d; m->stat[1] = d2h;
+    if (getenv("BZ2B200_MULTI_TRACE")) {
+        fprintf(stderr, "[multi decode] total %.2f ms, %zu windows of %zu bytes\n", ms_since(t0), m->win.size(), win);
+        for (int r = 0; r < m->n; r++) {
+            MRank &R = *m->rk[r];
+            fprintf(stderr, "[multi decode rank %d] upload+magics %.2f chain wait %.2f decode %.2f offsets+d2h %.2f ms\n", r,
+                    R.t_scan, R.t_wait, R.t_comp, R.t_d2h);
+        }
+    }
+    // ---- ordered fan-in: the first error in chain order wins; combined CRCs; block size the headers allow ----
+    // Every block is bounded by 100000 x the largest level among the first header and every header after a footer on
+    // the chain (windows decode with level-9 buffers).  bz2b200_decompress_stream takes the maximum over every footer
+    // magic followed by "BZh<level>", chance ones inside compressed data included; the two differ only where such a
+    // chance footer is followed by a larger level digit.  With several defects in one input the
+    // code returned may be E_FORMAT where the single-GPU call returns E_CRC or the reverse.
+    int level = in[3] - '0';
+    for (auto &W : m->win)
+        for (const DecEvent &e : W->events) if (e.kind == DEC_STREAM) level = std::max(level, (int)e.val);
+    const u32 max_block = (u32)level * 100000u;
+    u32 combined = 0;
+    bool fold = true;                                           // `combined` covers the whole stream so far
+    u64 total = 0;
+    for (auto &W : m->win) {
+        for (const DecEvent &e : W->events) {
+            if (e.kind == DEC_BLOCK) {
+                if (e.nblock > max_block) { m->err = "decode: block at bit " + std::to_string(e.bit) + " longer than its stream's level allows"; return BZ2B200_E_FORMAT; }
+                combined = crc_step(combined, e.val);
+            } else if (e.kind == DEC_FOOTER) {
+                if (fold && e.val != combined) { m->err = "decode: combined CRC mismatch at bit " + std::to_string(e.bit); return BZ2B200_E_CRC; }
+            } else {
+                combined = 0; fold = true;
+            }
+        }
+        if (W->rc < 0) { m->err = W->err; return W->rc; }
+        if (W->rc) fold = false;                                // stopped early: its events are incomplete
+        total += W->out_len;
+    }
+    for (auto &R : m->rk) if (R->rc) { m->err = "rank failed: " + R->err; return R->rc; }
+    for (auto &W : m->win) if (W->rc) { m->err = "decode: a window stopped without an error"; return BZ2B200_E_CUDA; }
+    if (m->win.back()->chain_out != DEC_ENDED) { m->err = "decode: the input does not end with a stream footer"; return BZ2B200_E_FORMAT; }
+    *out_len = (size_t)total;
+    if (total > out_cap) { m->err = "output buffer too small"; return BZ2B200_E_CAP; }
     return BZ2B200_OK;
     BZ_API_CATCH
 }

@@ -157,6 +157,19 @@ int  bz2b200_multi_devices(const bz2b200_mctx *m);
 bz2b200_ctx *bz2b200_multi_context(bz2b200_mctx *m, int rank);
 int  bz2b200_compress_stream_multi(bz2b200_mctx *m, const uint8_t *in, size_t n, int level,
                                    uint8_t *out, size_t out_cap, size_t *out_len);
+/* decompress (src/compression/decompress.rs:38) on the same GPUs: the input bz2b200_decompress_stream accepts (several
+ * streams one after the other, any levels, legacy randomised blocks) is cut into byte windows dealt round robin (about
+ * 24 MiB each; each is uploaded with 4 MiB of look-ahead, enough for the longest block that can start in it).  A GPU
+ * finds the block magics of its window and entropy-decodes them while the block chain arrives from the window before as
+ * one number through host memory; it hands the chain on before its inverse BWT, and copies every decoded batch over
+ * its own PCIe link straight to its place in `out` once the lengths of the windows before it are known.  The calling
+ * thread checks every stream's combined CRC and the block size its headers allow; block CRCs are checked on the GPUs.
+ * `out` receives exactly the bytes bz2b200_decompress_stream produces.  Return codes: those of
+ * bz2b200_decompress_stream for an input with a single defect; with several defects E_FORMAT and E_CRC may be
+ * swapped.  On BZ2B200_E_CAP, *out_len holds the exact decompressed size.  Inputs smaller than two windows are
+ * decoded by bz2b200_decompress_stream on the first GPU.  One call at a time per multi context. */
+int  bz2b200_decompress_stream_multi(bz2b200_mctx *m, const uint8_t *in, size_t n,
+                                     uint8_t *out, size_t out_cap, size_t *out_len);
 /* last call: [0] = bytes copied host -> device (all GPUs), [1] = device -> host */
 int  bz2b200_multi_stats(const bz2b200_mctx *m, uint64_t st[8]);
 

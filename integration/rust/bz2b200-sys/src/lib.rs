@@ -67,6 +67,8 @@ extern "C" {
     pub fn bz2b200_multi_context(m: *mut bz2b200_mctx, rank: c_int) -> *mut bz2b200_ctx;
     pub fn bz2b200_compress_stream_multi(m: *mut bz2b200_mctx, input: *const u8, n: usize, level: c_int,
         out: *mut u8, out_cap: usize, out_len: *mut usize) -> c_int;
+    pub fn bz2b200_decompress_stream_multi(m: *mut bz2b200_mctx, input: *const u8, n: usize, out: *mut u8,
+        out_cap: usize, out_len: *mut usize) -> c_int;
     pub fn bz2b200_multi_stats(m: *const bz2b200_mctx, st: *mut u64) -> c_int;
     // ---- stage seams (one per reference function) ----
     pub fn bz2b200_crc32(ctx: *mut bz2b200_ctx, data: *const u8, n: usize, crc: *mut u32) -> c_int;
