@@ -40,6 +40,7 @@ EXPORTS = [
     "bz2b200_create_multi", "bz2b200_destroy_multi", "bz2b200_last_error_multi", "bz2b200_multi_devices",
     "bz2b200_multi_context", "bz2b200_compress_stream_multi", "bz2b200_decompress_stream_multi", "bz2b200_multi_stats",
     "bz2b200_zstream_open", "bz2b200_zstream_write", "bz2b200_zstream_close",
+    "bz2b200_dstream_open", "bz2b200_dstream_write", "bz2b200_dstream_close",
 ]
 
 
@@ -121,6 +122,9 @@ def load_library():
     L.bz2b200_zstream_open.argtypes = [vp, C.c_int, SINK, vp, C.POINTER(vp)]
     L.bz2b200_zstream_write.argtypes = [vp, u8p, C.c_size_t]
     L.bz2b200_zstream_close.argtypes = [vp, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]
+    L.bz2b200_dstream_open.argtypes = [vp, SINK, vp, C.POINTER(vp)]
+    L.bz2b200_dstream_write.argtypes = [vp, u8p, C.c_size_t]
+    L.bz2b200_dstream_close.argtypes = [vp, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]
     _lib = L
     return L
 
@@ -437,6 +441,67 @@ class ZStream:
             raise self._err
         if rc != OK:
             raise Bz2B200Error(rc, self._L.bz2b200_last_error(self._eng._h).decode())
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+        return False
+
+
+class DStream:
+    """Streaming decompression (bz2b200_dstream_*): write() .bz2 input in pieces; checked output goes to `out.write`
+    (called on a library thread, in order).  out=None is test mode (bzip2 -t): every check runs, nothing is downloaded,
+    total_out still counts the decoded bytes.
+
+        with DStream(engine, fileobj) as d:
+            for piece in pieces: d.write(piece)
+    """
+
+    def __init__(self, engine, out=None):
+        self._L = engine._L
+        self._eng = engine
+        self._out = out
+        self._err = None
+        self._h = None
+        self.total_in = self.total_out = 0
+        self._cb = SINK()                   # a NULL sink: test mode
+        if out is not None:
+            def sink(_user, data, n):
+                try:
+                    self._out.write(C.string_at(data, n))
+                    return 0
+                except BaseException as e:  # an exception must not unwind through the C library
+                    self._err = e
+                    return 1
+            self._cb = SINK(sink)           # keep the callback object alive as long as the stream
+        h = C.c_void_p()
+        rc = self._L.bz2b200_dstream_open(engine._h, self._cb, None, C.byref(h))
+        if rc != OK:
+            raise Bz2B200Error(rc, "bz2b200_dstream_open")
+        self._h = h
+
+    def _raise(self, rc):
+        if self._err is not None:
+            raise self._err
+        raise Bz2B200Error(rc, self._L.bz2b200_last_error(self._eng._h).decode())
+
+    def write(self, data):
+        a = _np_u8(data)
+        rc = self._L.bz2b200_dstream_write(self._h, a.ctypes.data, a.size)
+        if rc != OK:
+            self._raise(rc)
+
+    def close(self):
+        if self._h is None:
+            return
+        ti, to = C.c_uint64(), C.c_uint64()
+        rc = self._L.bz2b200_dstream_close(self._h, C.byref(ti), C.byref(to))
+        self._h = None
+        self.total_in, self.total_out = ti.value, to.value
+        if self._err is not None or rc != OK:
+            self._raise(rc)
 
     def __enter__(self):
         return self

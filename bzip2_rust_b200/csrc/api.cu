@@ -10,7 +10,7 @@ static void release_device_buffers(bz2b200_ctx *c) {
                      &c->d_VALB, &c->d_thist, &c->d_tagg, &c->d_cnt, &c->d_bwt, &c->d_key, &c->d_mtfstate, &c->d_chunkrec, &c->d_R,
                      &c->d_sym, &c->d_m, &c->d_freq, &c->d_used, &c->d_agg2, &c->d_len6, &c->d_rfreq, &c->d_sel, &c->d_gbits,
                      &c->d_hdr, &c->d_bitoff, &c->d_out, &c->d_outbits, &c->d_hmisc, &c->d_in, &c->d_runflag, &c->d_misc,
-                     &c->d_stream, &c->d_dec1, &c->d_dec2, &c->d_dec3};
+                     &c->d_stream, &c->d_dec1, &c->d_dec2, &c->d_dec3, &c->d_dwin, &c->d_ddec[0], &c->d_ddec[1]};
     for (DevBuf *b : all) b->release();
 }
 
@@ -27,6 +27,7 @@ bz2b200_ctx::~bz2b200_ctx() {
     cudaSetDevice(device);
     release_device_buffers(this);
     h_stage.release(); h_small.release(); h_out.release();
+    for (int i = 0; i < 2; i++) { h_dstage[i].release(); h_dpiece[i].release(); }
     for (int i = 0; i < 8; i++) if (ev[i]) cudaEventDestroy(ev[i]);
     for (int i = 0; i < 2; i++) if (ev_dec[i]) cudaEventDestroy(ev_dec[i]);
     if (s_hi) cudaStreamDestroy(s_hi);

@@ -132,6 +132,10 @@ struct bz2b200_ctx {
     DevBuf d_len6, d_rfreq, d_sel, d_gbits, d_hdr, d_bitoff, d_out, d_outbits, d_hmisc;
     // ---- stream / rle1 / decode ----
     DevBuf d_in, d_runflag, d_misc, d_stream, d_dec1, d_dec2, d_dec3;
+    // ---- dstream (dstream.cu): window, batch outputs, staging and output pieces, kept for the next stream ----
+    DevBuf d_dwin, d_ddec[2];
+    PinBuf h_dstage[2], h_dpiece[2];
+    bool dstream_open = false;       // one dstream at a time uses them
 
     // ---- per-kernel profiling (timing level 2): CUDA events around every launch ----
     KStat kstat[K_COUNT];
@@ -285,7 +289,7 @@ int bz_compress_batch(bz2b200_ctx *ctx, const Batch &B, const u32 *d_crc, HufOut
 int bz_contexts_on_device(int device);
 std::mutex &bz_device_lock(int device);
 
-// ---- decode.cu: the decode core shared by bz2b200_decompress_stream and bz2b200_decompress_stream_multi ----
+// ---- decode.cu: the decode core shared by bz2b200_decompress_stream, bz2b200_decompress_stream_multi and the dstream ----
 // It decodes the chain of blocks and footers that starts in bits [8*lo, hi_bit) of the input; the device holds bytes
 // [lo, lo + len) of it, followed by 64 zero bytes.  Bit positions it reports are absolute (from the input's start).
 enum { DEC_BLOCK = 0, DEC_FOOTER = 1, DEC_STREAM = 2 };
@@ -311,12 +315,16 @@ struct DecSink {
     virtual ~DecSink() {}
 };
 struct DecWindow {
-    const u8 *in; size_t n;        // the whole input, host
+    const u8 *in; size_t in_lo, n; // host bytes [in_lo, n) of the input, in[0] = byte in_lo; n = the input's end when
+                                   // the window is the last one (a footer whose header byte would be n ends the input)
     const u8 *d_win; size_t lo, len;
     u64 hi_bit;                    // elements from here on belong to the next window (~0: none)
     long long expect;              // absolute bit of the first element, -1 = ask DecSink::chain_start
+    u32 combined;                  // running combined CRC of the stream at `expect` (when expect >= 0)
     u32 max_block;                 // buffers and bounds of every block
     const std::vector<u64> *cand;  // candidate bits relative to d_win, sorted by position, bit 63 = footer magic
 };
 int bz_dec_candidates(bz2b200_ctx *ctx, const u8 *d_win, size_t len, u32 cap, std::vector<u64> &cand);
+// test knob BZ2B200_MULTI_DEC_CHANCE: spurious block candidates, as chance magics inside compressed data would be
+void bz_add_chance_candidates(std::vector<u64> &cand);
 int bz_decode_core(bz2b200_ctx *ctx, const DecWindow &w, DecSink &sink, std::vector<DecEvent> &ev);

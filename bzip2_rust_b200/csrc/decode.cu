@@ -363,6 +363,19 @@ int bz_dec_candidates(bz2b200_ctx *ctx, const u8 *d_win, size_t len, u32 cap, st
     return BZ2B200_OK;
 }
 
+// test knob: a spurious block candidate at the first bit of the window and between any two candidates, as chance magics
+// inside compressed data would be
+void bz_add_chance_candidates(std::vector<u64> &cand) {
+    std::vector<u64> add;
+    if (cand.empty() || (cand[0] & ~FOOT) != 0) add.push_back(0);
+    for (size_t i = 0; i + 1 < cand.size(); i++) {
+        u64 a = cand[i] & ~FOOT, b = cand[i + 1] & ~FOOT;
+        if (b - a >= 2) add.push_back((a + b) / 2);
+    }
+    cand.insert(cand.end(), add.begin(), add.end());
+    std::sort(cand.begin(), cand.end(), [](u64 x, u64 y) { return (x & ~FOOT) < (y & ~FOOT); });
+}
+
 // A magic can also occur by chance inside entropy-coded data, and a file may hold several streams one after the other
 // (decompress.rs handles neither; libbz2 walks the blocks serially and accepts both).  So the candidates are only where
 // blocks MAY start: the chain is walked from every decoded block's end, candidates off the chain are dropped, and a
@@ -415,14 +428,14 @@ int bz_decode_core(bz2b200_ctx *ctx, const DecWindow &w, DecSink &sink, std::vec
     auto read32 = [&](u64 bit) {                                // 32 bits at an absolute bit offset of the host input
         size_t byte = (size_t)(bit >> 3); int sh = (int)(bit & 7);
         u64 v = 0;
-        for (int k = 0; k < 5; k++) v = (v << 8) | (byte + k < w.n ? w.in[byte + k] : 0);
+        for (int k = 0; k < 5; k++) v = (v << 8) | (byte + k < w.n ? w.in[byte + k - w.in_lo] : 0);
         return (u32)((v >> (8 - sh)) & 0xffffffffull);
     };
     size_t ci = 0;                                              // next candidate to look at
     bool known = w.expect >= 0;                                 // the chain start is known
     u64 expect = known ? (u64)w.expect - lo8 : 0;               // bit offset where the next block / footer must start
     bool comb_known = known;                                    // the window has seen the start of the current stream
-    u32 combined = 0;                                           // running combined CRC of the current stream
+    u32 combined = known ? w.combined : 0;                      // running combined CRC of the current stream
     bool have_batch = false;                                    // `starts` were decoded before the chain start was known
     std::vector<u64> starts, rends;
     const u64 range_limit = [] { const char *e = getenv("BZ2B200_DEC_RANGE_LIMIT"); return e ? (u64)strtoull(e, nullptr, 10) : 0ull; }();
@@ -440,11 +453,11 @@ int bz_decode_core(bz2b200_ctx *ctx, const DecWindow &w, DecSink &sink, std::vec
                 if (comb_known && stored != combined) return BZ2B200_E_CRC;                    // enforced, unlike decompress.rs:394-402
                 size_t hb = (size_t)((expect + lo8 + 80 + 7) / 8);
                 if (hb == w.n) { sink.chain_end(DEC_ENDED); return BZ2B200_OK; }
-                const u8 *in = w.in;
-                if (hb + 4 > w.n || in[hb] != 'B' || in[hb + 1] != 'Z' || in[hb + 2] != 'h' || in[hb + 3] < '1' || in[hb + 3] > '9') {
+                const u8 *in = hb + 4 <= w.n ? w.in + (hb - w.in_lo) : nullptr;   // hb > the footer's first byte >= in_lo
+                if (!in || in[0] != 'B' || in[1] != 'Z' || in[2] != 'h' || in[3] < '1' || in[3] > '9') {
                     ctx->err = "decode: trailing bytes after the stream footer"; return BZ2B200_E_FORMAT;
                 }
-                ev.push_back(DecEvent{(u64)hb * 8, (u32)(in[hb + 3] - '0'), 0, DEC_STREAM});
+                ev.push_back(DecEvent{(u64)hb * 8, (u32)(in[3] - '0'), 0, DEC_STREAM});
                 combined = 0; comb_known = true;
                 expect = (u64)hb * 8 + 32 - lo8;
                 continue;
@@ -647,7 +660,7 @@ extern "C" int bz2b200_decompress_stream(bz2b200_ctx *ctx, const uint8_t *in, si
         if (hb + 4 <= n && in[hb] == 'B' && in[hb + 1] == 'Z' && in[hb + 2] == 'h' && in[hb + 3] >= '1' && in[hb + 3] <= '9')
             level = std::max(level, in[hb + 3] - '0');
     }
-    DecWindow w{in, n, ctx->d_in.as<u8>(), 0, n, ~0ull, 32, (u32)level * 100000u, &cand};
+    DecWindow w{in, 0, n, ctx->d_in.as<u8>(), 0, n, ~0ull, 32, 0, (u32)level * 100000u, &cand};
     WholeSink sink;
     sink.ctx = ctx; sink.out = out; sink.out_cap = out_cap; sink.out_len = out_len;
     std::vector<DecEvent> ev;

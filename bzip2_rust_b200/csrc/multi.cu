@@ -117,7 +117,6 @@ int rank_fail(bz2b200_mctx *m, MRank &R, int rc, const char *what) {
 #define MCHECK(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { R.rc = BZ2B200_E_CUDA; R.err = std::string(#call) + ": " + cudaGetErrorString(e_); m->abort.store(1); return R.rc; } } while (0)
 
 const size_t LOOK0 = 4u << 20;               // look-ahead for the last block of a window, grown on demand
-constexpr u64 FOOT_BIT = 1ull << 63;          // a decoder candidate that is a footer magic
 inline size_t chunk_bytes() {
     static const size_t c = [] { const char *e = getenv("BZ2B200_E2E_CHUNK_MB"); int v = e ? atoi(e) : 8; return (size_t)(v < 1 ? 1 : v) << 20; }();
     return c;
@@ -339,19 +338,6 @@ struct WinSink : DecSink {
     }
 };
 
-// test knob: a spurious block candidate at the first bit of the window and between any two candidates, as chance magics
-// inside compressed data would be
-void add_chance_candidates(std::vector<u64> &cand) {
-    std::vector<u64> add;
-    if (cand.empty() || (cand[0] & ~FOOT_BIT) != 0) add.push_back(0);
-    for (size_t i = 0; i + 1 < cand.size(); i++) {
-        u64 a = cand[i] & ~FOOT_BIT, b = cand[i + 1] & ~FOOT_BIT;
-        if (b - a >= 2) add.push_back((a + b) / 2);
-    }
-    cand.insert(cand.end(), add.begin(), add.end());
-    std::sort(cand.begin(), cand.end(), [](u64 x, u64 y) { return (x & ~FOOT_BIT) < (y & ~FOOT_BIT); });
-}
-
 int run_dec_window(bz2b200_mctx *m, int r, size_t k, int slot) {
     MRank &R = *m->rk[r];
     MWin &W = *m->win[k];
@@ -375,11 +361,11 @@ int run_dec_window(bz2b200_mctx *m, int r, size_t k, int slot) {
         rc = bz_dec_candidates(ctx, d, len, (u32)std::min<size_t>(len / 4 + 64, 0x7fffff00u), cand);
         t_scan = ms_since(t0);
         if (!rc) {
-            if (chance) add_chance_candidates(cand);
+            if (chance) bz_add_chance_candidates(cand);
             // level-9 geometry: the headers of later windows are not known yet; the calling thread applies the block
             // size they allow
-            DecWindow w{m->in, m->nbytes, d, W.lo, len, k + 1 == nwin ? ~0ull : (u64)W.hi * 8, k == 0 ? 32ll : -1ll,
-                        BZ2B200_MAX_BLOCK, &cand};
+            DecWindow w{m->in, 0, m->nbytes, d, W.lo, len, k + 1 == nwin ? ~0ull : (u64)W.hi * 8, k == 0 ? 32ll : -1ll,
+                        0, BZ2B200_MAX_BLOCK, &cand};
             rc = bz_decode_core(ctx, w, sink, W.events);
         }
     }

@@ -135,6 +135,33 @@ int bz2b200_zstream_open(bz2b200_ctx *ctx, int level, bz2b200_sink sink, void *u
 int bz2b200_zstream_write(bz2b200_zstream *z, const uint8_t *data, size_t n);
 int bz2b200_zstream_close(bz2b200_zstream *z, uint64_t *total_in, uint64_t *total_out);
 
+/* ---- seam: decompress (src/compression/decompress.rs:38) as a pipeline: the input arrives in pieces ------------- */
+/* bzip2 -d / -t in bounded memory on an input of any size.  bz2b200_dstream_write copies the caller's bytes into
+ * page-locked staging (windows of 64 MiB); a worker thread uploads a full window behind the bytes carried from the one
+ * before and decodes the blocks that start before its last 4 MiB; a delivery thread downloads every checked batch in
+ * pieces of 32 MiB and calls `sink` on one piece while the next downloads and the next batch decodes.
+ *   Input: whatever bz2b200_decompress_stream accepts (one or more streams back to back, any levels, legacy
+ *   randomised blocks).  Output: the sink receives exactly the bytes bz2b200_decompress_stream produces, in order, on
+ *   one library thread (neither the caller's nor the decode worker's), for any piece sizes the caller writes.
+ *   Every byte the sink receives has passed its block CRC; a stream's combined CRC is checked when its footer is
+ *   reached; so after an error the sink has received a prefix of the correct output.
+ *   sink == NULL is test mode (bzip2 -t): every check runs, decoded bytes stay on the device, total_out counts them.
+ *   Errors are sticky: the next write or the close returns them.  For an input with a single defect the code is the
+ *   one bz2b200_decompress_stream returns for the same bytes (E_FORMAT or E_CRC), except that an input shorter than
+ *   14 bytes gives E_FORMAT at close (a stream cannot know its length when it opens).  A sink returning non-zero
+ *   aborts with E_ARG ("the sink reported an error").  There is no E_CAP.
+ *   bz2b200_dstream_close decodes what is left, waits for the sink to finish, fails with E_FORMAT if the input does
+ *   not end with a stream footer, and frees the stream (also after an error); on an error bz2b200_last_error(ctx)
+ *   says "dstream: ...".
+ * Host memory is a constant (staging and output pieces, about 200 MB) whatever the input and output sizes; these
+ * buffers stay with the context for its next dstream.  One dstream at a time per context (a second open returns
+ * E_ARG), and the context must not be used by other threads while a dstream is open on it (calls are serialised, so
+ * they would only wait). */
+typedef struct bz2b200_dstream bz2b200_dstream;
+int bz2b200_dstream_open(bz2b200_ctx *ctx, bz2b200_sink sink, void *user, bz2b200_dstream **out);
+int bz2b200_dstream_write(bz2b200_dstream *d, const uint8_t *data, size_t n);
+int bz2b200_dstream_close(bz2b200_dstream *d, uint64_t *total_in, uint64_t *total_out);
+
 /* ---- seam: compress (src/compression/compress.rs:40-136) on SEVERAL GPUs of one process -------------------- */
 /* The reference fans blocks out to rayon workers (compress.rs:125-132) and a writer thread puts them back in
  * order (compress.rs:74-122).  A multi context owns n_devices single-GPU contexts and one host thread per GPU

@@ -6,6 +6,7 @@ use std::os::raw::{c_char, c_int, c_void};
 #[repr(C)] pub struct bz2b200_ctx { _private: [u8; 0] }
 #[repr(C)] pub struct bz2b200_mctx { _private: [u8; 0] }
 #[repr(C)] pub struct bz2b200_zstream { _private: [u8; 0] }
+#[repr(C)] pub struct bz2b200_dstream { _private: [u8; 0] }
 pub type bz2b200_sink = Option<unsafe extern "C" fn(user: *mut c_void, data: *const u8, n: usize) -> c_int>;
 
 pub const BZ2B200_OK: c_int = 0;
@@ -59,6 +60,11 @@ extern "C" {
         out: *mut *mut bz2b200_zstream) -> c_int;
     pub fn bz2b200_zstream_write(z: *mut bz2b200_zstream, data: *const u8, n: usize) -> c_int;
     pub fn bz2b200_zstream_close(z: *mut bz2b200_zstream, total_in: *mut u64, total_out: *mut u64) -> c_int;
+    // ---- seam: decompress as a pipeline: pieces in, checked bytes to a sink (None: test mode) ----
+    pub fn bz2b200_dstream_open(ctx: *mut bz2b200_ctx, sink: bz2b200_sink, user: *mut c_void,
+        out: *mut *mut bz2b200_dstream) -> c_int;
+    pub fn bz2b200_dstream_write(d: *mut bz2b200_dstream, data: *const u8, n: usize) -> c_int;
+    pub fn bz2b200_dstream_close(d: *mut bz2b200_dstream, total_in: *mut u64, total_out: *mut u64) -> c_int;
     // ---- seam: compress on several GPUs of one process ----
     pub fn bz2b200_create_multi(n_devices: c_int, device_ids: *const c_int, out: *mut *mut bz2b200_mctx) -> c_int;
     pub fn bz2b200_destroy_multi(m: *mut bz2b200_mctx);

@@ -1,12 +1,19 @@
 """Decode rate of the stream bench.py compresses in its `e2e` leg, so that compress and decompress rates compare.
 
-    python tools/bench_decode.py --gpus 1 2 4 8 [--steps K] [--warmup W] [--size-mb 100]
+    python tools/bench_decode.py --gpus 1 2 4 8 [--steps K] [--warmup W] [--size-mb 100] [--dstream]
 
 Workload for world N: corpus.text(size_mb * 10^6, seed 2 + r) for r < N, concatenated, compressed at -9.  Pinned host
 buffers; W warm-up calls, then K calls timed with a host clock around each call (a call returns when its output is in
 host memory).  N = 1 times bz2b200_decompress_stream, N > 1 bz2b200_decompress_stream_multi on devices
 0..N-1 (modulo the visible devices: `distinct_gpus` says how many GPUs the ranks really had).  The output is compared
 with the input after the timed calls.  One JSON line per world size.
+
+--dstream adds two arms for world 1, timed in turn with the one-call arm (one-call, dstream, test mode, one-call, ...)
+on the same workload: "decode_dstream" writes the pinned compressed stream into a bz2b200_dstream in pieces of 16 MiB
+and its sink memmoves every piece into a pinned output buffer at a running offset; "decode_test" does the same in test
+mode (no sink, nothing downloaded).  Both are timed with a host clock from open to close.  The dstream's output is
+compared with the input after the timed calls, and test mode's total_out with the input's size.  They print one JSON
+line each after the one-call arm's.
 """
 import argparse
 import ctypes as C
@@ -53,6 +60,9 @@ def run(world, args, eng, info):
     in_ptr, out_ptr, cap = h_in.ctypes.data, h_out.ctypes.data, h_out.size
     ndev = torch.cuda.device_count()
     m = None
+    arms = []
+    if world == 1 and args.dstream:
+        arms = dstream_arms(eng, h_in, len(s), data.size)
     if world == 1:
         L, ln = eng._L, C.c_size_t()
 
@@ -68,11 +78,17 @@ def run(world, args, eng, info):
             return m.decompress_into(in_ptr, len(s), out_ptr, cap)
     for _ in range(args.warmup):
         call()
+        for arm in arms:
+            arm["call"]()
     times = []
     for _ in range(args.steps):
         t0 = time.perf_counter()
         n = call()
         times.append(time.perf_counter() - t0)
+        for arm in arms:
+            t0 = time.perf_counter()
+            arm["n"] = arm["call"]()
+            arm["times"].append(time.perf_counter() - t0)
     ok = n == data.size and np.array_equal(h_out[:n], data)
     st = m.stats() if m else {"h2d_bytes": len(s), "d2h_bytes": n}
     if m:
@@ -85,7 +101,53 @@ def run(world, args, eng, info):
            "library": os.environ.get("BZ2B200_LIB", "bzip2_rust_b200/libbz2b200.so")}
     rec.update(info)
     print(json.dumps(rec), flush=True)
+    for arm in arms:
+        a_ok = arm["n"] == data.size and (arm["out"] is None or np.array_equal(arm["out"][:data.size], data))
+        ms = 1e3 * float(np.median(arm["times"]))
+        r = {"metric": arm["metric"], "world": 1, "distinct_gpus": 1, "decompressed_MBps": data.size / 1e6 / (ms / 1e3),
+             "ms_per_call": ms, "ms_min": 1e3 * min(arm["times"]), "ms_max": 1e3 * max(arm["times"]), "steps": args.steps,
+             "piece_bytes": PIECE, "compressed_bytes": len(s), "decompressed_bytes": int(data.size),
+             "verified": bool(a_ok), "library": rec["library"]}
+        r.update(info)
+        print(json.dumps(r), flush=True)
+        ok = ok and a_ok
     return ok
+
+
+PIECE = 16 << 20
+
+
+def dstream_arms(eng, h_in, n_in, n_out):
+    """The dstream and test-mode arms: each a dict with `call` (-> total_out), `times`, `out` (pinned, or None)."""
+    L = eng._L
+    in_ptr = h_in.ctypes.data
+    out = pinned(n_out + 64)
+    out_ptr, pos = out.ctypes.data, [0]
+
+    def sink(_user, data, n):
+        if pos[0] + n > out.size:
+            return 1
+        C.memmove(out_ptr + pos[0], data, n)
+        pos[0] += n
+        return 0
+    cb = bz.SINK(sink)
+
+    def stream(test):
+        pos[0] = 0
+        h, ti, to = C.c_void_p(), C.c_uint64(), C.c_uint64()
+        rc = L.bz2b200_dstream_open(eng._h, bz.SINK() if test else cb, None, C.byref(h))
+        if rc == bz.OK:
+            for off in range(0, n_in, PIECE):
+                rc = L.bz2b200_dstream_write(h, in_ptr + off, min(PIECE, n_in - off))
+                if rc != bz.OK:
+                    break
+            rc2 = L.bz2b200_dstream_close(h, C.byref(ti), C.byref(to))
+            rc = rc if rc != bz.OK else rc2
+        if rc != bz.OK:
+            raise bz.Bz2B200Error(rc, L.bz2b200_last_error(eng._h).decode())
+        return to.value
+    return [{"metric": "decode_dstream", "call": lambda: stream(False), "times": [], "out": out, "cb": cb, "n": 0},
+            {"metric": "decode_test", "call": lambda: stream(True), "times": [], "out": None, "n": 0}]
 
 
 def main():
@@ -94,6 +156,7 @@ def main():
     ap.add_argument("--steps", type=int, default=10)
     ap.add_argument("--warmup", type=int, default=2)
     ap.add_argument("--size-mb", type=int, default=100)
+    ap.add_argument("--dstream", action="store_true", help="also time the streaming decoder and its test mode (world 1)")
     args = ap.parse_args()
     if args.steps < 1 or min(args.gpus) < 1:
         ap.error("--steps and --gpus must be at least 1")

@@ -79,25 +79,39 @@ def main(argv=None):
                     sys.stderr.write("  %s: %d -> %d bytes (%.3f:1)\n" % (name, z.total_in, z.total_out,
                                                                          z.total_in / max(1, z.total_out)))
                 continue
-            data = sys.stdin.buffer.read() if name == "-" else open(name, "rb").read()
-            out = eng.decompress(data)
+            # pipelined in bounded memory: the archive is read in pieces while earlier pieces are decoded and their
+            # checked bytes written; -t decodes and checks on the GPU without downloading anything
             oname = name[:-4] if name.endswith(".bz2") else name + ".out"
-            if mode == "t":
-                if not a.quiet:
-                    sys.stderr.write("%s: ok\n" % name)
+            to_stdout = a.stdout or name == "-"
+            if mode == "d" and not to_stdout and os.path.exists(oname) and not a.force:
+                sys.stderr.write("bz2b200: output file %s already exists (use -f)\n" % oname)
+                rc = 1
                 continue
-            if a.stdout or name == "-":
-                sys.stdout.buffer.write(out)
-            else:
-                if os.path.exists(oname) and not a.force:
-                    sys.stderr.write("bz2b200: output file %s already exists (use -f)\n" % oname)
-                    rc = 1
-                    continue
-                with open(oname, "wb") as f:
-                    f.write(out)                          # the input file stays (reference: "ALWAYS KEEPS")
+            src = sys.stdin.buffer if name == "-" else open(name, "rb")
+            dst = None
+            if mode == "d":
+                dst = sys.stdout.buffer if to_stdout else open(oname, "wb")
+            ok = False
+            try:
+                with bz.DStream(eng, dst) as ds:
+                    while True:
+                        piece = src.read(16 << 20)
+                        if not piece:
+                            break
+                        ds.write(piece)
+                ok = True
+            finally:
+                if src is not sys.stdin.buffer:
+                    src.close()
+                if dst is not None and dst is not sys.stdout.buffer:
+                    dst.close()                           # the input file stays (reference: "ALWAYS KEEPS")
+                    if not ok:
+                        os.remove(oname)                  # as bzip2 does: no partial output file after an error
+            if mode == "t" and not a.quiet:
+                sys.stderr.write("%s: ok\n" % name)
             if a.verbose and not a.quiet:
-                sys.stderr.write("  %s: %d -> %d bytes (%.3f:1)\n" % (name, len(data), len(out),
-                                                                     len(data) / max(1, len(out))))
+                sys.stderr.write("  %s: %d -> %d bytes (%.3f:1)\n" % (name, ds.total_in, ds.total_out,
+                                                                     ds.total_in / max(1, ds.total_out)))
         except (OSError, bz.Bz2B200Error) as e:
             sys.stderr.write("bz2b200: %s: %s\n" % (name, e))
             rc = 2
