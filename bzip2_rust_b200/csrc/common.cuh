@@ -328,3 +328,6 @@ int bz_dec_candidates(bz2b200_ctx *ctx, const u8 *d_win, size_t len, u32 cap, st
 // test knob BZ2B200_MULTI_DEC_CHANCE: spurious block candidates, as chance magics inside compressed data would be
 void bz_add_chance_candidates(std::vector<u64> &cand);
 int bz_decode_core(bz2b200_ctx *ctx, const DecWindow &w, DecSink &sink, std::vector<DecEvent> &ev);
+// BZ2B200_E_FORMAT (and `err`) when a block of `ev` is longer than 100000 x its own stream's level; `level` = the first
+// stream's, for blocks before any stream event
+int bz_check_block_sizes(std::string &err, int level, const std::vector<DecEvent> &ev);

@@ -17,8 +17,9 @@
 //                     (k_ibwt_coarse / _crank / _fill), k_ibwt_write replays each segment at its output offset
 //   k_dec_rle1_*      inverse RLE1 (count pass, then write pass at the block's output offset)
 //   CRC               block CRCs with the encoder's CRC kernels; combined CRC on the host.
-// The standard run semantics are used (a count byte follows every 4 equal bytes); the reference's
-// rle1_decode drops run expansion in a block's last 5 bytes (SURVEY D.6) -- libbz2 is the authority.
+// The standard run semantics are used (a count byte follows every 4 equal bytes, also at a block's end: without it
+// libbz2 reports the block corrupt, and so does this decoder); the reference's rle1_decode drops run expansion in a
+// block's last 5 bytes (SURVEY D.6) -- libbz2 is the authority.
 #include "common.cuh"
 #include "radix.cuh"
 #include <algorithm>
@@ -189,7 +190,9 @@ __global__ void __launch_bounds__(32) k_ibwt_rank(const u32 *len, const u32 *key
     nvisit[b] = v;
 }
 
-// thread per visit: replay the segment; text position i (0-based) receives L[P^(i+1)(key)]  (bwt_sort.rs:118-128)
+// thread per visit: replay the segment; text position i (0-based) receives L[P^(i+1)(key)]  (bwt_sort.rs:118-128), i < n.
+// That is n steps from the origin, as libbz2 walks them: position n - 1 holds L[P^n(key)], which is L[key] only when the
+// origin's cycle length divides n -- always so for a true BWT, not for every L a stream can carry.
 __global__ void __launch_bounds__(256) k_ibwt_write(const u32 *P, const u8 *L, const u32 *len, const u32 *keys, u32 stride,
                                                     const u32 *visit_split, const u32 *visit_off, u32 vstride,
                                                     const u32 *nvisit, u8 *out) {
@@ -199,17 +202,20 @@ __global__ void __launch_bounds__(256) k_ibwt_write(const u32 *P, const u8 *L, c
     u32 nreg = (n + SPLIT - 1) / SPLIT;
     u32 j = visit_split[(size_t)b * vstride + v];
     u32 off = visit_off[(size_t)b * vstride + v];
+    if (off > n) return;                                    // past the walk (k_ibwt_crank's visit count is an upper bound)
     u32 row = j < nreg ? j * SPLIT : key;
     const u32 *p = P + (size_t)b * stride;
     const u8 *l = L + (size_t)b * stride;
     u8 *o = out + (size_t)b * stride;
-    // row = P^off(key); position off-1 holds L[row] for off >= 1 and position n-1 holds L[key]
-    do {
-        u32 pos = off == 0 ? n - 1 : off - 1;
-        if (off < n) o[pos] = l[row];
+    // row = P^off(key): position off-1 holds L[row] for 1 <= off <= n.  No visit starts at off = n, so the visit that
+    // reaches it writes it even on a splitter row (a visit listed at n writes the same byte).
+    for (;;) {
+        if (off) o[off - 1] = l[row];
+        if (off == n) break;
         row = p[row];
         off++;
-    } while (!is_split(row, key) && off < n);
+        if (off < n && is_split(row, key)) break;
+    }
 }
 
 #include "decode4.cuh"        // entropy decode: header, symbols, chunked inverse MTF
@@ -591,7 +597,10 @@ int bz_decode_core(bz2b200_ctx *ctx, const DecWindow &w, DecSink &sink, std::vec
         BZ_CHECK(cudaMemcpyAsync(olen.data(), d_olen, (size_t)used * 8, cudaMemcpyDeviceToHost, st));
         BZ_CHECK(cudaStreamSynchronize(st));
         u64 btotal = 0;
-        for (u32 k = 0; k < used; k++) { ooff[k] = btotal; btotal += olen[k]; }
+        for (u32 k = 0; k < used; k++) {
+            if (olen[k] == RLE1_OPEN) { ctx->err = "decode: the block at bit " + std::to_string(starts[k] + lo8) + " ends with four equal bytes and no count byte"; return BZ2B200_E_FORMAT; }
+            ooff[k] = btotal; btotal += olen[k];
+        }
         u8 *d_out = nullptr, *h_out = nullptr;
         rc = sink.counted(btotal, last, &d_out, &h_out);
         if (rc) return rc;
@@ -618,6 +627,19 @@ int bz_decode_core(bz2b200_ctx *ctx, const DecWindow &w, DecSink &sink, std::vec
         rc = sink.ready(d_out, btotal);
         if (rc) return rc;
     }
+}
+
+// Every block is at most 100000 x the level of ITS stream's "BZh<level>", as libbz2 checks it; the events are in chain
+// order and a stream's header event precedes its blocks.  `level` is the first stream's.
+int bz_check_block_sizes(std::string &err, int level, const std::vector<DecEvent> &ev) {
+    for (const DecEvent &e : ev) {
+        if (e.kind == DEC_STREAM) level = (int)e.val;
+        else if (e.kind == DEC_BLOCK && e.nblock > (u32)level * 100000u) {
+            err = "decode: block at bit " + std::to_string(e.bit) + " longer than its stream's level allows";
+            return BZ2B200_E_FORMAT;
+        }
+    }
+    return BZ2B200_OK;
 }
 
 namespace {
@@ -654,7 +676,7 @@ extern "C" int bz2b200_decompress_stream(bz2b200_ctx *ctx, const uint8_t *in, si
     if (rc) return rc;
     if (cand.empty()) return BZ2B200_E_FORMAT;
     int level = in[3] - '0';
-    for (u64 c : cand) {                                        // geometry: the largest block size any stream header announces
+    for (u64 c : cand) {                                        // buffer geometry: the largest block size any header may announce
         if (!(c & FOOT)) continue;
         size_t hb = (size_t)(((c & ~FOOT) + 80 + 7) / 8);
         if (hb + 4 <= n && in[hb] == 'B' && in[hb + 1] == 'Z' && in[hb + 2] == 'h' && in[hb + 3] >= '1' && in[hb + 3] <= '9')
@@ -665,6 +687,8 @@ extern "C" int bz2b200_decompress_stream(bz2b200_ctx *ctx, const uint8_t *in, si
     sink.ctx = ctx; sink.out = out; sink.out_cap = out_cap; sink.out_len = out_len;
     std::vector<DecEvent> ev;
     rc = bz_decode_core(ctx, w, sink, ev);
+    if (rc) return rc;
+    rc = bz_check_block_sizes(ctx->err, in[3] - '0', ev);
     if (rc) return rc;
     *out_len = sink.total;
     return BZ2B200_OK;

@@ -24,7 +24,7 @@ struct DecTables {                     // per block, global memory
     u16 perm[6][258];
     int limit[6][22], base[6][22];
     u8 seq[256];                       // used byte values ascending = initial MTF list
-    u32 T, alpha, G, status;
+    u32 T, alpha, G, status;           // G = selectors kept (at most sel_stride)
     u32 crc, key;
     u64 data_bit;                      // first bit of the symbol data
     u64 end_bit;                       // bit after the EOB code            (k_dec_bounds)
@@ -96,8 +96,8 @@ __global__ void __launch_bounds__(32) k_dec_header(const u8 *in, size_t n, const
         if (nused == 0 && !s_status) s_status = 2;
         int alpha = nused + 2;
         int T = (int)br.get(3);
-        u32 G = br.get(15);
-        if (!s_status && (T < 2 || T > 6 || G < 1 || G > sel_stride)) s_status = 3;
+        u32 G = br.get(15);                                     // any 1..32767 (libbz2 1.0.8 ignores those past its 18002)
+        if (!s_status && (T < 2 || T > 6 || G < 1)) s_status = 3;
         s_T = T; s_alpha = alpha; s_G = G; s_selbit = br.bitpos();
     }
     __syncwarp();
@@ -105,9 +105,12 @@ __global__ void __launch_bounds__(32) k_dec_header(const u8 *in, size_t n, const
     // list of the table numbers.  Selector g ends at the g-th zero bit, so the warp finds them 1024 bits at a time
     // (zeros per word, one scan); the MTF list has 6 entries, so a lane replays its share of the numbers on the
     // identity list, the 32 results are composed in order, and the lane replays its share again from its true list.
+    // All G are scanned and checked (j < T), the code lengths start after the last; only the first Gs = min(G,
+    // sel_stride) are kept.  A block has at most max_block + 1 symbols, so it never needs more groups than that: one that
+    // runs past the kept selectors fails in k_dec_bounds, where libbz2 fails it too (18002 kept, more than 900 000 bytes).
     if (s_status == 0) {
         const int T = s_T;
-        const u32 G = s_G;
+        const u32 G = s_G, Gs = min(G, sel_stride);
         const u32 *wsrc = (const u32 *)in;
         const u64 lastw = (u64)((n + 3) / 4) - 1;
         u32 found = 0, carry = 0;
@@ -129,7 +132,7 @@ __global__ void __launch_bounds__(32) k_dec_header(const u8 *in, size_t n, const
                 const int pos = __clz(m);
                 const u32 j = lastpos < 0 ? ptr + (u32)pos : (u32)(pos - lastpos - 1);
                 if (j >= (u32)T) bad = true;
-                sel[gidx] = (u8)j;
+                if (gidx < Gs) sel[gidx] = (u8)j;
                 if (gidx == G - 1) s_lenbit = bp + (u64)pos + 1;
                 gidx++; lastpos = pos;
                 m &= ~(0x80000000u >> pos);
@@ -141,8 +144,8 @@ __global__ void __launch_bounds__(32) k_dec_header(const u8 *in, size_t n, const
         if (__any_sync(0xffffffffu, bad)) { if (lane == 0) s_status = 4; }
         __syncwarp();
         if (s_status == 0) {
-            const u32 per = (G + 31) / 32;
-            const u32 g0 = min(G, (u32)lane * per), g1 = min(G, g0 + per);
+            const u32 per = (Gs + 31) / 32;
+            const u32 g0 = min(Gs, (u32)lane * per), g1 = min(Gs, g0 + per);
             u32 Lp = 0x543210u;                                 // nibble k = table number at list position k
             for (u32 g = g0; g < g1; g++) {
                 const u32 j4 = 4u * sel[g];
@@ -230,7 +233,7 @@ __global__ void __launch_bounds__(32) k_dec_header(const u8 *in, size_t n, const
     for (int i = lane; i < 6 * 22; i += 32) { (&o->limit[0][0])[i] = (&limit[0][0])[i]; (&o->base[0][0])[i] = (&base[0][0])[i]; }
     for (int i = lane; i < 256; i += 32) o->seq[i] = seq[i];
     if (lane == 0) {
-        o->T = (u32)T; o->alpha = (u32)alpha; o->G = s_G; o->status = (u32)s_status; o->crc = s_crc; o->key = s_key;
+        o->T = (u32)T; o->alpha = (u32)alpha; o->G = min(s_G, sel_stride); o->status = (u32)s_status; o->crc = s_crc; o->key = s_key;
         o->data_bit = s_data; o->end_bit = 0; o->nsym = 0; o->ngroups = 0; o->nblock = 0; o->pad = s_rand;
     }
 }

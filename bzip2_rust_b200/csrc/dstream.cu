@@ -15,10 +15,10 @@
 // The bytes from where the chain leaves the window onward (at most LOOK + 1) are carried in front of the next window;
 // a window whose edge is not past the chain's start is carried whole and waits for more input.
 // The chain's start and the stream's running combined CRC are always known here, so every footer's combined CRC is
-// checked when it is reached.  Blocks are decoded with level-9 geometry; the rule that a block is at most 100000 x
-// the largest level of the first header and every header on the chain is applied at close (a later header can raise
-// it).  Host memory is the staging buffers and the output pieces whatever the input or output size; device memory is
-// the decode workspaces, one window and two batch outputs.  In test mode (no sink) nothing is downloaded.
+// checked when it is reached.  Blocks are decoded with level-9 geometry; the rule that a block is at most 100000 x the
+// level of its own stream's header is applied to each window's blocks once the window is decoded.  Host memory is the
+// staging buffers and the output pieces whatever the input or output size; device memory is the decode workspaces, one
+// window and two batch outputs.  In test mode (no sink) nothing is downloaded.
 #include "common.cuh"
 #include <algorithm>
 #include <condition_variable>
@@ -66,8 +66,7 @@ struct bz2b200_dstream {
     long long expect = 32;                   // absolute bit where the next chain element starts
     u32 combined = 0;                        // running combined CRC of the current stream
     bool ended = false;                      // the chain ended after the input's last footer
-    int level = 0;                           // largest level of the first header and every header on the chain
-    u32 max_nblock = 0; u64 max_bit = 0;     // longest block so far and where it starts
+    int level = 0;                           // level of the current stream's header (0: none seen yet)
     std::vector<u64> cand;
     std::vector<DecEvent> ev;
     u64 total_in = 0, total_out = 0;
@@ -147,13 +146,14 @@ int process(bz2b200_dstream *d, int slot, size_t len, bool eof) {
     d->ev.clear();
     rc = bz_decode_core(ctx, w, sink, d->ev);
     if (rc) return rc;
+    rc = bz_check_block_sizes(ctx->err, d->level, d->ev);
+    if (rc) return rc;
     for (const DecEvent &e : d->ev) {
         if (e.kind == DEC_BLOCK) {
             d->combined = crc_step(d->combined, e.val);
-            if (e.nblock > d->max_nblock) { d->max_nblock = e.nblock; d->max_bit = e.bit; }
         } else if (e.kind == DEC_STREAM) {
             d->combined = 0;
-            d->level = std::max(d->level, (int)e.val);
+            d->level = (int)e.val;
         }
     }
     if (eof) {
@@ -332,10 +332,6 @@ int bz2b200_dstream_close(bz2b200_dstream *d, uint64_t *total_in, uint64_t *tota
     try { rc = submit(d, true); } catch (...) { rc = BZ2B200_E_NOMEM; }
     finish(d);
     if (rc == BZ2B200_OK) rc = d->rc;
-    if (rc == BZ2B200_OK && d->max_nblock > (u32)d->level * 100000u) {
-        rc = BZ2B200_E_FORMAT;
-        d->err = "decode: block at bit " + std::to_string(d->max_bit) + " longer than its stream's level allows";
-    }
     if (rc == BZ2B200_OK && !d->ended) { rc = BZ2B200_E_FORMAT; d->err = "the input does not end with a stream footer"; }
     if (total_in) *total_in = d->total_in;
     if (total_out) *total_out = d->total_out;

@@ -642,27 +642,22 @@ int bz2b200_decompress_stream_multi(bz2b200_mctx *m, const uint8_t *in, size_t n
         }
     }
     // ---- ordered fan-in: the first error in chain order wins; combined CRCs; block size the headers allow ----
-    // Every block is bounded by 100000 x the largest level among the first header and every header after a footer on
-    // the chain (windows decode with level-9 buffers).  bz2b200_decompress_stream takes the maximum over every footer
-    // magic followed by "BZh<level>", chance ones inside compressed data included; the two differ only where such a
-    // chance footer is followed by a larger level digit.  With several defects in one input the
-    // code returned may be E_FORMAT where the single-GPU call returns E_CRC or the reverse.
+    // Every block is bounded by 100000 x the level of its own stream's header, as in libbz2 (windows decode with level-9
+    // buffers).  With several defects in one input the code returned may be E_FORMAT where the single-GPU call returns
+    // E_CRC or the reverse.
     int level = in[3] - '0';
-    for (auto &W : m->win)
-        for (const DecEvent &e : W->events) if (e.kind == DEC_STREAM) level = std::max(level, (int)e.val);
-    const u32 max_block = (u32)level * 100000u;
     u32 combined = 0;
     bool fold = true;                                           // `combined` covers the whole stream so far
     u64 total = 0;
     for (auto &W : m->win) {
         for (const DecEvent &e : W->events) {
             if (e.kind == DEC_BLOCK) {
-                if (e.nblock > max_block) { m->err = "decode: block at bit " + std::to_string(e.bit) + " longer than its stream's level allows"; return BZ2B200_E_FORMAT; }
+                if (e.nblock > (u32)level * 100000u) { m->err = "decode: block at bit " + std::to_string(e.bit) + " longer than its stream's level allows"; return BZ2B200_E_FORMAT; }
                 combined = crc_step(combined, e.val);
             } else if (e.kind == DEC_FOOTER) {
                 if (fold && e.val != combined) { m->err = "decode: combined CRC mismatch at bit " + std::to_string(e.bit); return BZ2B200_E_CRC; }
             } else {
-                combined = 0; fold = true;
+                combined = 0; fold = true; level = (int)e.val;
             }
         }
         if (W->rc < 0) { m->err = W->err; return W->rc; }
