@@ -40,7 +40,7 @@ EXPORTS = [
     "bz2b200_create_multi", "bz2b200_destroy_multi", "bz2b200_last_error_multi", "bz2b200_multi_devices",
     "bz2b200_multi_context", "bz2b200_compress_stream_multi", "bz2b200_decompress_stream_multi", "bz2b200_multi_stats",
     "bz2b200_zstream_open", "bz2b200_zstream_write", "bz2b200_zstream_close",
-    "bz2b200_dstream_open", "bz2b200_dstream_write", "bz2b200_dstream_close",
+    "bz2b200_dstream_open", "bz2b200_dstream_write", "bz2b200_dstream_close", "bz2b200_recover",
 ]
 
 
@@ -52,6 +52,17 @@ class Bz2B200Error(RuntimeError):
 
 _lib = None
 SINK = C.CFUNCTYPE(C.c_int, C.c_void_p, C.POINTER(C.c_uint8), C.c_size_t)     # bz2b200_sink
+REC_FOOTER, REC_NO_MAGIC = 1, 2
+
+
+class RecEntry(C.Structure):
+    """bz2b200_rec_entry: one block or footer found by bz2b200_recover."""
+    _fields_ = [("bit", C.c_uint64), ("end_bit", C.c_uint64), ("out_off", C.c_uint64), ("out_len", C.c_uint32),
+                ("crc", C.c_uint32), ("status", C.c_int32), ("flags", C.c_uint32)]
+
+    def __repr__(self):
+        return "RecEntry(bit=%d, end_bit=%d, out_off=%d, out_len=%d, crc=%#010x, status=%d, flags=%d)" % (
+            self.bit, self.end_bit, self.out_off, self.out_len, self.crc, self.status, self.flags)
 
 
 def load_library():
@@ -125,6 +136,8 @@ def load_library():
     L.bz2b200_dstream_open.argtypes = [vp, SINK, vp, C.POINTER(vp)]
     L.bz2b200_dstream_write.argtypes = [vp, u8p, C.c_size_t]
     L.bz2b200_dstream_close.argtypes = [vp, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]
+    L.bz2b200_recover.argtypes = [vp, u8p, C.c_size_t, SINK, vp, C.POINTER(RecEntry), C.c_uint32,
+                                  C.POINTER(C.c_uint32), C.POINTER(C.c_uint64)]
     _lib = L
     return L
 
@@ -364,6 +377,36 @@ class Engine:
                 continue
             self._chk(rc)
             return out[:n.value].tobytes()
+
+    def recover(self, data, out=None):
+        """Block recovery (bz2b200_recover): decodes every intact block of a possibly damaged .bz2 input.  The intact
+        bytes go to `out.write` in input order (out=None: a report-only scan, nothing is downloaded).  Returns
+        (total_out, [RecEntry, ...]): one entry per block candidate and footer, see include/bz2b200.h."""
+        a = _np_u8(data)
+        err = []
+        cb = SINK()                                             # a NULL sink: report only
+        if out is not None:
+            def sink(_user, p, n):
+                try:
+                    out.write(C.string_at(p, n))
+                    return 0
+                except BaseException as e:                      # an exception must not unwind through the C library
+                    err.append(e)
+                    return 1
+            cb = SINK(sink)
+        cap = a.size // 20_000 + 256                # room for small blocks; the bound that always suffices is ~6x the input
+        ents = (RecEntry * cap)()
+        nent, total = C.c_uint32(), C.c_uint64()
+        rc = self._L.bz2b200_recover(self._h, a.ctypes.data, a.size, cb, None, ents, cap, C.byref(nent), C.byref(total))
+        if err:
+            raise err[0]
+        if rc == E_CAP:                             # the sink has every byte; a report-only scan fetches all entries
+            cap = nent.value
+            ents = (RecEntry * cap)()
+            rc = self._L.bz2b200_recover(self._h, a.ctypes.data, a.size, SINK(), None, ents, cap, C.byref(nent),
+                                         C.byref(C.c_uint64()))
+        self._chk(rc)
+        return total.value, list(ents[:nent.value])
 
     def set_timing(self, level=1):
         """0 = off, 1 = per-stage events, 2 = also CUDA events around every kernel launch."""

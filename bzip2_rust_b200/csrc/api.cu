@@ -27,9 +27,10 @@ bz2b200_ctx::~bz2b200_ctx() {
     cudaSetDevice(device);
     release_device_buffers(this);
     h_stage.release(); h_small.release(); h_out.release();
-    for (int i = 0; i < 2; i++) { h_dstage[i].release(); h_dpiece[i].release(); }
+    for (int i = 0; i < 2; i++) { h_dstage[i].release(); h_dpiece[i].release(); h_rec[i].release(); }
     for (int i = 0; i < 8; i++) if (ev[i]) cudaEventDestroy(ev[i]);
     for (int i = 0; i < 2; i++) if (ev_dec[i]) cudaEventDestroy(ev_dec[i]);
+    for (int i = 0; i < 2; i++) if (ev_rec[i]) cudaEventDestroy(ev_rec[i]);
     if (s_hi) cudaStreamDestroy(s_hi);
     for (cudaEvent_t e : ev_pool) cudaEventDestroy(e);
     for (cudaEvent_t e : up_ev) cudaEventDestroy(e);
@@ -73,6 +74,7 @@ int bz2b200_trim(bz2b200_ctx *ctx) {
     if (cudaSetDevice(ctx->device) != cudaSuccess) return BZ2B200_E_CUDA;
     cudaStreamSynchronize(ctx->stream);
     release_device_buffers(ctx);
+    for (int i = 0; i < 2; i++) ctx->h_rec[i].release();
     ctx->shard = ShardPlan();                                    // a pending shard plan pointed into the freed scans
     return BZ2B200_OK;
 }

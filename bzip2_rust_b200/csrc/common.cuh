@@ -136,6 +136,9 @@ struct bz2b200_ctx {
     DevBuf d_dwin, d_ddec[2];
     PinBuf h_dstage[2], h_dpiece[2];
     bool dstream_open = false;       // one dstream at a time uses them
+    // ---- recovery (recover.cu): page-locked pieces of intact bytes on their way to the sink ----
+    PinBuf h_rec[2];
+    cudaEvent_t ev_rec[2] = {nullptr, nullptr};
 
     // ---- per-kernel profiling (timing level 2): CUDA events around every launch ----
     KStat kstat[K_COUNT];
@@ -324,6 +327,31 @@ struct DecWindow {
     u32 max_block;                 // buffers and bounds of every block
     const std::vector<u64> *cand;  // candidate bits relative to d_win, sorted by position, bit 63 = footer magic
 };
+constexpr u64 DEC_FOOT = 1ull << 63;         // candidate flag: a footer magic
+constexpr u32 DEC_BATCH = 128;               // candidate blocks decoded per pass (one pass for 100 MB at level 9)
+constexpr u64 RLE1_OPEN = ~0ull;             // RLE1 length of a block that ends with four equal bytes and no count byte
+// per candidate block, after the entropy decode: the tail of its decode tables (decode4.cuh DecTables)
+struct DecTail { u32 T, alpha, G, status, crc, key; u64 data_bit, end_bit; u32 nsym, ngroups, nblock, pad; };
+// The two steps of a batch of at most DEC_BATCH candidate blocks, in the context's decode workspaces.  `max_block`
+// bounds every block (the buffer strides).  bz_decode_core runs them on chain members, the recovery driver
+// (recover.cu) on every candidate.
+struct DecGeom {
+    u32 max_block, stride, sel_stride, max_sym, sym_stride, ch_stride;
+    explicit DecGeom(u32 max_block);
+};
+// (a) entropy decode of the candidates starting at bits `starts` of d_bits[0, n) (the data of candidate k does not
+// reach past rends[k] unless a chance magic cut it): header, group boundaries, symbols, inverse MTF -> the BWT
+// strings in ctx->d_T; db[k] = the candidate's DecTail (status 0 = parsed)
+int bz_dec_entropy(bz2b200_ctx *ctx, const DecGeom &g, const u8 *d_bits, size_t n, const std::vector<u64> &starts,
+                   const std::vector<u64> &rends, std::vector<DecTail> &db);
+// (b) of members k < nblk with hlen[k] > 0 (BWT length; 0 = skip): inverse BWT with origin pointers hkey, de-randomisation
+// where hrand[k], RLE1 count -> olen[k] (RLE1_OPEN: no count byte at the end).  Synchronises.
+int bz_dec_unbwt(bz2b200_ctx *ctx, const DecGeom &g, u32 nblk, const u32 *hlen, const u32 *hkey, const u32 *hrand,
+                 u64 *olen);
+// ... then the RLE1 write of those members at d_out + ooff[k] (d_out >= sum olen + 64 bytes) and their block CRCs
+// -> crcs[k], valid after the next synchronisation of ctx->stream.  olen = the counted lengths with RLE1_OPEN replaced
+// by 0: such a member is not written.
+int bz_dec_write(bz2b200_ctx *ctx, const DecGeom &g, u32 nblk, const u64 *olen, const u64 *ooff, u8 *d_out, u32 *crcs);
 int bz_dec_candidates(bz2b200_ctx *ctx, const u8 *d_win, size_t len, u32 cap, std::vector<u64> &cand);
 // test knob BZ2B200_MULTI_DEC_CHANCE: spurious block candidates, as chance magics inside compressed data would be
 void bz_add_chance_candidates(std::vector<u64> &cand);

@@ -343,12 +343,177 @@ __global__ void __launch_bounds__(512) k_derandomize(u8 *blk, const u32 *len, co
     }
 }
 
-namespace {
-struct DecTail { u32 T, alpha, G, status, crc, key; u64 data_bit, end_bit; u32 nsym, ngroups, nblock, pad; };
 static_assert(sizeof(DecTail) == sizeof(DecTables) - offsetof(DecTables, T), "DecTail mirrors the tail of DecTables");
-constexpr u64 FOOT = 1ull << 63;
-constexpr u32 DEC_BATCH = 128;           // candidate blocks decoded per pass (one pass for 100 MB at level 9)
+
+DecGeom::DecGeom(u32 mb) {
+    max_block = mb;
+    stride = ((max_block + 64 + BZ_TILE - 1) / BZ_TILE) * BZ_TILE;
+    sel_stride = max_block / 50 + 8;
+    max_sym = max_block + 2;                                    // every symbol but EOB yields at least one byte
+    sym_stride = ((max_sym + 64 + DCH - 1) / DCH) * DCH;
+    ch_stride = sym_stride / DCH + 2;
+}
+
+namespace {
+// the batch's device workspaces (grow-only context buffers) and where each array lives in them
+struct DecWork {
+    DecTables *tabs; u32 *gbit; u16 *sym; u8 *vid, *lists; u32 *ccount, *coff;
+    u64 *starts, *olen, *ooff; u32 *len, *keys, *rand, *se; u64 *rend;
+};
+int dec_work(bz2b200_ctx *ctx, const DecGeom &g, DecWork &W) {
+    const u32 NB = DEC_BATCH;
+    BZ_CHECK(ctx->d_T.ensure((size_t)NB * g.stride + 64));
+    BZ_CHECK(ctx->d_bwt.ensure((size_t)NB * g.stride + 64));
+    BZ_CHECK(ctx->d_sel.ensure((size_t)NB * g.sel_stride));
+    BZ_CHECK(ctx->d_gbits.ensure((size_t)NB * g.sel_stride * 4));
+    BZ_CHECK(ctx->d_sym.ensure((size_t)NB * g.sym_stride * 2));
+    BZ_CHECK(ctx->d_mtfstate.ensure((size_t)NB * g.ch_stride * 256));
+    BZ_CHECK(ctx->d_chunkrec.ensure((size_t)NB * g.ch_stride * 8));
+    BZ_CHECK(ctx->d_hdr.ensure((size_t)NB * sizeof(DecTables)));
+    BZ_CHECK(ctx->d_dec3.ensure((size_t)NB * (8 + 4 + 4 + 4 + 8 + 8 + 8 + 8) + 256));
+    BZ_CHECK(ctx->d_crc.ensure((size_t)NB * 4));
+    BZ_CHECK(ctx->d_KEYB.ensure((size_t)NB * g.sym_stride));
+    W.tabs = ctx->d_hdr.as<DecTables>();
+    W.gbit = ctx->d_gbits.as<u32>();
+    W.sym = ctx->d_sym.as<u16>();
+    W.vid = ctx->d_KEYB.as<u8>();                               // start-list position selected by every MTF symbol (k_dec_chunks -> k_dec_expand)
+    W.lists = ctx->d_mtfstate.as<u8>();
+    W.ccount = ctx->d_chunkrec.as<u32>();
+    W.coff = W.ccount + (size_t)NB * g.ch_stride;
+    W.starts = ctx->d_dec3.as<u64>();
+    W.olen = W.starts + NB;
+    W.ooff = W.olen + NB;
+    W.len = (u32 *)(W.ooff + NB);
+    W.keys = W.len + NB;
+    W.rand = W.keys + NB;
+    W.se = W.rand + NB;
+    W.rend = (u64 *)(W.se + 2 * (size_t)NB);                    // after the spans; 8-byte aligned (all counts are multiples of NB * 4, NB even)
+    if (!ctx->dec_attr_done) { BZ_CHECK(cudaFuncSetAttribute(k_dec_bounds, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)JRING_BYTES)); ctx->dec_attr_done = true; }
+    return BZ2B200_OK;
+}
 }  // namespace
+
+int bz_dec_entropy(bz2b200_ctx *ctx, const DecGeom &g, const u8 *d_bits, size_t n, const std::vector<u64> &starts,
+                   const std::vector<u64> &rends, std::vector<DecTail> &db) {
+    cudaStream_t st = ctx->stream;
+    DecWork W;
+    int rc = dec_work(ctx, g, W);
+    if (rc) return rc;
+    const u32 nb = (u32)starts.size();
+    const u32 sel_stride = g.sel_stride, sym_stride = g.sym_stride, ch_stride = g.ch_stride;
+    u64 max_range = 0;
+    for (u32 k = 0; k < nb; k++) max_range = std::max(max_range, rends[k] - starts[k]);
+    BZ_CHECK(cudaMemcpyAsync(W.starts, starts.data(), (size_t)nb * 8, cudaMemcpyHostToDevice, st));
+    BZ_CHECK(cudaMemcpyAsync(W.rend, rends.data(), (size_t)nb * 8, cudaMemcpyHostToDevice, st));
+    ctx->prof_begin(K_DEC_HEADER, 0); k_dec_header<<<nb, 32, 0, st>>>(d_bits, n, W.starts, ctx->d_sel.as<u8>(), sel_stride, W.tabs); LAUNCH_OK();
+    {   // group boundaries: jump tables (2 bytes per bit offset and table), and the walkers of the same blocks following
+        // them window by window from a second, high-priority stream (their few CTAs are placed as soon as the producer's
+        // first ones retire); in slices of the batch when the tables of all its blocks would not fit the budget
+        // (incompressible data: 88 MB per block).  The producer is launched first: a tool that serialises kernels in
+        // launch order (ncu, compute-sanitizer) then still terminates.
+        // The walkers spin until their producer's CTAs have run.  One context's walkers (at most DEC_BATCH CTAs, two per
+        // SM by shared memory) leave most SMs to its producer; the walkers of several contexts on one device could take
+        // every SM while their producers wait for one.  So when this process holds more than one context on the device,
+        // the phase runs under a per-device lock until its walkers are done: then the walkers on the device are those of
+        // one batch, and every other kernel of the process on it finishes without waiting for anything.  (The count is
+        // read without the lock: a context created while the device's only other context runs this phase unlocked
+        // overlaps it once -- two batches, at most 128 of the 148 SMs, still leave SMs to both producers.)
+        std::unique_lock<std::mutex> dev_lk;
+        if (bz_contexts_on_device(ctx->device) > 1) dev_lk = std::unique_lock<std::mutex>(bz_device_lock(ctx->device));
+        const u32 nwin_max = jump_windows(max_range);
+        const size_t jstride = (size_t)nwin_max * 6 * 2 * JW;
+        const size_t budget = (size_t)6 << 30;
+        const u32 slice = (u32)std::max<size_t>(1, std::min<size_t>(nb, budget / jstride));
+        BZ_CHECK(ctx->d_VALA.ensure((size_t)slice * jstride));
+        BZ_CHECK(ctx->d_VALB.ensure((size_t)slice * nwin_max * 4));
+        u32 *d_flags = ctx->d_VALB.as<u32>();
+        if (!ctx->s_hi) {
+            int lo = 0, hi_p = 0;
+            BZ_CHECK(cudaDeviceGetStreamPriorityRange(&lo, &hi_p));
+            BZ_CHECK(cudaStreamCreateWithPriority(&ctx->s_hi, cudaStreamNonBlocking, hi_p));
+            for (int q = 0; q < 2; q++) BZ_CHECK(cudaEventCreateWithFlags(&ctx->ev_dec[q], cudaEventDisableTiming));
+        }
+        for (u32 b0 = 0; b0 < nb; b0 += slice) {
+            const u32 cnt = std::min(slice, nb - b0);
+            BZ_CHECK(cudaMemsetAsync(d_flags, 0, (size_t)cnt * nwin_max * 4, st));
+            BZ_CHECK(cudaEventRecord(ctx->ev_dec[0], st));                   // headers parsed, flags clear, the previous slice done
+            ctx->prof_begin(K_DEC_JUMPS, (u64)cnt * jstride);
+            k_dec_jumps<<<dim3(cnt, nwin_max), 256, 0, st>>>(d_bits, n, W.tabs, W.rend, ctx->d_VALA.as<u8>(), jstride, d_flags, nwin_max, b0); LAUNCH_OK();
+            BZ_CHECK(cudaStreamWaitEvent(ctx->s_hi, ctx->ev_dec[0], 0));
+            k_dec_bounds<<<cnt, 32, JRING_BYTES, ctx->s_hi>>>(d_bits, n, ctx->d_sel.as<u8>(), sel_stride, W.tabs, W.rend, ctx->d_VALA.as<u8>(), jstride, d_flags, nwin_max, W.gbit, g.max_sym, b0);
+            ctx->launches++;
+            if (cudaGetLastError() != cudaSuccess) { ctx->err = "decode: k_dec_bounds launch"; cudaStreamSynchronize(st); return BZ2B200_E_CUDA; }
+            BZ_CHECK(cudaEventRecord(ctx->ev_dec[1], ctx->s_hi));
+            ctx->prof_begin(K_DEC_BOUNDS, n);                                // as timed on the main stream: what the walk adds after the producer
+            BZ_CHECK(cudaStreamWaitEvent(st, ctx->ev_dec[1], 0));
+            ctx->prof_end(); ctx->launches--;
+        }
+        if (dev_lk.owns_lock()) BZ_CHECK(cudaStreamSynchronize(ctx->s_hi));
+    }
+    dim3 gs((sel_stride + 127) / 128, nb);
+    ctx->prof_begin(K_DEC_SYMS, n); k_dec_syms<<<gs, 128, 0, st>>>(d_bits, n, ctx->d_sel.as<u8>(), sel_stride, W.tabs, W.gbit, W.sym, sym_stride); LAUNCH_OK();
+    dim3 gch((ch_stride + 7) / 8, nb);
+    ctx->prof_begin(K_DEC_CHUNKS, 0); k_dec_chunks<<<gch, 256, 0, st>>>(W.tabs, W.sym, sym_stride, W.lists, W.ccount, ch_stride, W.vid, g.max_block); LAUNCH_OK();
+    ctx->prof_begin(K_DEC_CHUNK_SCAN, 0); k_dec_chunk_scan<<<nb, 256, 0, st>>>(W.tabs, W.lists, W.ccount, W.coff, ch_stride, g.max_block); LAUNCH_OK();
+    ctx->prof_begin(K_DEC_EXPAND, 0); k_dec_expand<<<gch, 256, 0, st>>>(W.tabs, W.sym, sym_stride, W.lists, W.coff, ch_stride, W.vid, ctx->d_T.as<u8>(), g.stride); LAUNCH_OK();
+    db.resize(nb);
+    BZ_CHECK(cudaMemcpy2DAsync(db.data(), sizeof(DecTail), (const u8 *)W.tabs + offsetof(DecTables, T), sizeof(DecTables),
+                               sizeof(DecTail), nb, cudaMemcpyDeviceToHost, st));
+    BZ_CHECK(cudaStreamSynchronize(st));
+    return BZ2B200_OK;
+}
+
+int bz_dec_unbwt(bz2b200_ctx *ctx, const DecGeom &g, u32 nblk, const u32 *hlen, const u32 *hkey, const u32 *hrand, u64 *olen) {
+    cudaStream_t st = ctx->stream;
+    DecWork W;
+    int rc = dec_work(ctx, g, W);
+    if (rc) return rc;
+    u32 max_n = 0; u64 total_n = 0;
+    bool any_rand = false;
+    for (u32 k = 0; k < nblk; k++) { max_n = std::max(max_n, hlen[k]); total_n += hlen[k]; any_rand |= hlen[k] && hrand[k]; }
+    BZ_CHECK(cudaMemcpyAsync(W.len, hlen, (size_t)nblk * 4, cudaMemcpyHostToDevice, st));
+    BZ_CHECK(cudaMemcpyAsync(W.keys, hkey, (size_t)nblk * 4, cudaMemcpyHostToDevice, st));
+    BZ_CHECK(cudaMemcpyAsync(W.rand, hrand, (size_t)nblk * 4, cudaMemcpyHostToDevice, st));
+    // ---- inverse BWT (+ de-randomisation of legacy blocks) ----
+    Batch B;
+    B.nblk = (int)nblk; B.stride = g.stride; B.tiles = g.stride / BZ_TILE; B.max_n = max_n; B.nbits = 20; B.T = ctx->d_T.as<u8>();
+    B.len = W.len; B.total_n = total_n;
+    rc = ibwt_batch(ctx, B, W.keys, ctx->d_bwt.as<u8>());
+    if (rc) return rc;
+    if (any_rand) { ctx->prof_begin(K_DEC_MISC, total_n); k_derandomize<<<nblk, 512, 0, st>>>(ctx->d_bwt.as<u8>(), W.len, W.rand, g.stride); LAUNCH_OK(); }
+    // ---- inverse RLE1, count pass ----
+    ctx->prof_begin(K_DEC_RLE1_COUNT, total_n); k_rle1_inv<0><<<nblk, 256, 0, st>>>(ctx->d_bwt.as<u8>(), W.len, g.stride, W.olen, nullptr, nullptr); LAUNCH_OK();
+    BZ_CHECK(cudaMemcpyAsync(olen, W.olen, (size_t)nblk * 8, cudaMemcpyDeviceToHost, st));
+    BZ_CHECK(cudaStreamSynchronize(st));
+    return BZ2B200_OK;
+}
+
+int bz_dec_write(bz2b200_ctx *ctx, const DecGeom &g, u32 nblk, const u64 *olen, const u64 *ooff, u8 *d_out, u32 *crcs) {
+    cudaStream_t st = ctx->stream;
+    DecWork W;
+    int rc = dec_work(ctx, g, W);
+    if (rc) return rc;
+    u64 btotal = 0;
+    for (u32 k = 0; k < nblk; k++) btotal += olen[k];
+    BZ_CHECK(cudaMemcpyAsync(W.ooff, ooff, (size_t)nblk * 8, cudaMemcpyHostToDevice, st));
+    ctx->prof_begin(K_DEC_RLE1_WRITE, btotal); k_rle1_inv<1><<<nblk, 256, 0, st>>>(ctx->d_bwt.as<u8>(), W.len, g.stride, W.olen, W.ooff, d_out); LAUNCH_OK();
+    // block CRCs in sub-ranges of at most 2 GiB of output (a block decodes to at most ~46 MB; spans are 32-bit)
+    std::vector<u32> se(2 * (size_t)nblk);
+    for (u32 k0 = 0; k0 < nblk;) {
+        u32 k1 = k0; u64 sub = 0, max_span = 0;
+        while (k1 < nblk && (k1 == k0 || sub + olen[k1] <= (1ull << 31))) {
+            se[2 * k1] = (u32)sub; se[2 * k1 + 1] = (u32)(sub + olen[k1]);
+            sub += olen[k1]; max_span = std::max(max_span, olen[k1]); k1++;
+        }
+        BZ_CHECK(cudaMemcpyAsync(W.se + 2 * k0, se.data() + 2 * k0, (size_t)(k1 - k0) * 8, cudaMemcpyHostToDevice, st));
+        rc = bz_crc_spans_dev(ctx, d_out + ooff[k0], W.se + 2 * k0, k1 - k0, (u32)max_span, ctx->d_crc.as<u32>() + k0);
+        if (rc) return rc;
+        BZ_CHECK(cudaStreamSynchronize(st));                    // se is reused by the next sub-range
+        k0 = k1;
+    }
+    BZ_CHECK(cudaMemcpyAsync(crcs, ctx->d_crc.p, (size_t)nblk * 4, cudaMemcpyDeviceToHost, st));
+    return BZ2B200_OK;
+}
 
 // every bit offset of d_win[0, len) that looks like a block or footer magic, sorted; BZ2B200_E_FORMAT past `cap`
 int bz_dec_candidates(bz2b200_ctx *ctx, const u8 *d_win, size_t len, u32 cap, std::vector<u64> &cand) {
@@ -365,7 +530,7 @@ int bz_dec_candidates(bz2b200_ctx *ctx, const u8 *d_win, size_t len, u32 cap, st
     if (ncand > cap) { ctx->err = "decode: more magic candidates than the candidate buffer holds"; return BZ2B200_E_FORMAT; }
     cand.resize(ncand);
     if (ncand) BZ_CHECK(cudaMemcpy(cand.data(), d_cand, (size_t)ncand * 8, cudaMemcpyDeviceToHost));
-    std::sort(cand.begin(), cand.end(), [](u64 a, u64 b) { return (a & ~FOOT) < (b & ~FOOT); });
+    std::sort(cand.begin(), cand.end(), [](u64 a, u64 b) { return (a & ~DEC_FOOT) < (b & ~DEC_FOOT); });
     return BZ2B200_OK;
 }
 
@@ -373,13 +538,13 @@ int bz_dec_candidates(bz2b200_ctx *ctx, const u8 *d_win, size_t len, u32 cap, st
 // inside compressed data would be
 void bz_add_chance_candidates(std::vector<u64> &cand) {
     std::vector<u64> add;
-    if (cand.empty() || (cand[0] & ~FOOT) != 0) add.push_back(0);
+    if (cand.empty() || (cand[0] & ~DEC_FOOT) != 0) add.push_back(0);
     for (size_t i = 0; i + 1 < cand.size(); i++) {
-        u64 a = cand[i] & ~FOOT, b = cand[i + 1] & ~FOOT;
+        u64 a = cand[i] & ~DEC_FOOT, b = cand[i + 1] & ~DEC_FOOT;
         if (b - a >= 2) add.push_back((a + b) / 2);
     }
     cand.insert(cand.end(), add.begin(), add.end());
-    std::sort(cand.begin(), cand.end(), [](u64 x, u64 y) { return (x & ~FOOT) < (y & ~FOOT); });
+    std::sort(cand.begin(), cand.end(), [](u64 x, u64 y) { return (x & ~DEC_FOOT) < (y & ~DEC_FOOT); });
 }
 
 // A magic can also occur by chance inside entropy-coded data, and a file may hold several streams one after the other
@@ -389,47 +554,15 @@ void bz_add_chance_candidates(std::vector<u64> &cand) {
 // A window that does not know where its chain enters entropy-decodes the first batch of its candidates first: the true
 // start is the first element at or after the window's first bit, so it is among them.
 int bz_decode_core(bz2b200_ctx *ctx, const DecWindow &w, DecSink &sink, std::vector<DecEvent> &ev) {
-    cudaStream_t st = ctx->stream;
     const std::vector<u64> &cand = *w.cand;
     const size_t ncand = cand.size();
     const size_t n = w.len;                                     // bytes on the device
     const u64 lo8 = (u64)w.lo * 8;
     const u64 hi = w.hi_bit == ~0ull ? ~0ull : w.hi_bit - lo8;  // window-relative, like every bit below
     const u32 max_block = w.max_block;
-    const u32 stride = ((max_block + 64 + BZ_TILE - 1) / BZ_TILE) * BZ_TILE;
-    const u32 sel_stride = max_block / 50 + 8;
-    const u32 max_sym = max_block + 2;                           // every symbol but EOB yields at least one byte
-    const u32 sym_stride = ((max_sym + 64 + DCH - 1) / DCH) * DCH;
-    const u32 ch_stride = sym_stride / DCH + 2;
+    const DecGeom g(max_block);
     const u32 NB = DEC_BATCH;
-    BZ_CHECK(ctx->d_T.ensure((size_t)NB * stride + 64));
-    BZ_CHECK(ctx->d_bwt.ensure((size_t)NB * stride + 64));
-    BZ_CHECK(ctx->d_sel.ensure((size_t)NB * sel_stride));
-    BZ_CHECK(ctx->d_gbits.ensure((size_t)NB * sel_stride * 4));
-    BZ_CHECK(ctx->d_sym.ensure((size_t)NB * sym_stride * 2));
-    BZ_CHECK(ctx->d_mtfstate.ensure((size_t)NB * ch_stride * 256));
-    BZ_CHECK(ctx->d_chunkrec.ensure((size_t)NB * ch_stride * 8));
-    BZ_CHECK(ctx->d_hdr.ensure((size_t)NB * sizeof(DecTables)));
-    BZ_CHECK(ctx->d_dec3.ensure((size_t)NB * (8 + 4 + 4 + 4 + 8 + 8 + 8 + 8) + 256));
-    BZ_CHECK(ctx->d_crc.ensure((size_t)NB * 4));
-    DecTables *d_tabs = ctx->d_hdr.as<DecTables>();
-    u32 *d_gbit = ctx->d_gbits.as<u32>();
-    u16 *d_sym = ctx->d_sym.as<u16>();
-    BZ_CHECK(ctx->d_KEYB.ensure((size_t)NB * sym_stride));
-    u8 *d_vid = ctx->d_KEYB.as<u8>();                           // start-list position selected by every MTF symbol (k_dec_chunks -> k_dec_expand)
-    u8 *d_lists = ctx->d_mtfstate.as<u8>();
-    u32 *d_ccount = ctx->d_chunkrec.as<u32>();
-    u32 *d_coff = d_ccount + (size_t)NB * ch_stride;
-    u64 *d_starts = ctx->d_dec3.as<u64>();
-    u64 *d_olen = d_starts + NB;
-    u64 *d_ooff = d_olen + NB;
-    u32 *d_len = (u32 *)(d_ooff + NB);
-    u32 *d_keys = d_len + NB;
-    u32 *d_rand = d_keys + NB;
-    u32 *d_se = d_rand + NB;
-    u64 *d_rend = (u64 *)(d_se + 2 * (size_t)NB);                // after the spans; 8-byte aligned (all counts are multiples of NB * 4, NB even)
     const u8 *d_bits = w.d_win;
-    if (!ctx->dec_attr_done) { BZ_CHECK(cudaFuncSetAttribute(k_dec_bounds, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)JRING_BYTES)); ctx->dec_attr_done = true; }
 
     auto read32 = [&](u64 bit) {                                // 32 bits at an absolute bit offset of the host input
         size_t byte = (size_t)(bit >> 3); int sh = (int)(bit & 7);
@@ -446,14 +579,14 @@ int bz_decode_core(bz2b200_ctx *ctx, const DecWindow &w, DecSink &sink, std::vec
     std::vector<u64> starts, rends;
     const u64 range_limit = [] { const char *e = getenv("BZ2B200_DEC_RANGE_LIMIT"); return e ? (u64)strtoull(e, nullptr, 10) : 0ull; }();
     std::vector<DecTail> db;
-    std::vector<u32> hlen(NB), hkey(NB), hrand(NB), se(2 * (size_t)NB), crcs(NB);
+    std::vector<u32> hlen(NB), hkey(NB), hrand(NB), crcs(NB);
     std::vector<u64> olen(NB), ooff(NB);
     for (;;) {
         if (known) {
             if (expect >= hi) { sink.chain_end((long long)(expect + lo8)); return BZ2B200_OK; }
-            while (ci < ncand && (cand[ci] & ~FOOT) < expect) ci++;
-            if (ci == ncand || (cand[ci] & ~FOOT) != expect) { ctx->err = "decode: no block or footer magic at bit " + std::to_string(expect + lo8); return BZ2B200_E_FORMAT; }
-            if (cand[ci] & FOOT) {                              // end of a stream: combined CRC, then end of input or another stream
+            while (ci < ncand && (cand[ci] & ~DEC_FOOT) < expect) ci++;
+            if (ci == ncand || (cand[ci] & ~DEC_FOOT) != expect) { ctx->err = "decode: no block or footer magic at bit " + std::to_string(expect + lo8); return BZ2B200_E_FORMAT; }
+            if (cand[ci] & DEC_FOOT) {                              // end of a stream: combined CRC, then end of input or another stream
                 const u32 stored = read32(expect + lo8 + 48);
                 ev.push_back(DecEvent{expect + lo8, stored, 0, DEC_FOOTER});
                 if (comb_known && stored != combined) return BZ2B200_E_CRC;                    // enforced, unlike decompress.rs:394-402
@@ -478,77 +611,20 @@ int bz_decode_core(bz2b200_ctx *ctx, const DecWindow &w, DecSink &sink, std::vec
             // A block's data cannot reach past the next candidate -- unless that one is a chance magic inside it: the walk
             // then leaves the range its jump tables cover and finishes code by code.
             starts.clear(); rends.clear();
-            u64 max_range = 0;
             for (size_t k = ci; k < ncand && starts.size() < NB; k++) {
-                if (cand[k] & FOOT) continue;
-                if ((cand[k] & ~FOOT) >= hi) break;             // the next window's
-                u64 re = k + 1 < ncand ? (cand[k + 1] & ~FOOT) : (u64)n * 8;
+                if (cand[k] & DEC_FOOT) continue;
+                if ((cand[k] & ~DEC_FOOT) >= hi) break;             // the next window's
+                u64 re = k + 1 < ncand ? (cand[k + 1] & ~DEC_FOOT) : (u64)n * 8;
                 // no valid block is longer than 20 bits per symbol plus its header (symbol map, selectors, six tables): a
                 // damaged stream whose next magic is far away must not size the jump tables
                 re = std::min<u64>(re, cand[k] + (u64)20 * (max_block + 64) + ((u64)1 << 19));
                 if (range_limit) re = std::min(re, cand[k] + range_limit);     // test knob: as if a chance magic cut the range
                 starts.push_back(cand[k]); rends.push_back(re);
-                max_range = std::max(max_range, re - cand[k]);
             }
             nb = (u32)starts.size();
             if (nb) {
-                BZ_CHECK(cudaMemcpyAsync(d_starts, starts.data(), (size_t)nb * 8, cudaMemcpyHostToDevice, st));
-                BZ_CHECK(cudaMemcpyAsync(d_rend, rends.data(), (size_t)nb * 8, cudaMemcpyHostToDevice, st));
-                ctx->prof_begin(K_DEC_HEADER, 0); k_dec_header<<<nb, 32, 0, st>>>(d_bits, n, d_starts, ctx->d_sel.as<u8>(), sel_stride, d_tabs); LAUNCH_OK();
-                {   // group boundaries: jump tables (2 bytes per bit offset and table), and the walkers of the same blocks following
-                    // them window by window from a second, high-priority stream (their few CTAs are placed as soon as the producer's
-                    // first ones retire); in slices of the batch when the tables of all its blocks would not fit the budget
-                    // (incompressible data: 88 MB per block).  The producer is launched first: a tool that serialises kernels in
-                    // launch order (ncu, compute-sanitizer) then still terminates.
-                    // The walkers spin until their producer's CTAs have run.  One context's walkers (at most DEC_BATCH CTAs, two per
-                    // SM by shared memory) leave most SMs to its producer; the walkers of several contexts on one device could take
-                    // every SM while their producers wait for one.  So when this process holds more than one context on the device,
-                    // the phase runs under a per-device lock until its walkers are done: then the walkers on the device are those of
-                    // one batch, and every other kernel of the process on it finishes without waiting for anything.  (The count is
-                    // read without the lock: a context created while the device's only other context runs this phase unlocked
-                    // overlaps it once -- two batches, at most 128 of the 148 SMs, still leave SMs to both producers.)
-                    std::unique_lock<std::mutex> dev_lk;
-                    if (bz_contexts_on_device(ctx->device) > 1) dev_lk = std::unique_lock<std::mutex>(bz_device_lock(ctx->device));
-                    const u32 nwin_max = jump_windows(max_range);
-                    const size_t jstride = (size_t)nwin_max * 6 * 2 * JW;
-                    const size_t budget = (size_t)6 << 30;
-                    const u32 slice = (u32)std::max<size_t>(1, std::min<size_t>(nb, budget / jstride));
-                    BZ_CHECK(ctx->d_VALA.ensure((size_t)slice * jstride));
-                    BZ_CHECK(ctx->d_VALB.ensure((size_t)slice * nwin_max * 4));
-                    u32 *d_flags = ctx->d_VALB.as<u32>();
-                    if (!ctx->s_hi) {
-                        int lo = 0, hi_p = 0;
-                        BZ_CHECK(cudaDeviceGetStreamPriorityRange(&lo, &hi_p));
-                        BZ_CHECK(cudaStreamCreateWithPriority(&ctx->s_hi, cudaStreamNonBlocking, hi_p));
-                        for (int q = 0; q < 2; q++) BZ_CHECK(cudaEventCreateWithFlags(&ctx->ev_dec[q], cudaEventDisableTiming));
-                    }
-                    for (u32 b0 = 0; b0 < nb; b0 += slice) {
-                        const u32 cnt = std::min(slice, nb - b0);
-                        BZ_CHECK(cudaMemsetAsync(d_flags, 0, (size_t)cnt * nwin_max * 4, st));
-                        BZ_CHECK(cudaEventRecord(ctx->ev_dec[0], st));                   // headers parsed, flags clear, the previous slice done
-                        ctx->prof_begin(K_DEC_JUMPS, (u64)cnt * jstride);
-                        k_dec_jumps<<<dim3(cnt, nwin_max), 256, 0, st>>>(d_bits, n, d_tabs, d_rend, ctx->d_VALA.as<u8>(), jstride, d_flags, nwin_max, b0); LAUNCH_OK();
-                        BZ_CHECK(cudaStreamWaitEvent(ctx->s_hi, ctx->ev_dec[0], 0));
-                        k_dec_bounds<<<cnt, 32, JRING_BYTES, ctx->s_hi>>>(d_bits, n, ctx->d_sel.as<u8>(), sel_stride, d_tabs, d_rend, ctx->d_VALA.as<u8>(), jstride, d_flags, nwin_max, d_gbit, max_sym, b0);
-                        ctx->launches++;
-                        if (cudaGetLastError() != cudaSuccess) { ctx->err = "decode: k_dec_bounds launch"; cudaStreamSynchronize(st); return BZ2B200_E_CUDA; }
-                        BZ_CHECK(cudaEventRecord(ctx->ev_dec[1], ctx->s_hi));
-                        ctx->prof_begin(K_DEC_BOUNDS, n);                                // as timed on the main stream: what the walk adds after the producer
-                        BZ_CHECK(cudaStreamWaitEvent(st, ctx->ev_dec[1], 0));
-                        ctx->prof_end(); ctx->launches--;
-                    }
-                    if (dev_lk.owns_lock()) BZ_CHECK(cudaStreamSynchronize(ctx->s_hi));
-                }
-                dim3 gs((sel_stride + 127) / 128, nb);
-                ctx->prof_begin(K_DEC_SYMS, n); k_dec_syms<<<gs, 128, 0, st>>>(d_bits, n, ctx->d_sel.as<u8>(), sel_stride, d_tabs, d_gbit, d_sym, sym_stride); LAUNCH_OK();
-                dim3 gch((ch_stride + 7) / 8, nb);
-                ctx->prof_begin(K_DEC_CHUNKS, 0); k_dec_chunks<<<gch, 256, 0, st>>>(d_tabs, d_sym, sym_stride, d_lists, d_ccount, ch_stride, d_vid, max_block); LAUNCH_OK();
-                ctx->prof_begin(K_DEC_CHUNK_SCAN, 0); k_dec_chunk_scan<<<nb, 256, 0, st>>>(d_tabs, d_lists, d_ccount, d_coff, ch_stride, max_block); LAUNCH_OK();
-                ctx->prof_begin(K_DEC_EXPAND, 0); k_dec_expand<<<gch, 256, 0, st>>>(d_tabs, d_sym, sym_stride, d_lists, d_coff, ch_stride, d_vid, ctx->d_T.as<u8>(), stride); LAUNCH_OK();
-                db.resize(nb);
-                BZ_CHECK(cudaMemcpy2DAsync(db.data(), sizeof(DecTail), (const u8 *)d_tabs + offsetof(DecTables, T), sizeof(DecTables),
-                                           sizeof(DecTail), nb, cudaMemcpyDeviceToHost, st));
-                BZ_CHECK(cudaStreamSynchronize(st));
+                int rc = bz_dec_entropy(ctx, g, d_bits, n, starts, rends, db);
+                if (rc) return rc;
             }
         }
         if (!known) {                                           // the hand-off from the window before
@@ -562,14 +638,13 @@ int bz_decode_core(bz2b200_ctx *ctx, const DecWindow &w, DecSink &sink, std::vec
             continue;
         }
         // ---- the chain inside this batch: candidate k is a block iff the block before it ends exactly there ----
-        u32 max_n = 0, used = 0; u64 total_n = 0;
+        u32 used = 0;
         for (u32 k = 0; k < nb; k++) {
             hlen[k] = 0; hkey[k] = 0; hrand[k] = 0;
             if (starts[k] != expect) continue;                  // inside another block's data: not a block
             if (db[k].status != 0) { ctx->err = "decode: block at bit " + std::to_string(starts[k] + lo8) + " status " + std::to_string(db[k].status); return BZ2B200_E_FORMAT; }
             if (db[k].key >= db[k].nblock) { ctx->err = "decode: origin pointer outside the block"; return BZ2B200_E_FORMAT; }
             hlen[k] = db[k].nblock; hkey[k] = db[k].key; hrand[k] = db[k].pad;
-            max_n = std::max(max_n, hlen[k]); total_n += hlen[k];
             combined = ((combined << 1) | (combined >> 31)) ^ db[k].crc;                       // crc.rs:25-27
             ev.push_back(DecEvent{starts[k] + lo8, db[k].crc, db[k].nblock, DEC_BLOCK});
             expect = db[k].end_bit;
@@ -579,23 +654,11 @@ int bz_decode_core(bz2b200_ctx *ctx, const DecWindow &w, DecSink &sink, std::vec
         const bool last = expect >= hi;                         // the chain left the window: the next one may go on
         if (last) sink.chain_end((long long)(expect + lo8));
         // candidates up to the last block of the chain are consumed (the next loop skips what lies below `expect`)
-        while (ci < ncand && (cand[ci] & ~FOOT) <= starts[used - 1]) ci++;
-        BZ_CHECK(cudaMemcpyAsync(d_len, hlen.data(), (size_t)nb * 4, cudaMemcpyHostToDevice, st));
-        BZ_CHECK(cudaMemcpyAsync(d_keys, hkey.data(), (size_t)nb * 4, cudaMemcpyHostToDevice, st));
-        BZ_CHECK(cudaMemcpyAsync(d_rand, hrand.data(), (size_t)nb * 4, cudaMemcpyHostToDevice, st));
-        // ---- 3. inverse BWT (+ de-randomisation of legacy blocks) ----
-        Batch B;
-        B.nblk = (int)used; B.stride = stride; B.tiles = stride / BZ_TILE; B.max_n = max_n; B.nbits = 20; B.T = ctx->d_T.as<u8>();
-        B.len = d_len; B.total_n = total_n;
-        int rc = ibwt_batch(ctx, B, d_keys, ctx->d_bwt.as<u8>());
+        while (ci < ncand && (cand[ci] & ~DEC_FOOT) <= starts[used - 1]) ci++;
+        // ---- 3. inverse BWT (+ de-randomisation of legacy blocks), inverse RLE1 + CRC; the batch's bytes go where the
+        // sink says ----
+        int rc = bz_dec_unbwt(ctx, g, used, hlen.data(), hkey.data(), hrand.data(), olen.data());
         if (rc) return rc;
-        bool any_rand = false;
-        for (u32 k = 0; k < used; k++) any_rand |= hrand[k] != 0;
-        if (any_rand) { ctx->prof_begin(K_DEC_MISC, total_n); k_derandomize<<<used, 512, 0, st>>>(ctx->d_bwt.as<u8>(), d_len, d_rand, stride); LAUNCH_OK(); }
-        // ---- 4. inverse RLE1 + CRC; the batch's bytes go where the sink says ----
-        ctx->prof_begin(K_DEC_RLE1_COUNT, total_n); k_rle1_inv<0><<<used, 256, 0, st>>>(ctx->d_bwt.as<u8>(), d_len, stride, d_olen, nullptr, nullptr); LAUNCH_OK();
-        BZ_CHECK(cudaMemcpyAsync(olen.data(), d_olen, (size_t)used * 8, cudaMemcpyDeviceToHost, st));
-        BZ_CHECK(cudaStreamSynchronize(st));
         u64 btotal = 0;
         for (u32 k = 0; k < used; k++) {
             if (olen[k] == RLE1_OPEN) { ctx->err = "decode: the block at bit " + std::to_string(starts[k] + lo8) + " ends with four equal bytes and no count byte"; return BZ2B200_E_FORMAT; }
@@ -604,24 +667,10 @@ int bz_decode_core(bz2b200_ctx *ctx, const DecWindow &w, DecSink &sink, std::vec
         u8 *d_out = nullptr, *h_out = nullptr;
         rc = sink.counted(btotal, last, &d_out, &h_out);
         if (rc) return rc;
-        BZ_CHECK(cudaMemcpyAsync(d_ooff, ooff.data(), (size_t)used * 8, cudaMemcpyHostToDevice, st));
-        ctx->prof_begin(K_DEC_RLE1_WRITE, btotal); k_rle1_inv<1><<<used, 256, 0, st>>>(ctx->d_bwt.as<u8>(), d_len, stride, nullptr, d_ooff, d_out); LAUNCH_OK();
-        // block CRCs in sub-ranges of at most 2 GiB of output (a block decodes to at most ~46 MB; spans are 32-bit)
-        for (u32 k0 = 0; k0 < used;) {
-            u32 k1 = k0; u64 sub = 0, max_span = 0;
-            while (k1 < used && (k1 == k0 || sub + olen[k1] <= (1ull << 31))) {
-                se[2 * k1] = (u32)sub; se[2 * k1 + 1] = (u32)(sub + olen[k1]);
-                sub += olen[k1]; max_span = std::max(max_span, olen[k1]); k1++;
-            }
-            BZ_CHECK(cudaMemcpyAsync(d_se + 2 * k0, se.data() + 2 * k0, (size_t)(k1 - k0) * 8, cudaMemcpyHostToDevice, st));
-            rc = bz_crc_spans_dev(ctx, d_out + ooff[k0], d_se + 2 * k0, k1 - k0, (u32)max_span, ctx->d_crc.as<u32>() + k0);
-            if (rc) return rc;
-            BZ_CHECK(cudaStreamSynchronize(st));                // se is reused by the next sub-range
-            k0 = k1;
-        }
-        BZ_CHECK(cudaMemcpyAsync(crcs.data(), ctx->d_crc.p, (size_t)used * 4, cudaMemcpyDeviceToHost, st));
-        if (btotal && h_out) BZ_CHECK(cudaMemcpyAsync(h_out, d_out, (size_t)btotal, cudaMemcpyDeviceToHost, st));
-        BZ_CHECK(cudaStreamSynchronize(st));
+        rc = bz_dec_write(ctx, g, used, olen.data(), ooff.data(), d_out, crcs.data());
+        if (rc) return rc;
+        if (btotal && h_out) BZ_CHECK(cudaMemcpyAsync(h_out, d_out, (size_t)btotal, cudaMemcpyDeviceToHost, ctx->stream));
+        BZ_CHECK(cudaStreamSynchronize(ctx->stream));
         for (u32 k = 0; k < used; k++)
             if (hlen[k] && crcs[k] != db[k].crc) { ctx->err = "decode: CRC mismatch in the block at bit " + std::to_string(starts[k] + lo8); return BZ2B200_E_CRC; }   // enforced, unlike decompress.rs:379-386
         rc = sink.ready(d_out, btotal);
@@ -677,8 +726,8 @@ extern "C" int bz2b200_decompress_stream(bz2b200_ctx *ctx, const uint8_t *in, si
     if (cand.empty()) return BZ2B200_E_FORMAT;
     int level = in[3] - '0';
     for (u64 c : cand) {                                        // buffer geometry: the largest block size any header may announce
-        if (!(c & FOOT)) continue;
-        size_t hb = (size_t)(((c & ~FOOT) + 80 + 7) / 8);
+        if (!(c & DEC_FOOT)) continue;
+        size_t hb = (size_t)(((c & ~DEC_FOOT) + 80 + 7) / 8);
         if (hb + 4 <= n && in[hb] == 'B' && in[hb + 1] == 'Z' && in[hb + 2] == 'h' && in[hb + 3] >= '1' && in[hb + 3] <= '9')
             level = std::max(level, in[hb + 3] - '0');
     }

@@ -18,14 +18,14 @@ constexpr u32 FN_ID = (0u) | (1u << 3) | (2u << 6) | (3u << 9) | (4u << 12);
 constexpr u32 FN_EQ = (1u) | (2u << 3) | (3u << 6) | (4u << 9) | (0u << 12);    // 0->1 1->2 2->3 3->4 4->0(count)
 constexpr u32 FN_NE = (1u) | (1u << 3) | (1u << 6) | (1u << 9) | (0u << 12);    // 0..3->1 4->0(count)
 
-// WRITE = 0: outlen[b] = decoded length, or RLE1_OPEN for a block that ends with four equal bytes and no count byte
-// (libbz2 then takes a count from past the block's end and reports the block corrupt).  WRITE = 1: bytes written at
-// out + outoff[b].
-constexpr u64 RLE1_OPEN = ~0ull;
+// WRITE = 0: outlen[b] = decoded length, or RLE1_OPEN (common.cuh) for a block that ends with four equal bytes and no
+// count byte (libbz2 then takes a count from past the block's end and reports the block corrupt).  WRITE = 1: bytes
+// written at out + outoff[b], except for a block the count pass found open (no room is reserved for it).
 template <int WRITE>
 __global__ void __launch_bounds__(256) k_rle1_inv(const u8 *blk, const u32 *len, u32 stride, u64 *outlen, const u64 *outoff,
                                                   u8 *out) {
     u32 b = blockIdx.x;
+    if (WRITE && outlen[b] == RLE1_OPEN) return;
     const u8 *r = blk + (size_t)b * stride;
     u32 n = len[b];
     u8 *o = WRITE ? out + outoff[b] : nullptr;

@@ -230,6 +230,46 @@ int bz2b200_bwt_decode(bz2b200_ctx *ctx, uint32_t key, const uint8_t *bwt, uint3
 int bz2b200_decompress_stream(bz2b200_ctx *ctx, const uint8_t *in, size_t n, uint8_t *out, size_t out_cap,
                               size_t *out_len);
 
+/* ---- block recovery: every intact block of a damaged .bz2 input (what bzip2recover + bzip2 -d do, block by block) -- */
+/* A candidate is every bit offset of `in` where a block magic starts.  It is INTACT when its header and codes parse, its
+ * origin pointer is inside the block, the block is at most BZ2B200_MAX_BLOCK bytes (the BZh9 bound: stream headers are
+ * not trusted, they may be the damaged part), its RLE1 tail is closed (a count byte follows four equal bytes at its end)
+ * and the CRC of its bytes equals the stored one.  A candidate inside [bit, end_bit) of an earlier intact block is a
+ * chance magic in its data and is not listed; every other candidate is listed, in input order, with its status.
+ *   Lost magics: when an intact block ends at a bit where no block or footer magic starts, the bits there are decoded
+ *   as a block anyway; an intact one is listed with BZ2B200_REC_NO_MAGIC and its bytes are recovered, otherwise nothing
+ *   is listed there (the gap between entries shows the loss).
+ *   Footers are listed with BZ2B200_REC_FOOTER (bit = the footer magic, end_bit = bit + 80, crc = the stored combined
+ *   CRC).  A footer's status is 0 only when every block entry since the previous footer (or the input's start) is
+ *   intact and the fold of their CRCs equals the stored combined CRC, so 0 means "this stream is complete"; otherwise
+ *   BZ2B200_E_FORMAT when one of those blocks is damaged, BZ2B200_E_CRC when only the fold differs.  Stream headers are
+ *   neither needed nor listed.
+ * Output: `sink` receives the bytes of the intact blocks in input order, on the calling thread, in page-locked pieces
+ * of at most 32 MiB (kept by the context; bz2b200_trim frees them).  sink == NULL is a report-only scan: nothing is
+ * downloaded.  *total_out = the sum of out_len over the entries.  For every input bz2b200_decompress_stream accepts,
+ * the sink receives the same bytes and every entry has status 0.
+ * Return codes: BZ2B200_OK when the scan finished, however much damage it found (damage is reported in the entries).
+ * BZ2B200_E_CAP when there are more entries than ent_cap: the scan still runs to the end, the sink still receives every
+ * intact byte, the first ent_cap entries are written and *nent is the count needed; n / 32 + 64 + n / 8 always suffices
+ * (candidates are at most n / 32 + 64, rescued blocks fewer than n / 8 since each spans more than 64 bits).
+ * BZ2B200_E_ARG for a NULL ctx / in / nent / total_out, n == 0, ent == NULL with ent_cap > 0, an input larger than
+ * bz2b200_decompress_stream takes, or a sink returning non-zero.  BZ2B200_E_FORMAT only when the input holds more magics
+ * than the candidate buffer (n / 32 + 64).  The whole input is uploaded once.  The context decodes afterwards. */
+#define BZ2B200_REC_FOOTER   1u    /* the entry is a stream footer */
+#define BZ2B200_REC_NO_MAGIC 2u    /* an intact block found where the block before it ends, without its block magic */
+typedef struct {
+    uint64_t bit;       /* input bit offset where the block (its magic) or footer starts */
+    uint64_t end_bit;   /* bit after the block's last code; 0 when its header or codes did not parse */
+    uint64_t out_off;   /* offset in the recovered output where its bytes start (damaged block: where they would be) */
+    uint32_t out_len;   /* decoded bytes of an intact block, else 0 */
+    uint32_t crc;       /* stored block CRC, or a footer's stored combined CRC */
+    int32_t  status;    /* 0 intact; BZ2B200_E_FORMAT did not parse, or parsed but failed the origin-pointer,
+                           size or RLE1-tail check (end_bit then set); BZ2B200_E_CRC decoded, CRC differs */
+    uint32_t flags;     /* BZ2B200_REC_FOOTER, BZ2B200_REC_NO_MAGIC */
+} bz2b200_rec_entry;
+int bz2b200_recover(bz2b200_ctx *ctx, const uint8_t *in, size_t n, bz2b200_sink sink, void *user,
+                    bz2b200_rec_entry *ent, uint32_t ent_cap, uint32_t *nent, uint64_t *total_out);
+
 /* ---- measurement hooks ------------------------------------------------------------------- */
 /* Per-stage device time (ms, CUDA events on the context's stream) of the last compress call:
  * [0]=rle1+crc+split [1]=bwt [2]=mtf/rle2 [3]=huffman select+lengths [4]=bit pack [5]=total.

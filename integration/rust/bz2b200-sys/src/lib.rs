@@ -17,6 +17,21 @@ pub const BZ2B200_E_NOMEM: c_int = -4;
 pub const BZ2B200_E_FORMAT: c_int = -5;
 pub const BZ2B200_E_CRC: c_int = -6;
 pub const BZ2B200_MAX_BLOCK: u32 = 900_000;
+pub const BZ2B200_REC_FOOTER: u32 = 1;
+pub const BZ2B200_REC_NO_MAGIC: u32 = 2;
+
+/// One block candidate or footer found by `bz2b200_recover`.
+#[repr(C)]
+#[derive(Clone, Copy, Debug, Default)]
+pub struct bz2b200_rec_entry {
+    pub bit: u64,
+    pub end_bit: u64,
+    pub out_off: u64,
+    pub out_len: u32,
+    pub crc: u32,
+    pub status: i32,
+    pub flags: u32,
+}
 
 extern "C" {
     // ---- context ----
@@ -92,6 +107,9 @@ extern "C" {
     pub fn bz2b200_bwt_decode(ctx: *mut bz2b200_ctx, key: u32, bwt: *const u8, n: u32, out: *mut u8) -> c_int;
     pub fn bz2b200_decompress_stream(ctx: *mut bz2b200_ctx, input: *const u8, n: usize, out: *mut u8, out_cap: usize,
         out_len: *mut usize) -> c_int;
+    // ---- block recovery: every intact block of a damaged input to a sink (None: report only) ----
+    pub fn bz2b200_recover(ctx: *mut bz2b200_ctx, input: *const u8, n: usize, sink: bz2b200_sink, user: *mut c_void,
+        ent: *mut bz2b200_rec_entry, ent_cap: u32, nent: *mut u32, total_out: *mut u64) -> c_int;
     // ---- measurement hooks ----
     pub fn bz2b200_set_timing(ctx: *mut bz2b200_ctx, on: c_int);
     pub fn bz2b200_get_timing(ctx: *const bz2b200_ctx, ms: *mut f32) -> c_int;
