@@ -2,6 +2,7 @@
 import numpy as np
 import pytest
 
+import bwtcraft
 from bzip2_rust_b200 import corpus
 from inputs import small_cases
 
@@ -43,6 +44,50 @@ def test_all_256_symbols(engine, ref):
     _check(engine, ref, a.tobytes(), "rand256")       # eob = 257: freq[256] truncation case of SURVEY B.3
     a = np.concatenate([np.arange(256, dtype=np.uint8)[::-1], np.zeros(5000, dtype=np.uint8), np.arange(256, dtype=np.uint8)])
     _check(engine, ref, a.tobytes(), "desc_then_zero")
+
+
+def _used_value_blocks():
+    """[(name, block)] for the four register layouts of k_mtf_emit3, chosen by the count of used byte values (at most
+    32, 64 or 128, or more): 1, 2, 32, 33, 64, 65, 128, 129, 255 and 256 values, placed lowest, spread out (0 and 255
+    included) and highest.  A block spans four CH-byte chunks, has a run across the first chunk edge and one value
+    that is used in the last chunk only; blocks of exactly CH and CH + 1 bytes end the list."""
+    ch = bwtcraft.GEO["CH"]
+    rng = np.random.default_rng(6)
+    out = []
+
+    def fill(vals, n):
+        a = np.repeat(rng.choice(vals, n), rng.integers(1, 4, n))[:n]      # short runs of random values
+        a[:len(vals)] = rng.permutation(vals)                              # every value is used
+        return a
+
+    for count in (1, 2, 32, 33, 64, 65, 128, 129, 255, 256):
+        spread = [127] if count == 1 else [i * 255 // (count - 1) for i in range(count)]
+        for place, vals in (("low", list(range(count))), ("spread", spread), ("high", list(range(256 - count, 256)))):
+            vals = np.array(vals, dtype=np.uint8)
+            late = vals[len(vals) // 2] if count > 1 else None
+            early = vals[vals != late] if count > 1 else vals
+            n = 3 * ch + ch // 2
+            a = fill(early, n)
+            a[ch - 5:ch + 7] = early[-1]                                       # a run across the first chunk edge
+            if late is not None:
+                a[n - ch // 4::7] = late                                       # first used in the last chunk
+            out.append(("used%d_%s" % (count, place), a.tobytes()))
+        for n in (ch, ch + 1):
+            vals = np.array(spread, dtype=np.uint8)
+            out.append(("used%d_n%d" % (count, n), fill(vals, n).tobytes()))
+    return out
+
+
+def test_used_value_counts_at_the_emit_layout_edges(engine, ref):
+    blocks = _used_value_blocks()
+    for name, blk in blocks:
+        assert len(set(blk)) == int(name[4:].split("_")[0]), name
+        _check(engine, ref, blk, name)
+    crcs = [ref.crc(b) for _, b in blocks]
+    got = engine.compress_blocks([b for _, b in blocks], crcs)      # all four layouts in one launch
+    for (name, blk), c, (gb, gpad) in zip(blocks, crcs, got):
+        rb, rpad, _ = ref.compress_block(blk, c, ref.SPEC_FAST)
+        assert (gb, gpad) == (rb, rpad), name
 
 
 def test_full_size_block(engine, ref):
