@@ -23,6 +23,12 @@ SO_PATH = os.path.join(_HERE, "libbz2b200.so")
 
 OK, E_ARG, E_CAP, E_CUDA, E_NOMEM, E_FORMAT, E_CRC = 0, -1, -2, -3, -4, -5, -6
 MAX_BLOCK = 900000
+LIBBZ2 = 0x100        # BZ2B200_LIBBZ2: OR into a level for libbz2 1.0.8's exact bytes instead of the reference's
+
+
+def _lvl(level, libbz2):
+    """The `level` argument of the C ABI: libbz2=True selects libbz2-identical output (BZ2B200_LIBBZ2)."""
+    return int(level) | LIBBZ2 if libbz2 else level
 
 _ERRNAMES = {E_ARG: "bad argument", E_CAP: "output buffer too small", E_CUDA: "CUDA error",
              E_NOMEM: "out of memory", E_FORMAT: "malformed stream", E_CRC: "CRC mismatch"}
@@ -267,7 +273,7 @@ class Engine:
         self._chk(self._L.bz2b200_crc32(self._h, a.ctypes.data, a.size, C.byref(c)))
         return c.value
 
-    def rle1_split(self, data, level=9):
+    def rle1_split(self, data, level=9, libbz2=False):
         """RLE1Block iterator (rle1.rs:245-264) for the whole input -> list of (crc, block bytes, in_start, in_end)."""
         a = _np_u8(data)
         cap_blocks = (a.size * 5 // 4) // (level * 100000 - 19 - 8) + 4      # RLE1 can turn 4 input bytes into 5
@@ -277,32 +283,33 @@ class Engine:
         ioff = np.zeros(cap_blocks + 1, dtype=np.uint64)
         crc = np.zeros(cap_blocks, dtype=np.uint32)
         nb = C.c_uint32()
-        self._chk(self._L.bz2b200_rle1_split(self._h, a.ctypes.data, a.size, level, out.ctypes.data, cap,
+        self._chk(self._L.bz2b200_rle1_split(self._h, a.ctypes.data, a.size, _lvl(level, libbz2), out.ctypes.data, cap,
                                              roff.ctypes.data, ioff.ctypes.data, crc.ctypes.data, cap_blocks,
                                              C.byref(nb)))
         return [(int(crc[i]), out[int(roff[i]):int(roff[i + 1])].tobytes(), int(ioff[i]), int(ioff[i + 1]))
                 for i in range(nb.value)]
 
     # ---- whole stream ----------------------------------------------------------------
-    def compress(self, data, level=9):
-        """compress (compress.rs:40): returns the .bz2 stream for `data` at block size `level`."""
+    def compress(self, data, level=9, libbz2=False):
+        """compress (compress.rs:40): returns the .bz2 stream for `data` at block size `level`.  libbz2=True: the
+        bytes bzip2 1.0.8 writes (`bz2.compress(data, level)`) instead of the reference's."""
         a = _np_u8(data)
         cap = int(self._L.bz2b200_compress_bound(a.size))
         out = np.empty(cap, dtype=np.uint8)
         n = C.c_size_t()
-        self._chk(self._L.bz2b200_compress_stream(self._h, a.ctypes.data, a.size, level, out.ctypes.data, cap,
+        self._chk(self._L.bz2b200_compress_stream(self._h, a.ctypes.data, a.size, _lvl(level, libbz2), out.ctypes.data, cap,
                                                   C.byref(n)))
         return out[:n.value].tobytes()
 
-    def compress_dev(self, d_in_ptr, n, level, d_out_ptr, out_cap):
+    def compress_dev(self, d_in_ptr, n, level, d_out_ptr, out_cap, libbz2=False):
         """Device-resident variant: raw device pointers (e.g. torch tensor .data_ptr()). Returns length."""
         ln = C.c_size_t()
-        self._chk(self._L.bz2b200_compress_stream_dev(self._h, d_in_ptr, n, level, d_out_ptr, out_cap,
+        self._chk(self._L.bz2b200_compress_stream_dev(self._h, d_in_ptr, n, _lvl(level, libbz2), d_out_ptr, out_cap,
                                                       C.byref(ln)))
         return ln.value
 
     # ---- sharding helpers (SURVEY 8e) --------------------------------------------------
-    def stream_plan(self, data, level=9, dev_ptr=None):
+    def stream_plan(self, data, level=9, dev_ptr=None, libbz2=False):
         """Block start offsets of the whole stream (n+1 entries, last = len).  `dev_ptr` = the data already on
         this GPU (raw device pointer), otherwise `data` is uploaded window by window."""
         n = data if dev_ptr is not None else _np_u8(data).size
@@ -310,17 +317,19 @@ class Engine:
         starts = np.zeros(cap + 1, dtype=np.uint64)
         nb = C.c_uint32()
         if dev_ptr is not None:
-            self._chk(self._L.bz2b200_stream_plan_dev(self._h, dev_ptr, n, level, starts.ctypes.data, cap,
+            self._chk(self._L.bz2b200_stream_plan_dev(self._h, dev_ptr, n, _lvl(level, libbz2), starts.ctypes.data, cap,
                                                       C.byref(nb)))
         else:
             a = _np_u8(data)
-            self._chk(self._L.bz2b200_stream_plan(self._h, a.ctypes.data, a.size, level, starts.ctypes.data, cap,
+            self._chk(self._L.bz2b200_stream_plan(self._h, a.ctypes.data, a.size, _lvl(level, libbz2), starts.ctypes.data, cap,
                                                   C.byref(nb)))
         return starts[:nb.value + 1].copy()
 
-    def compress_range(self, data, level, starts, first, count, dev_ptr=None, dev_out=None, dev_out_cap=0):
+    def compress_range(self, data, level, starts, first, count, dev_ptr=None, dev_out=None, dev_out_cap=0,
+                       libbz2=False):
         """Blocks [first, first+count) of the stream as a bit string -> (bytes | None, nbits, crcs)."""
         nblocks = len(starts) - 1
+        level = _lvl(level, libbz2)
         starts = np.ascontiguousarray(starts, dtype=np.uint64)
         crcs = np.zeros(max(count, 1), dtype=np.uint32)
         bits = C.c_uint64()
@@ -337,14 +346,15 @@ class Engine:
                                                  first, count, out.ctypes.data, cap, C.byref(bits), crcs.ctypes.data))
         return out[:(bits.value + 7) // 8].tobytes(), int(bits.value), crcs[:count].copy()
 
-    def shard_scan(self, d_win_ptr, win_lo, win_len, n_total, level):
+    def shard_scan(self, d_win_ptr, win_lo, win_len, n_total, level, libbz2=False):
         """Per-position scans of a window (needs no hand-off; a following shard_plan on the same window reuses them)."""
-        self._chk(self._L.bz2b200_shard_scan_dev(self._h, d_win_ptr, win_lo, win_len, n_total, level))
+        self._chk(self._L.bz2b200_shard_scan_dev(self._h, d_win_ptr, win_lo, win_len, n_total, _lvl(level, libbz2)))
 
-    def shard_plan(self, d_win_ptr, win_lo, win_len, n_total, level, start, stop_at):
+    def shard_plan(self, d_win_ptr, win_lo, win_len, n_total, level, start, stop_at, libbz2=False):
         """Plans the blocks starting in [start, stop_at) -> (next_start, nblocks); raises E_CAP if the window is short."""
         nxt, nb = C.c_size_t(), C.c_uint32()
-        self._chk(self._L.bz2b200_shard_plan_dev(self._h, d_win_ptr, win_lo, win_len, n_total, level, start, stop_at,
+        self._chk(self._L.bz2b200_shard_plan_dev(self._h, d_win_ptr, win_lo, win_len, n_total, _lvl(level, libbz2),
+                                                 start, stop_at,
                                                  C.byref(nxt), C.byref(nb)))
         return nxt.value, nb.value
 
@@ -441,9 +451,11 @@ class ZStream:
 
         with ZStream(engine, fileobj, level=9) as z:
             for piece in pieces: z.write(piece)
+
+    libbz2=True: the stream bzip2 1.0.8 writes for the concatenated input.
     """
 
-    def __init__(self, engine, out, level=9):
+    def __init__(self, engine, out, level=9, libbz2=False):
         self._L = engine._L
         self._eng = engine
         self._out = out
@@ -459,7 +471,7 @@ class ZStream:
 
         self._cb = SINK(sink)               # keep the callback object alive as long as the stream
         h = C.c_void_p()
-        rc = self._L.bz2b200_zstream_open(engine._h, level, self._cb, None, C.byref(h))
+        rc = self._L.bz2b200_zstream_open(engine._h, _lvl(level, libbz2), self._cb, None, C.byref(h))
         if rc != OK:
             if self._err is not None:
                 raise self._err             # the sink failed on the stream header
@@ -587,11 +599,11 @@ class MultiEngine:
             raise Bz2B200Error(rc, self._L.bz2b200_last_error_multi(self._h).decode())
         return ln.value
 
-    def compress(self, data, level=9):
+    def compress(self, data, level=9, libbz2=False):
         a = _np_u8(data)
         cap = int(self._L.bz2b200_compress_bound(a.size))
         out = np.empty(cap, dtype=np.uint8)
-        n = self.compress_into(a.ctypes.data, a.size, level, out.ctypes.data, cap)
+        n = self.compress_into(a.ctypes.data, a.size, _lvl(level, libbz2), out.ctypes.data, cap)
         return out[:n].tobytes()
 
     def decompress_into(self, in_ptr, n, out_ptr, out_cap):
@@ -638,8 +650,8 @@ def default_engine():
     return _default
 
 
-def compress(data, level=9):
-    return default_engine().compress(data, level)
+def compress(data, level=9, libbz2=False):
+    return default_engine().compress(data, level, libbz2=libbz2)
 
 
 def decompress(data):
@@ -658,8 +670,9 @@ def rle2_mtf_encode(bwt):
     return default_engine().rle2_mtf_encode(bwt)
 
 
-def merge_streams(level, parts):
+def merge_streams(level, parts, libbz2=False):
     """Host-side ordered merge (bitwriter.rs:77-132): parts = [(bytes, nbits, [block crcs])]."""
+    level = _lvl(level, libbz2)
     L = load_library()
     n = len(parts)
     bufs = [np.frombuffer(p[0], dtype=np.uint8) for p in parts]

@@ -203,6 +203,7 @@ int bz2b200_bwt_encode_batch(bz2b200_ctx *ctx, int nblk, const uint8_t *const *i
     if (!ctx || nblk < 0 || (nblk && (!in || !n || !bwt || !key))) return BZ2B200_E_ARG;
     if (nblk == 0) return BZ2B200_OK;
     std::lock_guard<std::mutex> lk(ctx->mu);
+    ctx->mode = BZ_MODE_REF;                                    // per-block seams: reference semantics
     if (cudaSetDevice(ctx->device) != cudaSuccess) return BZ2B200_E_CUDA;
     Batch B;
     int rc = bz_stage_blocks(ctx, nblk, in, n, B);
@@ -275,10 +276,42 @@ extern "C" int bz2b200_mtf_rle2(bz2b200_ctx *ctx, const uint8_t *bwt, uint32_t n
 // ------------------------------------------------------------------------------------------
 // huf_encode seam and the batched compress_block seam
 // ------------------------------------------------------------------------------------------
+// BZ2B200_LIBBZ2: the origin pointer of every periodic block of the batch (k_bwt_out counted the other members of
+// rotation 0's class into d_key[nblk ..]) becomes the row libbz2's sort leaves rotation 0 in.  Only such blocks are
+// downloaded; consecutive equal blocks (the inside of a long run of one byte) reuse the last answer.
+static int libbz2_periodic_origins(bz2b200_ctx *ctx, const Batch &B) {
+    cudaStream_t st = ctx->stream;
+    const size_t nb = (size_t)B.nblk;
+    std::vector<u32> h(2 * nb), len(nb);
+    BZ_CHECK(cudaMemcpyAsync(h.data(), ctx->d_key.p, 2 * nb * 4, cudaMemcpyDeviceToHost, st));
+    BZ_CHECK(cudaMemcpyAsync(len.data(), B.len, nb * 4, cudaMemcpyDeviceToHost, st));
+    BZ_CHECK(cudaStreamSynchronize(st));
+    bool any = false;
+    for (size_t b = 0; b < nb; b++) {
+        if (h[nb + b] == 0) continue;
+        std::vector<u8> blk(len[b]);
+        BZ_CHECK(cudaMemcpyAsync(blk.data(), B.T + b * B.stride, len[b], cudaMemcpyDeviceToHost, st));
+        BZ_CHECK(cudaStreamSynchronize(st));
+        if (blk != ctx->lib_last_block) {
+            long long o = bz_libbz2_fallback_origin(blk.data(), len[b]);
+            if (o < 0) { ctx->err = "libbz2 mode: origin pointer of a periodic block"; return BZ2B200_E_CUDA; }
+            ctx->lib_last_block.swap(blk);
+            ctx->lib_last_origin = (u32)o;
+        }
+        h[b] = ctx->lib_last_origin;
+        any = true;
+    }
+    if (any) {
+        BZ_CHECK(cudaMemcpyAsync(ctx->d_key.p, h.data(), nb * 4, cudaMemcpyHostToDevice, st));
+        BZ_CHECK(cudaStreamSynchronize(st));                    // h is freed on return
+    }
+    return BZ2B200_OK;
+}
+
 int bz_compress_batch(bz2b200_ctx *ctx, const Batch &B, const u32 *d_crc, HufOut &H) {
     size_t ne = (size_t)B.nblk * B.stride;
     BZ_CHECK(ctx->d_bwt.ensure(ne));
-    BZ_CHECK(ctx->d_key.ensure((size_t)B.nblk * 4));
+    BZ_CHECK(ctx->d_key.ensure((size_t)B.nblk * 8));
     BZ_CHECK(ctx->d_sym.ensure(ne * 2));
     BZ_CHECK(ctx->d_m.ensure((size_t)B.nblk * 4));
     BZ_CHECK(ctx->d_freq.ensure((size_t)B.nblk * 256 * 4));
@@ -287,6 +320,7 @@ int bz_compress_batch(bz2b200_ctx *ctx, const Batch &B, const u32 *d_crc, HufOut
     if (ctx->timing) cudaEventRecord(ctx->ev[0], st);
     int rc = bz_bwt_batch(ctx, B, ctx->d_bwt.as<u8>(), ctx->d_key.as<u32>(), ctx->d_used.as<u32>());
     if (rc) return rc;
+    if (ctx->mode == BZ_MODE_LIBBZ2 && (rc = libbz2_periodic_origins(ctx, B))) return rc;
     if (ctx->timing) cudaEventRecord(ctx->ev[1], st);
     rc = bz_mtf_batch(ctx, B, ctx->d_bwt.as<u8>(), ctx->d_sym.as<u16>(), ctx->d_m.as<u32>(), ctx->d_freq.as<u32>(),
                       ctx->d_used.as<u8>(), true);
@@ -312,6 +346,7 @@ extern "C" int bz2b200_compress_blocks(bz2b200_ctx *ctx, int nblk, const uint8_t
     if (!ctx || nblk < 0 || (nblk && (!blk || !len || !crc || !out || !out_cap || !out_bits))) return BZ2B200_E_ARG;
     if (nblk == 0) return BZ2B200_OK;
     std::lock_guard<std::mutex> lk(ctx->mu);
+    ctx->mode = BZ_MODE_REF;                                    // per-block seams: reference semantics
     if (cudaSetDevice(ctx->device) != cudaSuccess) return BZ2B200_E_CUDA;
     Batch B;
     int rc = bz_stage_blocks(ctx, nblk, blk, len, B);
@@ -341,6 +376,7 @@ extern "C" int bz2b200_huffman(bz2b200_ctx *ctx, const uint16_t *sym, uint32_t m
     if (!ctx || !sym || !freq || !symmap || !out || !out_bits || m < 2 || m > BZ2B200_MAX_BLOCK + 1 || nmap < 2 || nmap > 17)
         return BZ2B200_E_ARG;
     std::lock_guard<std::mutex> lk(ctx->mu);
+    ctx->mode = BZ_MODE_REF;                                    // per-block seams: reference semantics
     if (cudaSetDevice(ctx->device) != cudaSuccess) return BZ2B200_E_CUDA;
     // used bitmap from the symbol map (decode_sym_map, symbol_map.rs:20-42)
     u32 ub[8] = {0, 0, 0, 0, 0, 0, 0, 0};

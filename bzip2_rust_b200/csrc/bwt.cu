@@ -19,7 +19,8 @@
 //             (group head, key2) with five sweep passes and k_list_refine splits the groups.
 //      Both rewrite SA and the ranks of the refined groups and re-compact what is still tied.  Stops when
 //      every list is empty or h >= n (rotations still tied are equal: periodic block).
-//   4. key = rank[0] (first row of the class of rotation 0), bwt[j] = T[(SA[j]-1) mod n].
+//   4. key = rank[0] (first row of the class of rotation 0), bwt[j] = T[(SA[j]-1) mod n].  With BZ2B200_LIBBZ2 the
+//      other members of that class are counted too: a periodic block gets libbz2's row from the host (libbz2_order.cu).
 // Steps 2 and 3 are single-pass kernels: the running (last head, list length) prefix over the tiles of a
 // block comes from a decoupled look-back on one 64-bit state word per tile.
 #include "common.cuh"
@@ -775,12 +776,25 @@ __global__ void __launch_bounds__(256) k_used_from_hist(const u32 *counts, u32 c
 // --------------------------------------------------------------------------------------
 // step 4
 // --------------------------------------------------------------------------------------
+// others (BZ2B200_LIBBZ2, zeroed before the launch): others[b] = the rotations other than 0 whose final rank is rank[0],
+// i.e. k - 1 for a periodic block u^k.  libbz2 stores the row where its own sort leaves rotation 0 among those k equal
+// rotations; the host finds it for the blocks with others[b] > 0 (bz_libbz2_fallback_origin).
 __global__ void __launch_bounds__(BZ_THREADS) k_bwt_out(const u8 *T, const u32 *len, const u32 *SA, const u32 *RANK,
-                                                        u8 *bwt, u32 *keyout, u32 stride) {
+                                                        u8 *bwt, u32 *keyout, u32 stride, u32 *others) {
     u32 b = blockIdx.y, n = len[b];
     size_t ob = (size_t)b * stride;
     u32 base = blockIdx.x * BZ_TILE;
     if (blockIdx.x == 0 && threadIdx.x == 0) keyout[b] = n ? RANK[ob] : 0;
+    if (others && base < n) {
+        const u32 r0 = RANK[ob];
+        u32 c = 0;
+        for (int r = 0; r < BZ_IPT; r++) {
+            u32 s = base + r * BZ_THREADS + threadIdx.x;
+            if (s < n && s != 0 && RANK[ob + s] == r0) c++;
+        }
+        c = __reduce_add_sync(0xffffffffu, c);
+        if ((threadIdx.x & 31) == 0 && c) atomicAdd(&others[b], c);
+    }
 #pragma unroll 4
     for (int r = 0; r < BZ_IPT; r++) {
         u32 j = base + r * BZ_THREADS + threadIdx.x;
@@ -947,7 +961,11 @@ int bz_bwt_batch(bz2b200_ctx *ctx, const Batch &B, u8 *d_bwt, u32 *d_key, u32 *d
     }
     if (h_cnt[2 * B.nblk + 1]) { ctx->err = "bwt: a local group exceeded its capacity"; return BZ2B200_E_CUDA; }
     // ---- 4. output ----
-    ctx->prof_begin(K_BWT_OUT, ne_act * 6); k_bwt_out<<<gfull, BZ_THREADS, 0, st>>>(B.T, B.len, SA, RANK, d_bwt, d_key, B.stride); LAUNCH_OK();
+    // BZ2B200_LIBBZ2: d_key has 2 * nblk entries, the second half receives the class counts of rotation 0
+    u32 *others = ctx->mode == BZ_MODE_LIBBZ2 ? d_key + B.nblk : nullptr;
+    if (others) BZ_CHECK(cudaMemsetAsync(others, 0, (size_t)B.nblk * 4, st));
+    ctx->prof_begin(K_BWT_OUT, ne_act * (others ? 10 : 6));
+    k_bwt_out<<<gfull, BZ_THREADS, 0, st>>>(B.T, B.len, SA, RANK, d_bwt, d_key, B.stride, others); LAUNCH_OK();
     ctx->bwt_stats[0] = (u64)B.nblk; ctx->bwt_stats[1] = ne_act; ctx->bwt_stats[2] = rounds; ctx->bwt_stats[3] = listsum;
     ctx->bwt_stats[4] = h_cnt[2 * B.nblk];                       // blocks of this batch the reference would send to SA-IS
     ctx->bwt_stats[5] += h_cnt[2 * B.nblk];                      // ... and since the context was created

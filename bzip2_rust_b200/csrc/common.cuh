@@ -78,8 +78,8 @@ struct Batch {
     u64 total_n;       // sum of block lengths (host copy, for profiling byte counts)
 };
 
-enum KernelId { K_RADIX_HIST0, K_RADIX_SCAN, K_RADIX_SCATTER0, K_REF_PATH, K_BYTE_HIST, K_DIGIT_SCAN, K_SWEEP_GATHER, K_SWEEP_CARRY, K_SWEEP_LIST, K_INIT_RANKS, K_LIST_KEY, K_LIST_REFINE, K_REFINE_LOCAL, K_BWT_OUT, K_USED, K_MTF_SUMMARY, K_MTF_SCAN, K_MTF_EMIT, K_HUF_INIT, K_HUF_SELECT, K_HUF_LENGTHS, K_HUF_GBITS, K_HUF_LAYOUT, K_HUF_EMIT, K_RLE_SCAN, K_RLE_CHAIN, K_RLE_EMIT, K_CRC_PIECES, K_CRC_FINAL, K_CONCAT, K_FOOTER, K_DEC_MISC, K_DEC_MAGIC, K_DEC_HEADER, K_DEC_JUMPS, K_DEC_BOUNDS, K_DEC_SYMS, K_DEC_CHUNKS, K_DEC_EXPAND, K_DEC_CHUNK_SCAN, K_IBWT_CHASE, K_IBWT_RANK, K_IBWT_WRITE, K_DEC_RLE1_COUNT, K_DEC_RLE1_WRITE, K_COUNT };
-static const char *const kKernelNames[] = { "k_radix_hist0", "k_radix_scan", "k_radix_scatter0", "k_ref_path", "k_byte_hist", "k_digit_scan", "k_sweep_gather", "k_sweep_carry", "k_sweep_list", "k_init_ranks", "k_list_key", "k_list_refine", "k_refine_local", "k_bwt_out", "k_used", "k_mtf_summary", "k_mtf_scan", "k_mtf_emit", "k_huf_init", "k_huf_select", "k_huf_lengths", "k_huf_gbits", "k_huf_layout", "k_huf_emit", "k_rle_scan", "k_rle_chain", "k_rle_emit", "k_crc_pieces", "k_crc_final", "k_concat", "k_footer", "k_dec_misc", "k_dec_find_magic", "k_dec_header", "k_dec_jumps", "k_dec_bounds", "k_dec_syms", "k_dec_chunks", "k_dec_expand", "k_dec_chunk_scan", "k_ibwt_chase", "k_ibwt_rank", "k_ibwt_write", "k_dec_rle1_count", "k_dec_rle1_write" };
+enum KernelId { K_RADIX_HIST0, K_RADIX_SCAN, K_RADIX_SCATTER0, K_REF_PATH, K_BYTE_HIST, K_DIGIT_SCAN, K_SWEEP_GATHER, K_SWEEP_CARRY, K_SWEEP_LIST, K_INIT_RANKS, K_LIST_KEY, K_LIST_REFINE, K_REFINE_LOCAL, K_BWT_OUT, K_USED, K_MTF_SUMMARY, K_MTF_SCAN, K_MTF_EMIT, K_HUF_INIT, K_HUF_SELECT, K_HUF_LENGTHS, K_HUF_GBITS, K_HUF_LAYOUT, K_HUF_EMIT, K_RLE_SCAN, K_RLE_CHAIN, K_RLE_EMIT, K_CRC_PIECES, K_CRC_FINAL, K_CONCAT, K_FOOTER, K_DEC_MISC, K_DEC_MAGIC, K_DEC_HEADER, K_DEC_JUMPS, K_DEC_BOUNDS, K_DEC_SYMS, K_DEC_CHUNKS, K_DEC_EXPAND, K_DEC_CHUNK_SCAN, K_IBWT_CHASE, K_IBWT_RANK, K_IBWT_WRITE, K_DEC_RLE1_COUNT, K_DEC_RLE1_WRITE, K_HUF_INIT_LIBBZ2, K_HUF_LENGTHS_LIBBZ2, K_COUNT };
+static const char *const kKernelNames[] = { "k_radix_hist0", "k_radix_scan", "k_radix_scatter0", "k_ref_path", "k_byte_hist", "k_digit_scan", "k_sweep_gather", "k_sweep_carry", "k_sweep_list", "k_init_ranks", "k_list_key", "k_list_refine", "k_refine_local", "k_bwt_out", "k_used", "k_mtf_summary", "k_mtf_scan", "k_mtf_emit", "k_huf_init", "k_huf_select", "k_huf_lengths", "k_huf_gbits", "k_huf_layout", "k_huf_emit", "k_rle_scan", "k_rle_chain", "k_rle_emit", "k_crc_pieces", "k_crc_final", "k_concat", "k_footer", "k_dec_misc", "k_dec_find_magic", "k_dec_header", "k_dec_jumps", "k_dec_bounds", "k_dec_syms", "k_dec_chunks", "k_dec_expand", "k_dec_chunk_scan", "k_ibwt_chase", "k_ibwt_rank", "k_ibwt_write", "k_dec_rle1_count", "k_dec_rle1_write", "k_huf_init_libbz2", "k_huf_lengths_libbz2" };
 
 struct KStat { double ms = 0; u64 launches = 0; u64 bytes = 0; };
 struct PendingEv { int id; u64 bytes; cudaEvent_t a, b; };
@@ -93,11 +93,26 @@ struct Arrival {
     size_t waited;       // events the compute stream already waits for
 };
 
+// Output contract of a compress call.  BZ_MODE_REF: the reference's bytes.  BZ_MODE_LIBBZ2 (BZ2B200_LIBBZ2 in the level
+// argument): libbz2 1.0.8's bytes.  Three stages read it (DESIGN.md §10): the block chain of
+// rle1.cu, the origin pointer of bwt.cu and the initial tables and code lengths of huff.cu; everything else is shared.
+enum BzMode { BZ_MODE_REF = 0, BZ_MODE_LIBBZ2 = 1 };
+// Splits the `level` argument of a compress entry point: 1..9, optionally ORed with BZ2B200_LIBBZ2.  false: E_ARG.
+inline bool bz_parse_level(int *level, int *mode) {
+    const int v = *level;
+    if (v & ~(int)(BZ2B200_LIBBZ2 | 0xffu)) return false;
+    const int l = v & 0xff;
+    if (l < 1 || l > 9) return false;
+    *level = l;
+    *mode = (v & (int)BZ2B200_LIBBZ2) ? BZ_MODE_LIBBZ2 : BZ_MODE_REF;
+    return true;
+}
+
 // Pending state of the three-phase sharding entry points (shard.cu): scan -> plan -> compress on one window.
 struct ShardPlan {
     bool scanned = false;
     const u8 *d_win = nullptr; size_t win_lo = 0, win_len = 0, n_total = 0; int level = 0;
-    bool planned = false;
+    bool planned = false; int mode = BZ_MODE_REF;      // mode: of the plan, for the compress phase
     bool eof = false; u32 off_from = 0, stop_rel = 0, s0 = 0, nb = 0;
 };
 
@@ -108,6 +123,9 @@ struct bz2b200_ctx {
     cudaStream_t s_up = nullptr, s_down = nullptr;      // host-buffer pipelining (stream.cu)
     std::vector<cudaEvent_t> up_ev;
     Arrival *arrival = nullptr;
+    int mode = BZ_MODE_REF;          // BzMode of the compress call in progress (the per-block seams set BZ_MODE_REF)
+    std::vector<u8> lib_last_block;  // BZ2B200_LIBBZ2: the last periodic block whose libbz2 origin was computed, and it
+    u32 lib_last_origin = 0;
     std::mutex mu;
     std::string err;
     u64 launches = 0;
@@ -280,6 +298,8 @@ struct HufOut {
 int bz_huf_batch(bz2b200_ctx *ctx, const Batch &B, const u16 *d_sym, const u32 *d_m, const u32 *d_freq,
                  const u8 *d_used, int emit_header, const u32 *d_crc, const u32 *d_key, HufOut &out);
 
+// libbz2_order.cu: row of rotation 0 after libbz2 1.0.8's fallbackSort of block[0, n) (-1: its stack would overflow)
+long long bz_libbz2_fallback_origin(const uint8_t *block, uint32_t n);
 // rle1.cu
 int bz_rle1_window(bz2b200_ctx *ctx, const u8 *d_x, u32 W, int level, bool is_eof, u32 off_from, u32 max_blocks,
                    Batch &B, u32 *nblocks, u32 *consumed, std::vector<u32> *h_spans, bool plan_only,

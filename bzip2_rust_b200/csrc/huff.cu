@@ -235,6 +235,133 @@ __global__ void __launch_bounds__(192) k_huf_lengths(HufWs W) {
     }
 }
 
+// ---- BZ2B200_LIBBZ2: libbz2's initial partition and code lengths (DESIGN.md §10) ----------
+// k_huf_init_libbz2: one CTA per block.  Exact counts of every MTF symbol 0..EOB (EOB once), then libbz2's partition
+// of the alphabet into nGroups ranges of about remF / nPart symbols each (the odd-numbered inner ranges give their
+// last symbol back).  Same outputs as k_huf_init.
+__global__ void __launch_bounds__(256) k_huf_init_libbz2(const u16 *sym, const u32 *m_in, const u32 *usedbits, HufWs W,
+                                                         u32 stride) {
+    u32 b = blockIdx.x;
+    u32 m = m_in[b];
+    int alpha = (int)used_count(usedbits + b * 8) + 2;          // nInUse + 2 = EOB + 1
+    int T = m < 200 ? 2 : m < 600 ? 3 : m < 1200 ? 4 : m < 2400 ? 5 : 6;
+    u8 *len = W.len6 + (size_t)b * 6 * NSYM;
+    __shared__ u32 mf[NSYM];
+    for (int i = threadIdx.x; i < 6 * NSYM; i += 256) len[i] = 15;
+    for (int i = threadIdx.x; i < NSYM; i += 256) mf[i] = 0;
+    __syncthreads();
+    const u16 *s = sym + (size_t)b * stride;
+    for (u32 i = threadIdx.x; i < m; i += 256) atomicAdd(&mf[s[i]], 1u);
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        int nPart = T, gs = 0;
+        u32 remF = m;
+        while (nPart > 0) {
+            u32 tFreq = remF / (u32)nPart, aFreq = 0;
+            int ge = gs - 1;
+            while (aFreq < tFreq && ge < alpha - 1) { ge++; aFreq += mf[ge]; }
+            if (ge > gs && nPart != T && nPart != 1 && ((T - nPart) % 2 == 1)) { aFreq -= mf[ge]; ge--; }
+            for (int v = gs; v <= ge; v++) len[(nPart - 1) * NSYM + v] = 0;
+            nPart--; gs = ge + 1; remF -= aFreq;
+        }
+        u32 *mi = W.misc + b * 8;
+        mi[0] = (u32)T; mi[1] = (m + BZ_GROUP - 1) / BZ_GROUP; mi[2] = (u32)alpha;
+    }
+    __syncthreads();
+    for (int v = threadIdx.x; v < NSYM; v += 256) {
+        u64 w = 0;
+        for (int t = 0; t < 6; t++) w |= (u64)len[t * NSYM + v] << (10 * t);
+        W.tab64[(size_t)b * NSYM + v] = w;
+    }
+}
+
+// k_huf_lengths_libbz2: one warp per (block, table), BZ2_hbMakeCodeLengths(maxLen = 17) restated exactly: a binary
+// heap of leaves keyed by weight = (freq or 1) << 8 | depth, ties broken by the heap's own sift order (part of the
+// output), parents weighted (sum of counts) | (1 + max depth); while a code is longer than 17 bits every count is
+// halved (1 + c / 2) and the tree is built again.  Lane 0 runs the heap (it is serial); the lanes walk the leaf depths.
+__global__ void __launch_bounds__(192) k_huf_lengths_libbz2(HufWs W) {
+    u32 b = blockIdx.x;
+    int t = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    int T = (int)W.misc[b * 8 + 0];
+    int alpha = (int)W.misc[b * 8 + 2];
+    __shared__ u32 weight[6][2 * NSYM + 2];
+    __shared__ int parent[6][2 * NSYM + 2];
+    __shared__ int heap[6][NSYM + 2];
+    u32 *rf = W.rfreq + ((size_t)b * 6 + t) * NSYM;
+    u8 *len = W.len6 + ((size_t)b * 6 + t) * NSYM;
+    if (t < T) {
+        u32 *wt = weight[t];
+        int *par = parent[t], *hp = heap[t];
+        for (int i = lane; i < alpha; i += 32) { u32 f = rf[i]; wt[i + 1] = (f == 0 ? 1u : f) << 8; }
+        for (int s = lane; s < NSYM; s += 32) rf[s] = 0;         // ready for the next pass
+        __syncwarp();
+        for (;;) {
+            if (lane == 0) {
+                int nNodes = alpha, nHeap = 0;
+                hp[0] = 0; wt[0] = 0; par[0] = -2;
+                for (int i = 1; i <= alpha; i++) {
+                    par[i] = -1;
+                    int z = ++nHeap; hp[z] = i;                              // UPHEAP(nHeap)
+                    int tmp = hp[z]; u32 wtmp = wt[tmp];
+                    while (wtmp < wt[hp[z >> 1]]) { hp[z] = hp[z >> 1]; z >>= 1; }
+                    hp[z] = tmp;
+                }
+                while (nHeap > 1) {
+                    int nn[2];
+                    for (int k = 0; k < 2; k++) {
+                        nn[k] = hp[1]; hp[1] = hp[nHeap--];                 // DOWNHEAP(1)
+                        int z = 1, tmp = hp[z]; u32 wtmp = wt[tmp];
+                        for (;;) {
+                            int y = z << 1;
+                            if (y > nHeap) break;
+                            if (y < nHeap && wt[hp[y + 1]] < wt[hp[y]]) y++;
+                            if (wtmp < wt[hp[y]]) break;
+                            hp[z] = hp[y]; z = y;
+                        }
+                        hp[z] = tmp;
+                    }
+                    int n1 = nn[0], n2 = nn[1];
+                    nNodes++;
+                    par[n1] = par[n2] = nNodes;
+                    u32 w1 = wt[n1], w2 = wt[n2];
+                    wt[nNodes] = ((w1 & 0xffffff00u) + (w2 & 0xffffff00u)) | (1u + max(w1 & 0xffu, w2 & 0xffu));
+                    par[nNodes] = -1;
+                    int z = ++nHeap; hp[z] = nNodes;                         // UPHEAP(nHeap)
+                    int tmp = hp[z]; u32 wtmp = wt[tmp];
+                    while (wtmp < wt[hp[z >> 1]]) { hp[z] = hp[z >> 1]; z >>= 1; }
+                    hp[z] = tmp;
+                }
+            }
+            __syncwarp();
+            int maxd = 0;
+            int dep[9];
+#pragma unroll
+            for (int k = 0; k < 9; k++) {
+                int i = lane + 32 * k + 1;
+                int d = 0;
+                if (i <= alpha) { int x = i; while (par[x] >= 0) { x = par[x]; d++; } }
+                dep[k] = d;
+                maxd = max(maxd, d);
+            }
+            maxd = __reduce_max_sync(0xffffffffu, maxd);
+            if (maxd <= 17) {
+#pragma unroll
+                for (int k = 0; k < 9; k++) { int i = lane + 32 * k; if (i < alpha) len[i] = (u8)dep[k]; }
+                break;
+            }
+            for (int i = lane + 1; i <= alpha; i += 32) wt[i] = (1u + (wt[i] >> 8) / 2) << 8;
+            __syncwarp();
+        }
+    }
+    __syncthreads();
+    u8 *l6 = W.len6 + (size_t)b * 6 * NSYM;
+    for (int s = threadIdx.x; s < NSYM; s += 192) {
+        u64 v = 0;
+        for (int q = 0; q < 6; q++) v |= (u64)l6[q * NSYM + s] << (10 * q);
+        W.tab64[(size_t)b * NSYM + s] = v;
+    }
+}
+
 // ---- k_huf_gbits: thread per group -----------------------------------------------------------
 __global__ void __launch_bounds__(256) k_huf_gbits(const u16 *sym, const u32 *m_in, HufWs W, u32 stride) {
     u32 b = blockIdx.y;
@@ -508,10 +635,13 @@ int bz_huf_batch(bz2b200_ctx *ctx, const Batch &B, const u16 *d_sym, const u32 *
     BZ_CHECK(cudaMemsetAsync(W.rfreq, 0, nb * 6 * NSYM * 4, st));
     BZ_CHECK(cudaMemsetAsync(ctx->d_out.p, 0, nb * out_stride, st));
     dim3 gg((maxG + 255) / 256, B.nblk);
-    ctx->prof_begin(K_HUF_INIT, (u64)B.nblk * 4096); k_huf_init<<<B.nblk, 256, 0, st>>>(d_m, d_freq, usedbits, W); LAUNCH_OK();
+    const bool lib = ctx->mode == BZ_MODE_LIBBZ2;
+    if (lib) { ctx->prof_begin(K_HUF_INIT_LIBBZ2, ne_act * 2); k_huf_init_libbz2<<<B.nblk, 256, 0, st>>>(d_sym, d_m, usedbits, W, B.stride); LAUNCH_OK(); }
+    else { ctx->prof_begin(K_HUF_INIT, (u64)B.nblk * 4096); k_huf_init<<<B.nblk, 256, 0, st>>>(d_m, d_freq, usedbits, W); LAUNCH_OK(); }
     for (int iter = 0; iter < 4; iter++) {                       // huffman.rs:114
         ctx->prof_begin(K_HUF_SELECT, ne_act * 2); k_huf_select<<<gg, 256, 0, st>>>(d_sym, d_m, W, B.stride); LAUNCH_OK();
-        ctx->prof_begin(K_HUF_LENGTHS, (u64)B.nblk * 6 * 258 * 5); k_huf_lengths<<<B.nblk, 192, 0, st>>>(W); LAUNCH_OK();
+        if (lib) { ctx->prof_begin(K_HUF_LENGTHS_LIBBZ2, (u64)B.nblk * 6 * 258 * 5); k_huf_lengths_libbz2<<<B.nblk, 192, 0, st>>>(W); LAUNCH_OK(); }
+        else { ctx->prof_begin(K_HUF_LENGTHS, (u64)B.nblk * 6 * 258 * 5); k_huf_lengths<<<B.nblk, 192, 0, st>>>(W); LAUNCH_OK(); }
     }
     ctx->prof_begin(K_HUF_GBITS, ne_act * 2); k_huf_gbits<<<gg, 256, 0, st>>>(d_sym, d_m, W, B.stride); LAUNCH_OK();
     ctx->prof_begin(K_HUF_LAYOUT, (u64)B.nblk * 4096); k_huf_layout<<<B.nblk, 256, 0, st>>>(W, usedbits, emit_header, d_crc, d_key, ctx->d_out.as<u8>(), out_stride,

@@ -85,7 +85,7 @@ struct bz2b200_mctx {
     int done = 0;
     bool quit = false;
     // the job
-    const u8 *in = nullptr; size_t nbytes = 0; int level = 9; u8 *out = nullptr; size_t out_cap = 0;
+    const u8 *in = nullptr; size_t nbytes = 0; int level = 9; u8 *out = nullptr; size_t out_cap = 0;   // level: the caller's argument, BZ2B200_LIBBZ2 included
     std::atomic<int> abort{0};
     std::string err;
     u64 stat[8] = {0};
@@ -489,7 +489,8 @@ bz2b200_ctx *bz2b200_multi_context(bz2b200_mctx *m, int rank) { return (m && ran
 int bz2b200_compress_stream_multi(bz2b200_mctx *m, const uint8_t *in, size_t n, int level, uint8_t *out,
                                   size_t out_cap, size_t *out_len) {
     BZ_API_TRY
-    if (!m || (!in && n) || !out || !out_len || level < 1 || level > 9) return BZ2B200_E_ARG;
+    int lv = level, mode = BZ_MODE_REF;                      // m->level keeps the flag for the shard entry points
+    if (!m || (!in && n) || !out || !out_len || !bz_parse_level(&lv, &mode)) return BZ2B200_E_ARG;
     std::lock_guard<std::mutex> call(m->call_mu);
     // small inputs (or one device): the single-GPU path, same bytes
     if (m->n == 1 || n < (size_t)m->n * (8u << 20)) {
@@ -556,7 +557,7 @@ int bz2b200_compress_stream_multi(bz2b200_mctx *m, const uint8_t *in, size_t n, 
         }
         for (u32 c : W->crcs) combined = crc_step(combined, c);            // bitwriter.rs:89-91
     }
-    out[0] = 'B'; out[1] = 'Z'; out[2] = 'h'; out[3] = (u8)('0' + level);  // bitwriter.rs:67-72
+    out[0] = 'B'; out[1] = 'Z'; out[2] = 'h'; out[3] = (u8)('0' + lv);  // bitwriter.rs:67-72
     size_t len = (size_t)((pos + 80 + 7) / 8);
     if (len > out_cap) return BZ2B200_E_CAP;
     const u8 foot[10] = {0x17, 0x72, 0x45, 0x38, 0x50, 0x90, (u8)(combined >> 24), (u8)(combined >> 16), (u8)(combined >> 8), (u8)combined};

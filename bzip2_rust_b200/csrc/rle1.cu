@@ -15,7 +15,9 @@
 // whose output offset reaches block_size-1, the cursor-parity rule of the reference's stride-2 scan
 // ("a group at q is seen at cursor q if q-start is odd, else at q+1"), and the exit cursor
 // c = start+1 | start+R | start+R+1.  A block that begins inside a run restarts the run count, so
-// its first run is parsed from the block start in closed form.
+// its first run is parsed from the block start in closed form.  With BZ2B200_LIBBZ2 the chain is libbz2's instead
+// (plan_block_libbz2): a block ends at the first chunk end where OUT reaches OUT[s] + B, and runs are chunked from
+// their own start across block starts; both chain variants (BZ2B200_CHAIN_TABLES) evaluate links with it.
 // Finally one thread per input byte writes the RLE1 bytes straight into the fixed-stride batch
 // text array consumed by the BWT stage, and the block CRCs are computed as a polynomial in
 // X = x^(8*PIECE) over end-aligned pieces (leading zero bytes do not change a zero-init CRC).
@@ -259,6 +261,7 @@ struct ChainArgs {
     u32 out_w;        // OUT[W]: RLE1 bytes of the whole window (read once by the kernel)
     u32 off_from;     // EOF bookkeeping: a group starting at/after this position since the last refill puts the
                       // reference's `remaining` counter one high (rle1.rs:207) -- see DESIGN.md "EOF corner"
+    u32 mode;         // BzMode: BZ_MODE_LIBBZ2 plans libbz2's blocks (plan_block_libbz2)
     BlockRec *rec; u32 *nrec; u32 *consumed;
 };
 
@@ -308,11 +311,70 @@ __device__ __forceinline__ u32 exit_cursor(u32 g, long long R) {   // SURVEY App
     return (R & 1) ? g + (u32)R : g + (u32)R + 1;
 }
 
+enum { PLAN_OK = 0, PLAN_STOP = 1, PLAN_SEARCH = 2 };
+
+// libbz2's block (DESIGN.md §10): every maximal run is cut greedily from its own start into
+// chunks of at most 255 bytes (RLE1 size: the length below 4, else 5), and a block ends right after the first chunk at
+// which its RLE1 length reaches B.  A block start is therefore a chunk boundary, chunking from it is the global one,
+// and OUT (which counts exactly those chunks, 5 bytes at a group start) gives the whole link: the first run is cut
+// from s (the window may have begun inside it), then a lower bound on OUT and a round-up to the end of the chunk that
+// crossed B.  No cursor parity and no end-of-file arm.  The record uses BlockRec's fields the way k_rle_emit reads them:
+// [s, re) is the first run chunked from s, [re, e) the global parse, g_last = e (no trailing literals).
+template <bool COOP>
+__device__ __forceinline__ int plan_block_libbz2(const ChainArgs &a, u32 s, BlockRec &r) {
+    const u32 W = a.W, B = a.B;
+    const u32 margin = a.is_eof ? 0u : 1024u;
+    r.s = s; r.last = 0;
+    u32 re = run_end_from(a.RS, W, s);
+    if (!a.is_eof && re + margin > W) return PLAN_STOP;         // run may continue past the window
+    const u32 Lc = re - s, nfull = Lc / 255u, rem = Lc % 255u;
+    const u32 jb = (B + 4) / 5;                                 // full chunks that reach B on their own
+    u32 e, out_len;
+    if (jb <= nfull) {                                          // B is reached inside the first run
+        e = s + 255u * jb; out_len = 5u * jb;
+        r.re = e; r.out_re = out_len;
+    } else {
+        const u32 out_re = 5u * nfull + (rem >= 4 ? 5u : rem);
+        r.re = re; r.out_re = out_re;
+        if (out_re >= B) { e = re; out_len = out_re; }          // ... by the run's last, shorter chunk
+        else {
+            const long long off = (long long)out_re - (long long)a.OUT[re];
+            const long long target = (long long)B - off;        // first x > re with OUT[x] >= target
+            if ((long long)a.out_w < target) {
+                if (!a.is_eof) return PLAN_STOP;
+                e = W; out_len = (u32)((long long)a.out_w + off);
+            } else {
+                u32 x1;
+                if (COOP) x1 = warp_lower_bound(a.OUT, re, W, target);
+                else {
+                    u32 lo = re, hi = W;
+                    while (lo < hi) {
+                        u32 mid = lo + (hi - lo) / 2;
+                        if ((long long)a.OUT[mid] >= target) hi = mid; else lo = mid + 1;
+                    }
+                    x1 = lo;
+                }
+                // byte x1 - 1 emitted the bytes that crossed B: a group start (its chunk ends where group_end says) or a
+                // literal of a chunk of 1 to 3 equal bytes (the chunk ends with the run)
+                const u32 p = x1 - 1;
+                if (a.OUT[x1] - a.OUT[p] == 5u) e = group_end(a.x, W, p);
+                else { e = x1; const u8 c = a.x[p]; while (e < W && a.x[e] == c) e++; }
+                out_len = (u32)((long long)a.OUT[e] + off);
+            }
+        }
+    }
+    if (a.is_eof) { if (e == W) r.last = 1; }
+    else if (e + margin > W) return PLAN_STOP;                  // needs bytes beyond this window
+    r.e = e; r.g_last = e; r.out_g = out_len; r.out_len = out_len;
+    if (r.out_len > a.max_out) return PLAN_STOP;
+    return PLAN_OK;
+}
+
 // One block of the chain: the block that starts at input position s.  COOP = true: called by all lanes with the
 // same s (the binary search over OUT is warp cooperative); COOP = false would let a lane plan on its own.
-enum { PLAN_OK = 0, PLAN_STOP = 1, PLAN_SEARCH = 2 };
 template <bool COOP>
 __device__ __forceinline__ int plan_block(const ChainArgs &a, u32 s, BlockRec &r) {
+    if (a.mode == BZ_MODE_LIBBZ2) return plan_block_libbz2<COOP>(a, s, r);
     const u32 W = a.W, B = a.B;
     const u32 margin = a.is_eof ? 0u : 1024u;
     r.s = s; r.last = 0;
@@ -764,6 +826,7 @@ int bz_rle1_window(bz2b200_ctx *ctx, const u8 *d_x, u32 W, int level, bool is_eo
     ChainArgs a;
     a.x = d_x; a.RS = RS; a.OUT = OUT; a.LASTQ = LASTQ; a.W = W; a.B = Bsz; a.is_eof = is_eof ? 1u : 0u;
     a.max_blocks = max_blocks; a.max_out = max_n; a.off_from = off_from; a.stop_at = stop_at; a.s0 = s0;
+    a.mode = (u32)ctx->mode;
     a.rec = rec; a.nrec = d_small; a.consumed = d_small + 1;
     if (plan_only && skip_chain) { *nblocks = 0; *consumed = 0; return BZ2B200_OK; }   // scan-only call
     if (!skip_chain) {

@@ -64,9 +64,11 @@ int bz_shard_post_upload(bz2b200_ctx *ctx, const u8 *h_src, u8 *d_win, size_t wi
 
 int bz_shard_scan_arriving(bz2b200_ctx *ctx, u8 *d_win, size_t win_lo, size_t win_len, size_t n_total, int level,
                            size_t chunk, std::vector<cudaEvent_t> &evs) {
-    if (!ctx || !d_win || level < 1 || level > 9 || win_lo + win_len > n_total || win_len > 0xFFFFFF00ull || win_len == 0)
+    int mode = BZ_MODE_REF;
+    if (!ctx || !d_win || !bz_parse_level(&level, &mode) || win_lo + win_len > n_total || win_len > 0xFFFFFF00ull || win_len == 0)
         return BZ2B200_E_ARG;
     std::lock_guard<std::mutex> lk(ctx->mu);
+    ctx->mode = mode;
     if (cudaSetDevice(ctx->device) != cudaSuccess) return BZ2B200_E_CUDA;
     size_t nchunks = (win_len + chunk - 1) / chunk;
     if (evs.size() < nchunks) return BZ2B200_E_ARG;
@@ -88,9 +90,11 @@ extern "C" {
 int bz2b200_shard_scan_dev(bz2b200_ctx *ctx, const uint8_t *d_win, size_t win_lo, size_t win_len, size_t n_total,
                            int level) {
     BZ_API_TRY
-    if (!ctx || !d_win || level < 1 || level > 9 || win_lo + win_len > n_total || win_len > 0xFFFFFF00ull || win_len == 0)
+    int mode = BZ_MODE_REF;
+    if (!ctx || !d_win || !bz_parse_level(&level, &mode) || win_lo + win_len > n_total || win_len > 0xFFFFFF00ull || win_len == 0)
         return BZ2B200_E_ARG;
     std::lock_guard<std::mutex> lk(ctx->mu);
+    ctx->mode = mode;
     if (cudaSetDevice(ctx->device) != cudaSuccess) return BZ2B200_E_CUDA;
     return do_scan(ctx, ctx->shard, d_win, win_lo, win_len, n_total, level);
     BZ_API_CATCH
@@ -102,10 +106,12 @@ int bz2b200_shard_scan_dev(bz2b200_ctx *ctx, const uint8_t *d_win, size_t win_lo
 int bz2b200_shard_plan_dev(bz2b200_ctx *ctx, const uint8_t *d_win, size_t win_lo, size_t win_len, size_t n_total,
                            int level, size_t start, size_t stop_at, size_t *next_start, uint32_t *nblocks) {
     BZ_API_TRY
-    if (!ctx || !d_win || !next_start || !nblocks || level < 1 || level > 9 || win_lo + win_len > n_total ||
+    int mode = BZ_MODE_REF;
+    if (!ctx || !d_win || !next_start || !nblocks || !bz_parse_level(&level, &mode) || win_lo + win_len > n_total ||
         win_len > 0xFFFFFF00ull)
         return BZ2B200_E_ARG;
     std::lock_guard<std::mutex> lk(ctx->mu);
+    ctx->mode = mode;
     if (cudaSetDevice(ctx->device) != cudaSuccess) return BZ2B200_E_CUDA;
     ShardPlan &P = ctx->shard;
     P.planned = false;
@@ -115,7 +121,7 @@ int bz2b200_shard_plan_dev(bz2b200_ctx *ctx, const uint8_t *d_win, size_t win_lo
     if (start < win_lo) return BZ2B200_E_ARG;
     if (start >= win_lo + win_len) return BZ2B200_E_CAP;          // window does not reach the first block yet
     bool same = P.scanned && P.d_win == d_win && P.win_lo == win_lo && P.win_len == win_len && P.n_total == n_total &&
-                P.level == level;
+                P.level == level;          // the scans do not depend on the mode
     if (!same) {
         int rc = do_scan(ctx, P, d_win, win_lo, win_len, n_total, level);
         if (rc) return rc;
@@ -132,7 +138,7 @@ int bz2b200_shard_plan_dev(bz2b200_ctx *ctx, const uint8_t *d_win, size_t win_lo
     if (consumed < stop_rel && !(eof && consumed == W)) return BZ2B200_E_CAP;   // ran out of window (or 4096 blocks)
     *next_start = win_lo + consumed;
     *nblocks = nb;
-    P.planned = true; P.eof = eof; P.off_from = off_from; P.stop_rel = stop_rel; P.s0 = s0; P.nb = nb;
+    P.planned = true; P.eof = eof; P.off_from = off_from; P.stop_rel = stop_rel; P.s0 = s0; P.nb = nb; P.mode = mode;
     return BZ2B200_OK;
     BZ_API_CATCH
 }
@@ -148,6 +154,7 @@ int bz2b200_shard_compress_dev(bz2b200_ctx *ctx, uint8_t *d_out, size_t out_cap,
     ShardPlan &P = ctx->shard;
     if (!P.planned) { ctx->err = "shard_compress: no pending plan"; return BZ2B200_E_ARG; }
     P.planned = false;
+    ctx->mode = P.mode;
     *out_bits = 0;
     cudaStream_t st = ctx->stream;
     if (ctx->timing) cudaEventRecord(ctx->ev_total[0], st);

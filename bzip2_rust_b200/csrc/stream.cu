@@ -232,9 +232,11 @@ size_t bz2b200_compress_bound(size_t n) {
 int bz2b200_compress_stream_dev(bz2b200_ctx *ctx, const uint8_t *d_in, size_t n, int level, uint8_t *d_out,
                                 size_t out_cap, size_t *out_len) {
     BZ_API_TRY
-    if (!ctx || (!d_in && n) || !d_out || !out_len || level < 1 || level > 9) return BZ2B200_E_ARG;
+    int mode = BZ_MODE_REF;
+    if (!ctx || (!d_in && n) || !d_out || !out_len || !bz_parse_level(&level, &mode)) return BZ2B200_E_ARG;
     if ((uintptr_t)d_out & 3u) return BZ2B200_E_ARG;            // the bit merge works on 32-bit words of d_out
     std::lock_guard<std::mutex> lk(ctx->mu);
+    ctx->mode = mode;
     if (cudaSetDevice(ctx->device) != cudaSuccess) return BZ2B200_E_CUDA;
     u64 bits = 0;
     int rc = compress_core(ctx, d_in, n, level, d_out, out_cap & ~(size_t)3, &bits, true, true, n, 0, 0xFFFFFFFFu, nullptr);
@@ -247,8 +249,10 @@ int bz2b200_compress_stream_dev(bz2b200_ctx *ctx, const uint8_t *d_in, size_t n,
 int bz2b200_compress_stream(bz2b200_ctx *ctx, const uint8_t *in, size_t n, int level, uint8_t *out, size_t out_cap,
                             size_t *out_len) {
     BZ_API_TRY
-    if (!ctx || (!in && n) || !out || !out_len || level < 1 || level > 9) return BZ2B200_E_ARG;
+    int mode = BZ_MODE_REF;
+    if (!ctx || (!in && n) || !out || !out_len || !bz_parse_level(&level, &mode)) return BZ2B200_E_ARG;
     std::lock_guard<std::mutex> lk(ctx->mu);
+    ctx->mode = mode;
     if (cudaSetDevice(ctx->device) != cudaSuccess) return BZ2B200_E_CUDA;
     // knobs: windows per call (1 = upload everything, compress, download) and upload chunk size
     static const int n_windows = [] { const char *e = getenv("BZ2B200_E2E_WINDOWS"); int v = e ? atoi(e) : 1; return v < 1 ? 1 : v; }();
@@ -317,9 +321,11 @@ int bz2b200_crc32(bz2b200_ctx *ctx, const uint8_t *data, size_t n, uint32_t *crc
 int bz2b200_rle1_split(bz2b200_ctx *ctx, const uint8_t *in, size_t n, int level, uint8_t *rle1_out, size_t rle1_cap,
                        uint64_t *rle1_off, uint64_t *in_off, uint32_t *crc, uint32_t cap_blocks, uint32_t *nblocks) {
     BZ_API_TRY
-    if (!ctx || (!in && n) || !rle1_out || !rle1_off || !in_off || !crc || !nblocks || level < 1 || level > 9)
+    int mode = BZ_MODE_REF;
+    if (!ctx || (!in && n) || !rle1_out || !rle1_off || !in_off || !crc || !nblocks || !bz_parse_level(&level, &mode))
         return BZ2B200_E_ARG;
     std::lock_guard<std::mutex> lk(ctx->mu);
+    ctx->mode = mode;
     if (cudaSetDevice(ctx->device) != cudaSuccess) return BZ2B200_E_CUDA;
     int rc = upload(ctx, in, n, ctx->d_in);
     if (rc) return rc;
@@ -359,8 +365,10 @@ int bz2b200_rle1_split(bz2b200_ctx *ctx, const uint8_t *in, size_t n, int level,
 int bz2b200_stream_plan(bz2b200_ctx *ctx, const uint8_t *in, size_t n, int level, uint64_t *block_start, uint32_t cap,
                         uint32_t *nblocks) {
     BZ_API_TRY
-    if (!ctx || (!in && n) || !block_start || !nblocks || level < 1 || level > 9) return BZ2B200_E_ARG;
+    int mode = BZ_MODE_REF;
+    if (!ctx || (!in && n) || !block_start || !nblocks || !bz_parse_level(&level, &mode)) return BZ2B200_E_ARG;
     std::lock_guard<std::mutex> lk(ctx->mu);
+    ctx->mode = mode;
     if (cudaSetDevice(ctx->device) != cudaSuccess) return BZ2B200_E_CUDA;
     // plan window by window; only the window being planned has to be resident
     size_t pos = 0;
@@ -391,12 +399,14 @@ int bz2b200_compress_range(bz2b200_ctx *ctx, const uint8_t *in, size_t n, int le
                            uint32_t nblocks_total, uint32_t first, uint32_t count, uint8_t *out, size_t out_cap,
                            uint64_t *out_bits, uint32_t *block_crcs) {
     BZ_API_TRY
-    if (!ctx || !in || !block_start || !out || !out_bits || !block_crcs || level < 1 || level > 9 ||
+    int mode = BZ_MODE_REF;
+    if (!ctx || !in || !block_start || !out || !out_bits || !block_crcs || !bz_parse_level(&level, &mode) ||
         first + count > nblocks_total)
         return BZ2B200_E_ARG;
     *out_bits = 0;
     if (count == 0) return BZ2B200_OK;
     std::lock_guard<std::mutex> lk(ctx->mu);
+    ctx->mode = mode;
     if (cudaSetDevice(ctx->device) != cudaSuccess) return BZ2B200_E_CUDA;
     size_t a = (size_t)block_start[first], b = (size_t)block_start[first + count];
     bool to_eof = (first + count == nblocks_total);
@@ -428,7 +438,8 @@ int bz2b200_merge_streams(int level, int nparts, const uint8_t *const *part, con
                           const uint32_t *const *part_crcs, const uint32_t *part_ncrc, uint8_t *out, size_t out_cap,
                           size_t *out_len) {
     BZ_API_TRY
-    if (level < 1 || level > 9 || nparts < 0 || !out || !out_len) return BZ2B200_E_ARG;
+    int mode = BZ_MODE_REF;
+    if (!bz_parse_level(&level, &mode) || nparts < 0 || !out || !out_len) return BZ2B200_E_ARG;
     u64 total = 32 + 80;
     for (int i = 0; i < nparts; i++) total += part_bits[i];
     size_t len = (size_t)((total + 7) / 8);
@@ -492,8 +503,10 @@ int bz2b200_merge_streams(int level, int nparts, const uint8_t *const *part, con
 extern "C" int bz2b200_stream_plan_dev(bz2b200_ctx *ctx, const uint8_t *d_in, size_t n, int level,
                                        uint64_t *block_start, uint32_t cap, uint32_t *nblocks) {
     BZ_API_TRY
-    if (!ctx || (!d_in && n) || !block_start || !nblocks || level < 1 || level > 9) return BZ2B200_E_ARG;
+    int mode = BZ_MODE_REF;
+    if (!ctx || (!d_in && n) || !block_start || !nblocks || !bz_parse_level(&level, &mode)) return BZ2B200_E_ARG;
     std::lock_guard<std::mutex> lk(ctx->mu);
+    ctx->mode = mode;
     if (cudaSetDevice(ctx->device) != cudaSuccess) return BZ2B200_E_CUDA;
     size_t pos = 0;
     u32 total = 0;
@@ -522,12 +535,14 @@ extern "C" int bz2b200_compress_range_dev(bz2b200_ctx *ctx, const uint8_t *d_in,
                                           uint32_t count, uint8_t *d_out, size_t out_cap, uint64_t *out_bits,
                                           uint32_t *block_crcs) {
     BZ_API_TRY
-    if (!ctx || !d_in || !block_start || !d_out || !out_bits || !block_crcs || level < 1 || level > 9 ||
+    int mode = BZ_MODE_REF;
+    if (!ctx || !d_in || !block_start || !d_out || !out_bits || !block_crcs || !bz_parse_level(&level, &mode) ||
         first + count > nblocks_total || ((uintptr_t)d_out & 3u))
         return BZ2B200_E_ARG;
     *out_bits = 0;
     if (count == 0) return BZ2B200_OK;
     std::lock_guard<std::mutex> lk(ctx->mu);
+    ctx->mode = mode;
     if (cudaSetDevice(ctx->device) != cudaSuccess) return BZ2B200_E_CUDA;
     size_t a = (size_t)block_start[first], b = (size_t)block_start[first + count];
     bool to_eof = (first + count == nblocks_total);

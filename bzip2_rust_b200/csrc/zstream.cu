@@ -27,6 +27,7 @@ int bz_concat_blocks(bz2b200_ctx *ctx, const HufOut &H, u32 nb, const u64 *hoff,
 struct bz2b200_zstream {
     bz2b200_ctx *ctx = nullptr;
     int level = 9;
+    int mode = BZ_MODE_REF;
     bz2b200_sink sink = nullptr;
     void *user = nullptr;
     size_t WF = 64u << 20;                   // fresh bytes per window
@@ -69,6 +70,7 @@ int emit(bz2b200_zstream *z, const u8 *p, size_t n) {
 int process(bz2b200_zstream *z, int slot, size_t len, bool eof) {
     bz2b200_ctx *ctx = z->ctx;
     std::lock_guard<std::mutex> lk(ctx->mu);
+    ctx->mode = z->mode;
     if (cudaSetDevice(ctx->device) != cudaSuccess) return BZ2B200_E_CUDA;
     cudaStream_t st = ctx->stream;
     const size_t W = z->tail_len + len;
@@ -183,10 +185,11 @@ extern "C" {
 
 int bz2b200_zstream_open(bz2b200_ctx *ctx, int level, bz2b200_sink sink, void *user, bz2b200_zstream **out) {
     BZ_API_TRY
-    if (!ctx || !sink || !out || level < 1 || level > 9) return BZ2B200_E_ARG;
+    int mode = BZ_MODE_REF;
+    if (!ctx || !sink || !out || !bz_parse_level(&level, &mode)) return BZ2B200_E_ARG;
     *out = nullptr;
     std::unique_ptr<bz2b200_zstream> z(new bz2b200_zstream());
-    z->ctx = ctx; z->level = level; z->sink = sink; z->user = user;
+    z->ctx = ctx; z->level = level; z->mode = mode; z->sink = sink; z->user = user;
     if (const char *e = getenv("BZ2B200_ZSTREAM_WINDOW_MB")) { int v = atoi(e); if (v >= 1 && v <= 1024) z->WF = (size_t)v << 20; }
     if (cudaSetDevice(ctx->device) != cudaSuccess) return BZ2B200_E_CUDA;
     for (int i = 0; i < 2; i++) if (z->stage[i].ensure(z->WF) != cudaSuccess) return BZ2B200_E_NOMEM;

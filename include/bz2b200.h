@@ -46,6 +46,19 @@ enum {
 
 #define BZ2B200_MAX_BLOCK 900000u   /* largest RLE1 block accepted (level 9: 899 986, rle1.rs:110) */
 
+/* libbz2-identical output: OR into `level` (level | BZ2B200_LIBBZ2) at every entry point that takes one --
+ * compress_stream(_dev), zstream_open, compress_stream_multi, stream_plan / compress_range (and _dev),
+ * shard_scan_dev / shard_plan_dev, rle1_split, merge_streams (which only writes the header digit).  The stream is then
+ * byte for byte what bzip2 1.0.8 writes through BZ2_bzCompress with BZ_RUN then BZ_FINISH (`bzip2 -<level>`, Python's
+ * bz2; not BZ2_bzBuffToBuffCompress, which keeps a last byte that fills a block in that block): libbz2's block cuts,
+ * its origin pointer for periodic blocks (where its fallbackSort leaves rotation 0), its initial table partition and its
+ * heap-built code lengths (DESIGN.md §10).  Known exception: a periodic block of 10000 bytes or more that libbz2's
+ * mainSort finishes within its work budget (a few long periods, e.g. u^3 with |u| = 4000); the stream then differs in
+ * that block's 24-bit origin pointer only and decodes to the same bytes.  Without the flag the output is the reference's, as before.  The level is
+ * level & 0xff and must be 1..9; any other bit set returns BZ2B200_E_ARG.  The per-block seams (compress_blocks,
+ * bwt_encode, huffman, mtf_rle2) take no level and always keep the reference's semantics. */
+#define BZ2B200_LIBBZ2 0x100u
+
 /* ---- context ---------------------------------------------------------------------------- */
 /* device < 0 selects the current CUDA device. */
 int  bz2b200_create(int device, bz2b200_ctx **out);

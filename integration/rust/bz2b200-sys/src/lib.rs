@@ -17,6 +17,8 @@ pub const BZ2B200_E_NOMEM: c_int = -4;
 pub const BZ2B200_E_FORMAT: c_int = -5;
 pub const BZ2B200_E_CRC: c_int = -6;
 pub const BZ2B200_MAX_BLOCK: u32 = 900_000;
+/// OR into `level` for the bytes bzip2 1.0.8 (libbz2) writes instead of the reference's.
+pub const BZ2B200_LIBBZ2: c_int = 0x100;
 pub const BZ2B200_REC_FOOTER: u32 = 1;
 pub const BZ2B200_REC_NO_MAGIC: u32 = 2;
 

@@ -1,12 +1,13 @@
 #!/usr/bin/env python
 """bz2b200 -- command line front end with the reference's flag surface (src/tools/cli.rs:113-303).
 
-    bz2b200_cli.py [-1..-9|--fast|--best] [-z|-d|-t] [-k] [-f] [-c] [-q] [-v] FILE...
+    bz2b200_cli.py [-1..-9|--fast|--best] [--libbz2] [-z|-d|-t] [-k] [-f] [-c] [-q] [-v] FILE...
     bz2b200_cli.py --recover [-f] [-c] [-q] FILE.bz2...
 
 Only block size (-1..-9), mode (-z/-d/-t) and the file list change the output, exactly as in the reference
 (compress.rs:50-55 reads only files[0] and block_size; this tool also accepts several files and stdin/stdout, which
-the reference advertises in its help text but does not implement, cli.rs:331-333).
+the reference advertises in its help text but does not implement, cli.rs:331-333).  --libbz2 compresses to the bytes
+bzip2 1.0.8 writes (`bzip2 -c -<level>`) instead of the reference's.
 Compression writes FILE.bz2 (compress.rs:59-60); decompression strips ".bz2" (the reference appends ".txt", an
 author's test convenience, decompress.rs:67-70 -- not reproduced).  Input files are ALWAYS kept, as in the reference
 (cli.rs:314 "-k --keep ... ALWAYS KEEPS"; compress.rs never reads keep_input_files): -k is accepted and changes nothing.
@@ -96,6 +97,8 @@ def main(argv=None):
     ap.add_argument("-t", "--test", dest="mode", action="store_const", const="t")
     ap.add_argument("--recover", dest="mode", action="store_const", const="r",
                     help="write the intact blocks of damaged archives to FILE.recovered and report the losses")
+    ap.add_argument("--libbz2", action="store_true",
+                    help="compress to exactly the bytes bzip2 1.0.8 (libbz2) writes for the same block size")
     ap.add_argument("-k", "--keep", action="store_true", help="keep input files (always the case, as in the reference)")
     ap.add_argument("-f", "--force", action="store_true", help="overwrite existing output files")
     ap.add_argument("-c", "--stdout", action="store_true", help="write to standard output")
@@ -134,7 +137,7 @@ def main(argv=None):
                 src = sys.stdin.buffer if name == "-" else open(name, "rb")
                 dst = sys.stdout.buffer if to_stdout else open(oname, "wb")
                 try:
-                    with bz.ZStream(eng, dst, level) as z:
+                    with bz.ZStream(eng, dst, level, libbz2=a.libbz2) as z:
                         while True:
                             piece = src.read(16 << 20)
                             if not piece:
