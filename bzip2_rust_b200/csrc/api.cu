@@ -30,7 +30,7 @@ bz2b200_ctx::~bz2b200_ctx() {
     for (int i = 0; i < 2; i++) { h_dstage[i].release(); h_dpiece[i].release(); h_rec[i].release(); }
     for (int i = 0; i < 8; i++) if (ev[i]) cudaEventDestroy(ev[i]);
     for (int i = 0; i < 2; i++) if (ev_dec[i]) cudaEventDestroy(ev_dec[i]);
-    for (int i = 0; i < 2; i++) if (ev_rec[i]) cudaEventDestroy(ev_rec[i]);
+    for (int i = 0; i < 2; i++) { if (ev_rec[i]) cudaEventDestroy(ev_rec[i]); if (ev_dpiece[i]) cudaEventDestroy(ev_dpiece[i]); }
     if (s_hi) cudaStreamDestroy(s_hi);
     for (cudaEvent_t e : ev_pool) cudaEventDestroy(e);
     for (cudaEvent_t e : up_ev) cudaEventDestroy(e);

@@ -5,6 +5,7 @@
 #include <stddef.h>
 #include <mutex>
 #include <string>
+#include <utility>
 #include <vector>
 #include <new>
 #include "../../include/bz2b200.h"
@@ -108,6 +109,9 @@ inline bool bz_parse_level(int *level, int *mode) {
     return true;
 }
 
+// A stream's combined CRC after one more block (crc.rs:25-27, bitwriter.rs:89-91)
+inline u32 bz_crc_step(u32 combined, u32 block_crc) { return ((combined << 1) | (combined >> 31)) ^ block_crc; }
+
 // Pending state of the three-phase sharding entry points (shard.cu): scan -> plan -> compress on one window.
 struct ShardPlan {
     bool scanned = false;
@@ -153,6 +157,7 @@ struct bz2b200_ctx {
     // ---- dstream (dstream.cu): window, batch outputs, staging and output pieces, kept for the next stream ----
     DevBuf d_dwin, d_ddec[2];
     PinBuf h_dstage[2], h_dpiece[2];
+    cudaEvent_t ev_dpiece[2] = {nullptr, nullptr};
     bool dstream_open = false;       // one dstream at a time uses them
     // ---- recovery (recover.cu): page-locked pieces of intact bytes on their way to the sink ----
     PinBuf h_rec[2];
@@ -359,6 +364,9 @@ struct DecGeom {
     u32 max_block, stride, sel_stride, max_sym, sym_stride, ch_stride;
     explicit DecGeom(u32 max_block);
 };
+// Longest span, in bits, a block of at most `max_block` bytes can have: 20 bits per symbol plus its header (symbol map,
+// selectors, six tables).  A damaged stream whose next magic is far away must not size the jump tables beyond it.
+constexpr u64 bz_dec_span_bits(u32 max_block) { return (u64)20 * (max_block + 64) + ((u64)1 << 19); }
 // (a) entropy decode of the candidates starting at bits `starts` of d_bits[0, n) (the data of candidate k does not
 // reach past rends[k] unless a chance magic cut it): header, group boundaries, symbols, inverse MTF -> the BWT
 // strings in ctx->d_T; db[k] = the candidate's DecTail (status 0 = parsed)
@@ -372,10 +380,49 @@ int bz_dec_unbwt(bz2b200_ctx *ctx, const DecGeom &g, u32 nblk, const u32 *hlen, 
 // -> crcs[k], valid after the next synchronisation of ctx->stream.  olen = the counted lengths with RLE1_OPEN replaced
 // by 0: such a member is not written.
 int bz_dec_write(bz2b200_ctx *ctx, const DecGeom &g, u32 nblk, const u64 *olen, const u64 *ooff, u8 *d_out, u32 *crcs);
-int bz_dec_candidates(bz2b200_ctx *ctx, const u8 *d_win, size_t len, u32 cap, std::vector<u64> &cand);
-// test knob BZ2B200_MULTI_DEC_CHANCE: spurious block candidates, as chance magics inside compressed data would be
-void bz_add_chance_candidates(std::vector<u64> &cand);
+// Makes d_win[0, len) ready for bz_decode_core: zeroes the 64 bytes behind it (word loads of the entropy stage read past
+// the last byte) and finds its magic candidates, at most len / bytes_per_cand + 64 of them (more: BZ2B200_E_FORMAT).
+// `chance` adds spurious block candidates, as chance magics inside compressed data would be (test knob
+// BZ2B200_MULTI_DEC_CHANCE).
+int bz_dec_prepare(bz2b200_ctx *ctx, u8 *d_win, size_t len, size_t bytes_per_cand, bool chance, std::vector<u64> &cand);
+// The whole input in[0, n) to ctx->d_in, prepared with at most n / 32 + 64 candidates
+int bz_dec_upload(bz2b200_ctx *ctx, const u8 *in, size_t n, bool chance, std::vector<u64> &cand);
 int bz_decode_core(bz2b200_ctx *ctx, const DecWindow &w, DecSink &sink, std::vector<DecEvent> &ev);
-// BZ2B200_E_FORMAT (and `err`) when a block of `ev` is longer than 100000 x its own stream's level; `level` = the first
-// stream's, for blocks before any stream event
-int bz_check_block_sizes(std::string &err, int level, const std::vector<DecEvent> &ev);
+
+// The rules over a chain of events: a block is at most 100000 x the level of its own stream's "BZh<level>", as libbz2
+// checks it, and each footer holds the fold of its stream's block CRCs.
+struct DecFold {
+    int level;                     // level of the current stream
+    u32 combined;                  // fold of the current stream's block CRCs so far
+    bool known;                    // `combined` covers the whole current stream
+};
+// Applies `ev` (chain order) to `f`: BZ2B200_E_FORMAT or BZ2B200_E_CRC, with `err` set, at the first event that breaks a rule
+int bz_dec_fold(DecFold &f, const std::vector<DecEvent> &ev, std::string &err);
+
+// Level (1..9) of the stream header "BZh<level>" at p[0, avail); 0 when it is not one (decompress.rs:46-62)
+inline int bz_header_level(const u8 *p, size_t avail) {
+    return avail >= 4 && p[0] == 'B' && p[1] == 'Z' && p[2] == 'h' && p[3] >= '1' && p[3] <= '9' ? p[3] - '0' : 0;
+}
+// 32 bits at bit offset `bit` of in[0, n), zero bits past n
+inline u32 bz_read32(const u8 *in, size_t n, u64 bit) {
+    const size_t byte = (size_t)(bit >> 3);
+    u64 v = 0;
+    for (size_t k = 0; k < 5; k++) v = (v << 8) | (byte + k < n ? in[byte + k] : 0);
+    return (u32)(v >> (8 - (bit & 7)));
+}
+constexpr u64 DEC_MAX_INPUT = 0xFFFFFF00ull * 4ull;   // largest input a whole-input decode accepts
+// Argument and header checks of bz2b200_decompress_stream and bz2b200_decompress_stream_multi (the caller checks its
+// context): BZ2B200_E_ARG, BZ2B200_E_FORMAT or BZ2B200_OK
+inline int bz_dec_check_input(const u8 *in, size_t n, const u8 *out, size_t out_cap, const size_t *out_len) {
+    if (!in || !out_len || (!out && out_cap) || n < 14 || n > DEC_MAX_INPUT) return BZ2B200_E_ARG;
+    return bz_header_level(in, n) ? BZ2B200_OK : BZ2B200_E_FORMAT;
+}
+
+// Device ranges of decoded bytes, in output order
+typedef std::vector<std::pair<const u8 *, u64>> DecRanges;
+constexpr size_t DEC_PIECE = 32u << 20;      // page-locked piece of output on its way to a sink
+// Downloads `ranges` on `st` through the two pieces buf[2] (ev[2]: their events, created on first use) and hands each
+// piece to `sink`: piece i downloads while the sink takes piece i - 1, across range boundaries too.  Synchronises `st`
+// before it returns, also after an error.  BZ2B200_E_ARG: the sink returned non-zero.  Sets no error text (the dstream's
+// delivery thread calls it without the context's lock).
+int bz_deliver_pieces(const DecRanges &ranges, cudaStream_t st, PinBuf *buf, cudaEvent_t *ev, bz2b200_sink sink, void *user);

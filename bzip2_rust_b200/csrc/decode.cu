@@ -515,6 +515,7 @@ int bz_dec_write(bz2b200_ctx *ctx, const DecGeom &g, u32 nblk, const u64 *olen, 
     return BZ2B200_OK;
 }
 
+namespace {
 // every bit offset of d_win[0, len) that looks like a block or footer magic, sorted; BZ2B200_E_FORMAT past `cap`
 int bz_dec_candidates(bz2b200_ctx *ctx, const u8 *d_win, size_t len, u32 cap, std::vector<u64> &cand) {
     cudaStream_t st = ctx->stream;
@@ -546,6 +547,21 @@ void bz_add_chance_candidates(std::vector<u64> &cand) {
     cand.insert(cand.end(), add.begin(), add.end());
     std::sort(cand.begin(), cand.end(), [](u64 x, u64 y) { return (x & ~DEC_FOOT) < (y & ~DEC_FOOT); });
 }
+}  // namespace
+
+int bz_dec_prepare(bz2b200_ctx *ctx, u8 *d_win, size_t len, size_t bytes_per_cand, bool chance, std::vector<u64> &cand) {
+    BZ_CHECK(cudaMemsetAsync(d_win + len, 0, 64, ctx->stream));
+    int rc = bz_dec_candidates(ctx, d_win, len, (u32)std::min<size_t>(len / bytes_per_cand + 64, 0x7fffff00u), cand);
+    if (rc) return rc;
+    if (chance) bz_add_chance_candidates(cand);
+    return BZ2B200_OK;
+}
+
+int bz_dec_upload(bz2b200_ctx *ctx, const u8 *in, size_t n, bool chance, std::vector<u64> &cand) {
+    BZ_CHECK(ctx->d_in.ensure(n + 64));
+    BZ_CHECK(cudaMemcpyAsync(ctx->d_in.p, in, n, cudaMemcpyHostToDevice, ctx->stream));
+    return bz_dec_prepare(ctx, ctx->d_in.as<u8>(), n, 32, chance, cand);
+}
 
 // A magic can also occur by chance inside entropy-coded data, and a file may hold several streams one after the other
 // (decompress.rs handles neither; libbz2 walks the blocks serially and accepts both).  So the candidates are only where
@@ -563,13 +579,6 @@ int bz_decode_core(bz2b200_ctx *ctx, const DecWindow &w, DecSink &sink, std::vec
     const DecGeom g(max_block);
     const u32 NB = DEC_BATCH;
     const u8 *d_bits = w.d_win;
-
-    auto read32 = [&](u64 bit) {                                // 32 bits at an absolute bit offset of the host input
-        size_t byte = (size_t)(bit >> 3); int sh = (int)(bit & 7);
-        u64 v = 0;
-        for (int k = 0; k < 5; k++) v = (v << 8) | (byte + k < w.n ? w.in[byte + k - w.in_lo] : 0);
-        return (u32)((v >> (8 - sh)) & 0xffffffffull);
-    };
     size_t ci = 0;                                              // next candidate to look at
     bool known = w.expect >= 0;                                 // the chain start is known
     u64 expect = known ? (u64)w.expect - lo8 : 0;               // bit offset where the next block / footer must start
@@ -587,16 +596,15 @@ int bz_decode_core(bz2b200_ctx *ctx, const DecWindow &w, DecSink &sink, std::vec
             while (ci < ncand && (cand[ci] & ~DEC_FOOT) < expect) ci++;
             if (ci == ncand || (cand[ci] & ~DEC_FOOT) != expect) { ctx->err = "decode: no block or footer magic at bit " + std::to_string(expect + lo8); return BZ2B200_E_FORMAT; }
             if (cand[ci] & DEC_FOOT) {                              // end of a stream: combined CRC, then end of input or another stream
-                const u32 stored = read32(expect + lo8 + 48);
+                // the footer's first byte is >= in_lo
+                const u32 stored = bz_read32(w.in, w.n - w.in_lo, expect + lo8 + 48 - (u64)w.in_lo * 8);
                 ev.push_back(DecEvent{expect + lo8, stored, 0, DEC_FOOTER});
                 if (comb_known && stored != combined) return BZ2B200_E_CRC;                    // enforced, unlike decompress.rs:394-402
                 size_t hb = (size_t)((expect + lo8 + 80 + 7) / 8);
                 if (hb == w.n) { sink.chain_end(DEC_ENDED); return BZ2B200_OK; }
-                const u8 *in = hb + 4 <= w.n ? w.in + (hb - w.in_lo) : nullptr;   // hb > the footer's first byte >= in_lo
-                if (!in || in[0] != 'B' || in[1] != 'Z' || in[2] != 'h' || in[3] < '1' || in[3] > '9') {
-                    ctx->err = "decode: trailing bytes after the stream footer"; return BZ2B200_E_FORMAT;
-                }
-                ev.push_back(DecEvent{(u64)hb * 8, (u32)(in[3] - '0'), 0, DEC_STREAM});
+                const int level = hb < w.n ? bz_header_level(w.in + (hb - w.in_lo), w.n - hb) : 0;
+                if (!level) { ctx->err = "decode: trailing bytes after the stream footer"; return BZ2B200_E_FORMAT; }
+                ev.push_back(DecEvent{(u64)hb * 8, (u32)level, 0, DEC_STREAM});
                 combined = 0; comb_known = true;
                 expect = (u64)hb * 8 + 32 - lo8;
                 continue;
@@ -615,9 +623,7 @@ int bz_decode_core(bz2b200_ctx *ctx, const DecWindow &w, DecSink &sink, std::vec
                 if (cand[k] & DEC_FOOT) continue;
                 if ((cand[k] & ~DEC_FOOT) >= hi) break;             // the next window's
                 u64 re = k + 1 < ncand ? (cand[k + 1] & ~DEC_FOOT) : (u64)n * 8;
-                // no valid block is longer than 20 bits per symbol plus its header (symbol map, selectors, six tables): a
-                // damaged stream whose next magic is far away must not size the jump tables
-                re = std::min<u64>(re, cand[k] + (u64)20 * (max_block + 64) + ((u64)1 << 19));
+                re = std::min<u64>(re, cand[k] + bz_dec_span_bits(max_block));
                 if (range_limit) re = std::min(re, cand[k] + range_limit);     // test knob: as if a chance magic cut the range
                 starts.push_back(cand[k]); rends.push_back(re);
             }
@@ -645,7 +651,7 @@ int bz_decode_core(bz2b200_ctx *ctx, const DecWindow &w, DecSink &sink, std::vec
             if (db[k].status != 0) { ctx->err = "decode: block at bit " + std::to_string(starts[k] + lo8) + " status " + std::to_string(db[k].status); return BZ2B200_E_FORMAT; }
             if (db[k].key >= db[k].nblock) { ctx->err = "decode: origin pointer outside the block"; return BZ2B200_E_FORMAT; }
             hlen[k] = db[k].nblock; hkey[k] = db[k].key; hrand[k] = db[k].pad;
-            combined = ((combined << 1) | (combined >> 31)) ^ db[k].crc;                       // crc.rs:25-27
+            combined = bz_crc_step(combined, db[k].crc);
             ev.push_back(DecEvent{starts[k] + lo8, db[k].crc, db[k].nblock, DEC_BLOCK});
             expect = db[k].end_bit;
             used = k + 1;
@@ -678,17 +684,37 @@ int bz_decode_core(bz2b200_ctx *ctx, const DecWindow &w, DecSink &sink, std::vec
     }
 }
 
-// Every block is at most 100000 x the level of ITS stream's "BZh<level>", as libbz2 checks it; the events are in chain
-// order and a stream's header event precedes its blocks.  `level` is the first stream's.
-int bz_check_block_sizes(std::string &err, int level, const std::vector<DecEvent> &ev) {
+int bz_dec_fold(DecFold &f, const std::vector<DecEvent> &ev, std::string &err) {
     for (const DecEvent &e : ev) {
-        if (e.kind == DEC_STREAM) level = (int)e.val;
-        else if (e.kind == DEC_BLOCK && e.nblock > (u32)level * 100000u) {
-            err = "decode: block at bit " + std::to_string(e.bit) + " longer than its stream's level allows";
-            return BZ2B200_E_FORMAT;
+        if (e.kind == DEC_BLOCK) {
+            if (e.nblock > (u32)f.level * 100000u) { err = "decode: block at bit " + std::to_string(e.bit) + " longer than its stream's level allows"; return BZ2B200_E_FORMAT; }
+            f.combined = bz_crc_step(f.combined, e.val);
+        } else if (e.kind == DEC_FOOTER) {
+            if (f.known && e.val != f.combined) { err = "decode: combined CRC mismatch at bit " + std::to_string(e.bit); return BZ2B200_E_CRC; }
+        } else {
+            f = DecFold{(int)e.val, 0, true};
         }
     }
     return BZ2B200_OK;
+}
+
+int bz_deliver_pieces(const DecRanges &ranges, cudaStream_t st, PinBuf *buf, cudaEvent_t *ev, bz2b200_sink sink, void *user) {
+    DecRanges pieces;
+    for (const auto &r : ranges)
+        for (u64 o = 0; o < r.second; o += DEC_PIECE) pieces.push_back({r.first + o, std::min<u64>(DEC_PIECE, r.second - o)});
+    int rc = BZ2B200_OK;
+    for (int i = 0; i < 2 && !pieces.empty() && !rc; i++)
+        if (buf[i].ensure(DEC_PIECE) != cudaSuccess ||
+            (!ev[i] && cudaEventCreateWithFlags(&ev[i], cudaEventDisableTiming) != cudaSuccess)) rc = BZ2B200_E_CUDA;
+    for (size_t i = 0; i <= pieces.size() && !rc; i++) {
+        if (i < pieces.size() &&            // the buffer's previous piece (i - 2) went to the sink in the last round
+            (cudaMemcpyAsync(buf[i & 1].p, pieces[i].first, (size_t)pieces[i].second, cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+             cudaEventRecord(ev[i & 1], st) != cudaSuccess)) rc = BZ2B200_E_CUDA;
+        else if (i > 0 && cudaEventSynchronize(ev[(i - 1) & 1]) != cudaSuccess) rc = BZ2B200_E_CUDA;
+        else if (i > 0 && sink(user, buf[(i - 1) & 1].as<u8>(), (size_t)pieces[i - 1].second) != 0) rc = BZ2B200_E_ARG;
+    }
+    if (cudaStreamSynchronize(st) != cudaSuccess && !rc) rc = BZ2B200_E_CUDA;   // also after an error: no copy may still write a piece
+    return rc;
 }
 
 namespace {
@@ -710,26 +736,22 @@ struct WholeSink : DecSink {
 extern "C" int bz2b200_decompress_stream(bz2b200_ctx *ctx, const uint8_t *in, size_t n, uint8_t *out, size_t out_cap,
                                          size_t *out_len) {
     BZ_API_TRY
-    if (!ctx || !in || !out_len || (!out && out_cap) || n < 14 || n > 0xFFFFFF00ull * 4ull) return BZ2B200_E_ARG;
-    if (in[0] != 'B' || in[1] != 'Z' || in[2] != 'h' || in[3] < '1' || in[3] > '9') return BZ2B200_E_FORMAT;   // decompress.rs:46-62
+    if (!ctx) return BZ2B200_E_ARG;
+    int rc = bz_dec_check_input(in, n, out, out_cap, out_len);
+    if (rc) return rc;
     std::lock_guard<std::mutex> lk(ctx->mu);
     if (cudaSetDevice(ctx->device) != cudaSuccess) return BZ2B200_E_CUDA;
-    cudaStream_t st = ctx->stream;
     *out_len = 0;
-    BZ_CHECK(ctx->d_in.ensure(n + 64));
-    BZ_CHECK(cudaMemcpyAsync(ctx->d_in.p, in, n, cudaMemcpyHostToDevice, st));
-    BZ_CHECK(cudaMemsetAsync(ctx->d_in.as<u8>() + n, 0, 64, st));       // word loads of the entropy stage read past the last byte
     // ---- 1. every bit offset that looks like a block or footer magic ----
     std::vector<u64> cand;
-    int rc = bz_dec_candidates(ctx, ctx->d_in.as<u8>(), n, (u32)std::min<size_t>(n / 32 + 64, 0x7fffff00u), cand);
+    rc = bz_dec_upload(ctx, in, n, false, cand);
     if (rc) return rc;
     if (cand.empty()) return BZ2B200_E_FORMAT;
     int level = in[3] - '0';
     for (u64 c : cand) {                                        // buffer geometry: the largest block size any header may announce
         if (!(c & DEC_FOOT)) continue;
         size_t hb = (size_t)(((c & ~DEC_FOOT) + 80 + 7) / 8);
-        if (hb + 4 <= n && in[hb] == 'B' && in[hb + 1] == 'Z' && in[hb + 2] == 'h' && in[hb + 3] >= '1' && in[hb + 3] <= '9')
-            level = std::max(level, in[hb + 3] - '0');
+        if (hb < n) level = std::max(level, bz_header_level(in + hb, n - hb));
     }
     DecWindow w{in, 0, n, ctx->d_in.as<u8>(), 0, n, ~0ull, 32, 0, (u32)level * 100000u, &cand};
     WholeSink sink;
@@ -737,7 +759,8 @@ extern "C" int bz2b200_decompress_stream(bz2b200_ctx *ctx, const uint8_t *in, si
     std::vector<DecEvent> ev;
     rc = bz_decode_core(ctx, w, sink, ev);
     if (rc) return rc;
-    rc = bz_check_block_sizes(ctx->err, in[3] - '0', ev);
+    DecFold fold{in[3] - '0', 0, true};
+    rc = bz_dec_fold(fold, ev, ctx->err);
     if (rc) return rc;
     *out_len = sink.total;
     return BZ2B200_OK;

@@ -10,15 +10,15 @@
 //                    on one piece while the next one downloads and the next batch decodes
 // so reading the input overlaps upload and kernels, and the sink's writing overlaps download and kernels.
 // Window edges depend only on absolute input positions: window k ends at byte (k + 1) * WF (or at the input's end).
-// LOOK (4 MiB) exceeds the bound on a block's span, 20 x (900000 + 64) + 2^19 bits ~ 2.3 MB, so an element that starts
-// before the edge ends inside the window, and a footer before the edge is never taken for the end of the input.
+// LOOK (4 MiB) exceeds the bound on a block's span (bz_dec_span_bits, ~2.3 MB), so an element that starts before the edge
+// ends inside the window, and a footer before the edge is never taken for the end of the input.
 // The bytes from where the chain leaves the window onward (at most LOOK + 1) are carried in front of the next window;
 // a window whose edge is not past the chain's start is carried whole and waits for more input.
 // The chain's start and the stream's running combined CRC are always known here, so every footer's combined CRC is
-// checked when it is reached.  Blocks are decoded with level-9 geometry; the rule that a block is at most 100000 x the
-// level of its own stream's header is applied to each window's blocks once the window is decoded.  Host memory is the
-// staging buffers and the output pieces whatever the input or output size; device memory is the decode workspaces, one
-// window and two batch outputs.  In test mode (no sink) nothing is downloaded.
+// checked when it is reached.  Blocks are decoded with level-9 geometry; the rules over the chain (bz_dec_fold) are
+// applied to each window's events once the window is decoded.  Host memory is the staging buffers and the output pieces
+// whatever the input or output size; device memory is the decode workspaces, one window and two batch outputs.  In test
+// mode (no sink) nothing is downloaded.
 #include "common.cuh"
 #include <algorithm>
 #include <condition_variable>
@@ -30,9 +30,8 @@
 
 namespace {
 const size_t LOOK = 4u << 20;            // look-ahead behind a window's decode edge (the multi decoder's)
+static_assert((u64)LOOK * 8 > bz_dec_span_bits(BZ2B200_MAX_BLOCK), "an element that starts before the edge ends in the window");
 const size_t PREFIX = LOOK + 64;         // room in front of each staging buffer for the carried tail
-const size_t PIECE = 32u << 20;          // page-locked output piece
-inline u32 crc_step(u32 s, u32 b) { return ((s << 1) | (s >> 31)) ^ b; }   // crc.rs:25-27
 }  // namespace
 
 struct bz2b200_dstream {
@@ -57,16 +56,13 @@ struct bz2b200_dstream {
     u64 queued = 0, delivered = 0;           // batches handed to / finished by the delivery thread
     bool out_quit = false;
     bool out_failed = false;                 // the sink or a download failed: the sink receives nothing more
-    PinBuf *piece = nullptr;                 // [2] (the context's)
-    cudaEvent_t ev_piece[2] = {nullptr, nullptr};
     // worker state
     DevBuf *d_win = nullptr, *d_dec = nullptr;   // the context's: one window, two batch outputs ([2])
     u64 nbatch = 0;                          // batches counted so far (d_dec[nbatch & 1] is the next one's)
     size_t tail_len = 0; u64 tail_lo = 0;    // carried bytes in front of the next staging buffer, and their input offset
     long long expect = 32;                   // absolute bit where the next chain element starts
-    u32 combined = 0;                        // running combined CRC of the current stream
+    DecFold fold{0, 0, true};                // the chain's rules so far (level 0: no window decoded yet)
     bool ended = false;                      // the chain ended after the input's last footer
-    int level = 0;                           // level of the current stream's header (0: none seen yet)
     std::vector<u64> cand;
     std::vector<DecEvent> ev;
     u64 total_in = 0, total_out = 0;
@@ -125,37 +121,27 @@ int process(bz2b200_dstream *d, int slot, size_t len, bool eof) {
     const u8 *h = d->stage[slot].as<u8>() + PREFIX - d->tail_len;
     const size_t W = d->tail_len + len;
     const u64 lo = d->tail_lo, end = lo + W;
-    if (d->level == 0) {                                        // the first window (>= 1024 bytes unless it is the last)
+    if (d->fold.level == 0) {                                   // the first window (>= 1024 bytes unless it is the last)
         if (eof && d->total_in < 14) { ctx->err = "the input is shorter than 14 bytes"; return BZ2B200_E_FORMAT; }
-        if (h[0] != 'B' || h[1] != 'Z' || h[2] != 'h' || h[3] < '1' || h[3] > '9') { ctx->err = "the input does not start with BZh<level>"; return BZ2B200_E_FORMAT; }
-        d->level = h[3] - '0';
+        d->fold.level = bz_header_level(h, W);
+        if (!d->fold.level) { ctx->err = "the input does not start with BZh<level>"; return BZ2B200_E_FORMAT; }
     }
     const u64 hi = eof ? ~0ull : (end > LOOK ? (u64)(end - LOOK) * 8 : 0);
     if (!eof && hi <= (u64)d->expect) return carry(d, slot, h, lo, W, (u64)d->expect / 8);   // wait for more input
     BZ_CHECK(d->d_win->ensure(W + 64));
     u8 *dw = d->d_win->as<u8>();
     BZ_CHECK(cudaMemcpyAsync(dw, h, W, cudaMemcpyHostToDevice, st));
-    BZ_CHECK(cudaMemsetAsync(dw + W, 0, 64, st));              // word loads of the entropy stage read past the last byte
     // at most one magic per 32 bits whatever the data: a window is never refused where the whole input is accepted
-    int rc = bz_dec_candidates(ctx, dw, W, (u32)std::min<size_t>(W / 4 + 64, 0x7fffff00u), d->cand);
+    int rc = bz_dec_prepare(ctx, dw, W, 4, d->chance, d->cand);
     if (rc) return rc;
-    if (d->chance) bz_add_chance_candidates(d->cand);
-    DecWindow w{h, (size_t)lo, (size_t)end, dw, (size_t)lo, W, hi, d->expect, d->combined, BZ2B200_MAX_BLOCK, &d->cand};
+    DecWindow w{h, (size_t)lo, (size_t)end, dw, (size_t)lo, W, hi, d->expect, d->fold.combined, BZ2B200_MAX_BLOCK, &d->cand};
     DSink sink;
     sink.d = d; sink.ctx = ctx;
     d->ev.clear();
     rc = bz_decode_core(ctx, w, sink, d->ev);
     if (rc) return rc;
-    rc = bz_check_block_sizes(ctx->err, d->level, d->ev);
+    rc = bz_dec_fold(d->fold, d->ev, ctx->err);
     if (rc) return rc;
-    for (const DecEvent &e : d->ev) {
-        if (e.kind == DEC_BLOCK) {
-            d->combined = crc_step(d->combined, e.val);
-        } else if (e.kind == DEC_STREAM) {
-            d->combined = 0;
-            d->level = (int)e.val;
-        }
-    }
     if (eof) {
         if (sink.end != DEC_ENDED) { ctx->err = "decode: the input does not end with a stream footer"; return BZ2B200_E_FORMAT; }
         d->ended = true;
@@ -188,28 +174,6 @@ void worker(bz2b200_dstream *d) {
     }
 }
 
-// one batch to the sink: piece i downloads while the sink takes piece i - 1
-int deliver(bz2b200_dstream *d, const u8 *src, u64 n) {
-    cudaStream_t s = d->ctx->s_down;
-    int rc = BZ2B200_OK;
-    u64 prev = 0;
-    for (u64 off = 0, i = 0; off < n || prev; i++) {
-        u64 sz = std::min<u64>(PIECE, n - off);
-        if (sz) {
-            if (cudaMemcpyAsync(d->piece[i & 1].p, src + off, (size_t)sz, cudaMemcpyDeviceToHost, s) != cudaSuccess ||
-                cudaEventRecord(d->ev_piece[i & 1], s) != cudaSuccess) { rc = BZ2B200_E_CUDA; break; }
-            off += sz;
-        }
-        if (prev) {
-            if (cudaEventSynchronize(d->ev_piece[(i - 1) & 1]) != cudaSuccess) { rc = BZ2B200_E_CUDA; break; }
-            if (d->sink(d->user, d->piece[(i - 1) & 1].as<u8>(), (size_t)prev) != 0) { rc = BZ2B200_E_ARG; break; }
-        }
-        prev = sz;
-    }
-    cudaStreamSynchronize(s);                                   // also after an error: the pieces stay untouched
-    return rc;
-}
-
 void delivery(bz2b200_dstream *d) {
     cudaSetDevice(d->ctx->device);
     for (;;) {
@@ -222,7 +186,8 @@ void delivery(bz2b200_dstream *d) {
             j = d->jobs.front(); d->jobs.pop_front();
             skip = d->out_failed;       // a decode error leaves the batches checked before it to be delivered
         }
-        int rc = skip ? BZ2B200_OK : deliver(d, j.d, j.n);
+        bz2b200_ctx *ctx = d->ctx;
+        int rc = skip ? BZ2B200_OK : bz_deliver_pieces({{j.d, j.n}}, ctx->s_down, ctx->h_dpiece, ctx->ev_dpiece, d->sink, d->user);
         {
             std::lock_guard<std::mutex> lk(d->mu);
             if (rc) d->out_failed = true;
@@ -263,7 +228,6 @@ void finish(bz2b200_dstream *d) {
     cudaSetDevice(ctx->device);
     cudaStreamSynchronize(ctx->stream);
     if (ctx->s_hi) cudaStreamSynchronize(ctx->s_hi);
-    for (int i = 0; i < 2; i++) if (d->ev_piece[i]) cudaEventDestroy(d->ev_piece[i]);
     std::lock_guard<std::mutex> lk(ctx->mu);
     ctx->dstream_open = false;
 }
@@ -283,17 +247,14 @@ int bz2b200_dstream_open(bz2b200_ctx *ctx, bz2b200_sink sink, void *user, bz2b20
         ctx->dstream_open = true;
     }
     d->ctx = ctx; d->sink = sink; d->user = user;
-    d->stage = ctx->h_dstage; d->piece = ctx->h_dpiece; d->d_win = &ctx->d_dwin; d->d_dec = ctx->d_ddec;
+    d->stage = ctx->h_dstage; d->d_win = &ctx->d_dwin; d->d_dec = ctx->d_ddec;
     if (const char *e = getenv("BZ2B200_DSTREAM_WINDOW")) { long long v = atoll(e); if (v >= 1024 && v <= (1ll << 30)) d->WF = (size_t)v; }
     d->chance = getenv("BZ2B200_MULTI_DEC_CHANCE") != nullptr;
     int rc = cudaSetDevice(ctx->device) != cudaSuccess ? BZ2B200_E_CUDA : BZ2B200_OK;
     for (int i = 0; i < 2 && !rc; i++) if (d->stage[i].ensure(PREFIX + d->WF) != cudaSuccess) rc = BZ2B200_E_NOMEM;
     if (sink && !rc) {
         std::lock_guard<std::mutex> lk(ctx->mu);
-        for (int i = 0; i < 2 && !rc; i++) {
-            if (d->piece[i].ensure(PIECE) != cudaSuccess) rc = BZ2B200_E_NOMEM;
-            else if (cudaEventCreateWithFlags(&d->ev_piece[i], cudaEventDisableTiming) != cudaSuccess) rc = BZ2B200_E_CUDA;
-        }
+        for (int i = 0; i < 2 && !rc; i++) if (ctx->h_dpiece[i].ensure(DEC_PIECE) != cudaSuccess) rc = BZ2B200_E_NOMEM;
         if (!rc && !ctx->s_up &&
             (cudaStreamCreateWithFlags(&ctx->s_up, cudaStreamNonBlocking) != cudaSuccess ||
              cudaStreamCreateWithFlags(&ctx->s_down, cudaStreamNonBlocking) != cudaSuccess)) rc = BZ2B200_E_CUDA;

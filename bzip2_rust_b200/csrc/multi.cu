@@ -117,6 +117,7 @@ int rank_fail(bz2b200_mctx *m, MRank &R, int rc, const char *what) {
 #define MCHECK(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { R.rc = BZ2B200_E_CUDA; R.err = std::string(#call) + ": " + cudaGetErrorString(e_); m->abort.store(1); return R.rc; } } while (0)
 
 const size_t LOOK0 = 4u << 20;               // look-ahead for the last block of a window, grown on demand
+static_assert((u64)LOOK0 * 8 > bz_dec_span_bits(BZ2B200_MAX_BLOCK), "a block that starts in a decode window ends in its upload");
 inline size_t chunk_bytes() {
     static const size_t c = [] { const char *e = getenv("BZ2B200_E2E_CHUNK_MB"); int v = e ? atoi(e) : 8; return (size_t)(v < 1 ? 1 : v) << 20; }();
     return c;
@@ -355,13 +356,11 @@ int run_dec_window(bz2b200_mctx *m, int r, size_t k, int slot) {
         std::lock_guard<std::mutex> lk(ctx->mu);
         ctx->err.clear();
         MCHECK(cudaStreamWaitEvent(ctx->stream, W.ev_up, 0));
-        MCHECK(cudaMemsetAsync(d + len, 0, 64, ctx->stream));  // word loads of the entropy stage read past the last byte
         std::vector<u64> cand;
         // at most one magic per 32 bits whatever the data: a window is never refused where the whole input is accepted
-        rc = bz_dec_candidates(ctx, d, len, (u32)std::min<size_t>(len / 4 + 64, 0x7fffff00u), cand);
+        rc = bz_dec_prepare(ctx, d, len, 4, chance, cand);
         t_scan = ms_since(t0);
         if (!rc) {
-            if (chance) bz_add_chance_candidates(cand);
             // level-9 geometry: the headers of later windows are not known yet; the calling thread applies the block
             // size they allow
             DecWindow w{m->in, 0, m->nbytes, d, W.lo, len, k + 1 == nwin ? ~0ull : (u64)W.hi * 8, k == 0 ? 32ll : -1ll,
@@ -431,8 +430,6 @@ void worker(bz2b200_mctx *m, int r) {
         m->cv_done.notify_all();
     }
 }
-
-inline u32 crc_step(u32 s, u32 b) { return ((s << 1) | (s >> 31)) ^ b; }   // crc.rs:25-27
 
 }  // namespace
 
@@ -555,7 +552,7 @@ int bz2b200_compress_stream_multi(bz2b200_mctx *m, const uint8_t *in, size_t n, 
             if (W->seam) out[W->byte_lo] |= W->first_byte;
             pos += W->bits;
         }
-        for (u32 c : W->crcs) combined = crc_step(combined, c);            // bitwriter.rs:89-91
+        for (u32 c : W->crcs) combined = bz_crc_step(combined, c);         // bitwriter.rs:89-91
     }
     out[0] = 'B'; out[1] = 'Z'; out[2] = 'h'; out[3] = (u8)('0' + lv);  // bitwriter.rs:67-72
     size_t len = (size_t)((pos + 80 + 7) / 8);
@@ -588,15 +585,16 @@ int bz2b200_compress_stream_multi(bz2b200_mctx *m, const uint8_t *in, size_t n, 
 int bz2b200_decompress_stream_multi(bz2b200_mctx *m, const uint8_t *in, size_t n, uint8_t *out, size_t out_cap,
                                     size_t *out_len) {
     BZ_API_TRY
-    if (!m || !in || !out_len || (!out && out_cap) || n < 14 || n > 0xFFFFFF00ull * 4ull) return BZ2B200_E_ARG;
-    if (in[0] != 'B' || in[1] != 'Z' || in[2] != 'h' || in[3] < '1' || in[3] > '9') return BZ2B200_E_FORMAT;
+    if (!m) return BZ2B200_E_ARG;
+    int rc = bz_dec_check_input(in, n, out, out_cap, out_len);
+    if (rc) return rc;
     std::lock_guard<std::mutex> call(m->call_mu);
     *out_len = 0;
     size_t win = std::min(DEC_WIN_MAX, std::max(DEC_WIN_MIN, ((n + 2 * (size_t)m->n - 1) / (2 * (size_t)m->n) + 4095) & ~(size_t)4095));
     if (const char *e = getenv("BZ2B200_MULTI_DEC_WINDOW")) { long long v = atoll(e); if (v >= 1024) win = (size_t)v; }
     // small inputs (or one device): the single-GPU path
     if (m->n == 1 || n < 2 * win) {
-        int rc = bz2b200_decompress_stream(m->rk[0]->ctx, in, n, out, out_cap, out_len);
+        rc = bz2b200_decompress_stream(m->rk[0]->ctx, in, n, out, out_cap, out_len);
         // That call stops at the first batch that does not fit; the caller is owed the exact size, so the input is decoded
         // again into scratch memory (growing twofold while it does not fit) to learn it.  A defect behind the point where
         // the first call stopped does not change the code: it stays E_CAP, with the size the first call reported.
@@ -646,23 +644,13 @@ int bz2b200_decompress_stream_multi(bz2b200_mctx *m, const uint8_t *in, size_t n
     // Every block is bounded by 100000 x the level of its own stream's header, as in libbz2 (windows decode with level-9
     // buffers).  With several defects in one input the code returned may be E_FORMAT where the single-GPU call returns
     // E_CRC or the reverse.
-    int level = in[3] - '0';
-    u32 combined = 0;
-    bool fold = true;                                           // `combined` covers the whole stream so far
+    DecFold fold{in[3] - '0', 0, true};
     u64 total = 0;
     for (auto &W : m->win) {
-        for (const DecEvent &e : W->events) {
-            if (e.kind == DEC_BLOCK) {
-                if (e.nblock > (u32)level * 100000u) { m->err = "decode: block at bit " + std::to_string(e.bit) + " longer than its stream's level allows"; return BZ2B200_E_FORMAT; }
-                combined = crc_step(combined, e.val);
-            } else if (e.kind == DEC_FOOTER) {
-                if (fold && e.val != combined) { m->err = "decode: combined CRC mismatch at bit " + std::to_string(e.bit); return BZ2B200_E_CRC; }
-            } else {
-                combined = 0; fold = true; level = (int)e.val;
-            }
-        }
+        rc = bz_dec_fold(fold, W->events, m->err);
+        if (rc) return rc;
         if (W->rc < 0) { m->err = W->err; return W->rc; }
-        if (W->rc) fold = false;                                // stopped early: its events are incomplete
+        if (W->rc) fold.known = false;                          // stopped early: its events are incomplete
         total += W->out_len;
     }
     for (auto &R : m->rk) if (R->rc) { m->err = "rank failed: " + R->err; return R->rc; }

@@ -11,64 +11,24 @@
 // part), that bit is decoded as a block anyway, before the candidates after it: the batch is cut after the intact block,
 // and the next batch is [that bit, the candidates after it].  The cut re-decodes the members behind it, which costs time
 // on damaged inputs only.
-// Intact bytes leave a batch in input order, copied down in page-locked pieces of 32 MiB (two, kept by the context):
-// piece i downloads while the sink takes piece i - 1 on the calling thread.
+// Intact bytes leave a batch in input order through bz_deliver_pieces, in the context's two page-locked pieces of
+// recovery: piece i downloads while the sink takes piece i - 1 on the calling thread.
 #include "common.cuh"
 #include <algorithm>
 #include <stdlib.h>
-#include <utility>
-
-namespace {
-const size_t PIECE = 32u << 20;
-inline u32 crc_step(u32 s, u32 b) { return ((s << 1) | (s >> 31)) ^ b; }   // crc.rs:25-27
-
-typedef std::vector<std::pair<const u8 *, u64>> Runs;   // device ranges of intact bytes, in input order
-
-int deliver(bz2b200_ctx *ctx, const Runs &runs, bz2b200_sink sink, void *user) {
-    cudaStream_t st = ctx->stream;
-    Runs pieces;
-    for (const auto &r : runs)
-        for (u64 o = 0; o < r.second; o += PIECE) pieces.push_back({r.first + o, std::min<u64>(PIECE, r.second - o)});
-    if (pieces.empty()) return BZ2B200_OK;
-    for (int i = 0; i < 2; i++) {
-        BZ_CHECK(ctx->h_rec[i].ensure(PIECE));
-        if (!ctx->ev_rec[i]) BZ_CHECK(cudaEventCreateWithFlags(&ctx->ev_rec[i], cudaEventDisableTiming));
-    }
-    int rc = BZ2B200_OK;
-    for (size_t i = 0; i <= pieces.size(); i++) {
-        if (i < pieces.size()) {            // the buffer's previous piece (i - 2) went to the sink in the last round
-            BZ_CHECK(cudaMemcpyAsync(ctx->h_rec[i & 1].p, pieces[i].first, (size_t)pieces[i].second, cudaMemcpyDeviceToHost, st));
-            BZ_CHECK(cudaEventRecord(ctx->ev_rec[i & 1], st));
-        }
-        if (i > 0) {
-            BZ_CHECK(cudaEventSynchronize(ctx->ev_rec[(i - 1) & 1]));
-            if (sink(user, ctx->h_rec[(i - 1) & 1].as<u8>(), (size_t)pieces[i - 1].second) != 0) {
-                ctx->err = "recover: the sink reported an error"; rc = BZ2B200_E_ARG; break;
-            }
-        }
-    }
-    BZ_CHECK(cudaStreamSynchronize(st));    // also after an error: no copy may still write a piece
-    return rc;
-}
-
-}  // namespace
 
 extern "C" int bz2b200_recover(bz2b200_ctx *ctx, const uint8_t *in, size_t n, bz2b200_sink sink, void *user,
                                bz2b200_rec_entry *ent, uint32_t ent_cap, uint32_t *nent, uint64_t *total_out) {
     BZ_API_TRY
-    if (!ctx || !in || n == 0 || !nent || !total_out || (!ent && ent_cap) || n > 0xFFFFFF00ull * 4ull) return BZ2B200_E_ARG;
+    if (!ctx || !in || n == 0 || !nent || !total_out || (!ent && ent_cap) || n > DEC_MAX_INPUT) return BZ2B200_E_ARG;
     *nent = 0; *total_out = 0;
     std::lock_guard<std::mutex> lk(ctx->mu);
     if (cudaSetDevice(ctx->device) != cudaSuccess) return BZ2B200_E_CUDA;
     cudaStream_t st = ctx->stream;
-    BZ_CHECK(ctx->d_in.ensure(n + 64));
-    BZ_CHECK(cudaMemcpyAsync(ctx->d_in.p, in, n, cudaMemcpyHostToDevice, st));
-    BZ_CHECK(cudaMemsetAsync(ctx->d_in.as<u8>() + n, 0, 64, st));       // word loads of the entropy stage read past the last byte
-    const u8 *d_bits = ctx->d_in.as<u8>();
     std::vector<u64> cand;
-    int rc = bz_dec_candidates(ctx, d_bits, n, (u32)std::min<size_t>(n / 32 + 64, 0x7fffff00u), cand);
+    int rc = bz_dec_upload(ctx, in, n, getenv("BZ2B200_MULTI_DEC_CHANCE") != nullptr, cand);
     if (rc) return rc;
-    if (getenv("BZ2B200_MULTI_DEC_CHANCE")) bz_add_chance_candidates(cand);
+    const u8 *d_bits = ctx->d_in.as<u8>();
     const size_t ncand = cand.size();
     const u64 nbits = (u64)n * 8;
     const DecGeom g(BZ2B200_MAX_BLOCK);
@@ -76,12 +36,6 @@ extern "C" int bz2b200_recover(bz2b200_ctx *ctx, const uint8_t *in, size_t n, bz
     auto at = [&](size_t k) { return cand[k] & ~DEC_FOOT; };
     auto first_at_or_after = [&](u64 bit) {
         return (size_t)(std::lower_bound(cand.begin(), cand.end(), bit, [](u64 c, u64 b) { return (c & ~DEC_FOOT) < b; }) - cand.begin());
-    };
-    auto read32 = [&](u64 bit) {                                // 32 bits at a bit offset of the input
-        size_t byte = (size_t)(bit >> 3); int sh = (int)(bit & 7);
-        u64 v = 0;
-        for (int k = 0; k < 5; k++) v = (v << 8) | (byte + k < n ? in[byte + k] : 0);
-        return (u32)((v >> (8 - sh)) & 0xffffffffull);
     };
 
     u32 count = 0;                                              // entries found (written while below ent_cap)
@@ -109,7 +63,7 @@ extern "C" int bz2b200_recover(bz2b200_ctx *ctx, const uint8_t *in, size_t n, bz
         for (u32 m = 0; m < nb; m++) {                          // as in bz_decode_core: up to the next candidate, bounded
             size_t k = first_at_or_after(starts[m] + 1);
             u64 re = k < ncand ? at(k) : nbits;
-            rends.push_back(std::min<u64>(re, starts[m] + (u64)20 * (g.max_block + 64) + ((u64)1 << 19)));
+            rends.push_back(std::min<u64>(re, starts[m] + bz_dec_span_bits(g.max_block)));
         }
         // ---- the two decode steps on every member; verdicts ----
         u32 nblk = 0;
@@ -142,7 +96,7 @@ extern "C" int bz2b200_recover(bz2b200_ctx *ctx, const uint8_t *in, size_t n, bz
                 if (status[m] == BZ2B200_OK && crcs[m] != db[m].crc) status[m] = BZ2B200_E_CRC;
         }
         // ---- entries in input order; an intact block without a magic at its end cuts the batch there ----
-        Runs runs;
+        DecRanges runs;
         size_t next_pos = kend;
         long long next_rescue = -1;
         auto block = [&](u32 m, u32 flags) {                   // true: the batch is cut after this member
@@ -152,7 +106,7 @@ extern "C" int bz2b200_recover(bz2b200_ctx *ctx, const uint8_t *in, size_t n, bz
             const bool ok = status[m] == BZ2B200_OK;
             emit(bz2b200_rec_entry{b, db[m].status == 0 ? db[m].end_bit : 0, out_total, ok ? (u32)olen[m] : 0u, db[m].crc,
                                    status[m], flags});
-            comb = crc_step(comb, db[m].crc);
+            comb = bz_crc_step(comb, db[m].crc);
             stream_ok &= ok;
             if (!ok) return false;
             const u64 e = db[m].end_bit;
@@ -171,7 +125,7 @@ extern "C" int bz2b200_recover(bz2b200_ctx *ctx, const uint8_t *in, size_t n, bz
             if (cand[k] & DEC_FOOT) {
                 const u64 b = at(k);
                 if (b < cover) continue;                        // a chance magic inside an intact block
-                const u32 stored = read32(b + 48);
+                const u32 stored = bz_read32(in, n, b + 48);
                 const int s = !stream_ok ? BZ2B200_E_FORMAT : comb != stored ? BZ2B200_E_CRC : BZ2B200_OK;
                 emit(bz2b200_rec_entry{b, b + 80, out_total, 0u, stored, s, BZ2B200_REC_FOOTER});
                 comb = 0; stream_ok = true;
@@ -180,8 +134,8 @@ extern "C" int bz2b200_recover(bz2b200_ctx *ctx, const uint8_t *in, size_t n, bz
             }
         }
         if (sink) {
-            rc = deliver(ctx, runs, sink, user);
-            if (rc) return rc;
+            rc = bz_deliver_pieces(runs, st, ctx->h_rec, ctx->ev_rec, sink, user);
+            if (rc) { ctx->err = rc == BZ2B200_E_ARG ? "recover: the sink reported an error" : "recover: download of intact bytes failed"; return rc; }
         }
         pos = next_pos; rescue = next_rescue;
     }

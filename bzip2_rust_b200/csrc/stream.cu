@@ -55,8 +55,6 @@ __global__ void k_header_footer(u32 *dst, int level, u64 pos, u32 combined, int 
     }
 }
 
-inline u32 stream_crc_step(u32 s, u32 b) { return ((s << 1) | (s >> 31)) ^ b; }   // crc.rs:25-27
-
 constexpr size_t WINDOW = 256u << 20;       // input bytes planned per pass
 constexpr u32 MAX_BATCH_BLOCKS = 4096;
 constexpr size_t MAX_BATCH_BYTES = 272u << 20;   // RLE1 bytes per BWT batch (workspace ~40 B per byte)
@@ -182,7 +180,7 @@ static int compress_core(bz2b200_ctx *ctx, const u8 *d_in, size_t n, int level, 
             hoff[k] = bitpos;
             bitpos += hbits[k];
             maxbits = std::max(maxbits, hbits[k]);
-            combined = stream_crc_step(combined, hcrc[k]);      // bitwriter.rs:89-91
+            combined = bz_crc_step(combined, hcrc[k]);   // bitwriter.rs:89-91
             if (crcs_out) crcs_out->push_back(hcrc[k]);
         }
         if ((bitpos + 80 + 7) / 8 + 8 > out_cap) return BZ2B200_E_CAP;
@@ -449,7 +447,7 @@ int bz2b200_merge_streams(int level, int nparts, const uint8_t *const *part, con
     u64 pos = 32;
     u32 combined = 0;
     for (int i = 0; i < nparts; i++) {
-        for (u32 k = 0; k < part_ncrc[i]; k++) combined = stream_crc_step(combined, part_crcs[i][k]);
+        for (u32 k = 0; k < part_ncrc[i]; k++) combined = bz_crc_step(combined, part_crcs[i][k]);
         u64 nb = part_bits[i];
         size_t nbytes = (size_t)((nb + 7) / 8);
         int sh = (int)(pos & 7);

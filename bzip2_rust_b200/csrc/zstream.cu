@@ -57,8 +57,6 @@ struct bz2b200_zstream {
 
 namespace {
 
-inline u32 crc_step(u32 s, u32 b) { return ((s << 1) | (s >> 31)) ^ b; }   // crc.rs:25-27
-
 int emit(bz2b200_zstream *z, const u8 *p, size_t n) {
     if (n == 0) return BZ2B200_OK;
     z->total_out += n;
@@ -108,7 +106,7 @@ int process(bz2b200_zstream *z, int slot, size_t len, bool eof) {
         for (u32 k = 0; k < nb; k++) {
             if (hbits[k] == ~0ull) { z->err = "huffman: packed block exceeds its slot"; return BZ2B200_E_CAP; }
             hoff[k] = pos; pos += hbits[k]; maxbits = std::max(maxbits, hbits[k]);
-            z->combined = crc_step(z->combined, hcrc[k]);       // bitwriter.rs:89-91
+            z->combined = bz_crc_step(z->combined, hcrc[k]);    // bitwriter.rs:89-91
         }
         const size_t nbytes = (size_t)((pos + 7) / 8);
         BZ_CHECK(z->d_out.ensure(nbytes + 64));
