@@ -47,6 +47,7 @@ EXPORTS = [
     "bz2b200_multi_context", "bz2b200_compress_stream_multi", "bz2b200_decompress_stream_multi", "bz2b200_multi_stats",
     "bz2b200_zstream_open", "bz2b200_zstream_write", "bz2b200_zstream_close",
     "bz2b200_dstream_open", "bz2b200_dstream_write", "bz2b200_dstream_close", "bz2b200_recover",
+    "bz2b200_rstream_open", "bz2b200_rstream_write", "bz2b200_rstream_close",
 ]
 
 
@@ -69,6 +70,9 @@ class RecEntry(C.Structure):
     def __repr__(self):
         return "RecEntry(bit=%d, end_bit=%d, out_off=%d, out_len=%d, crc=%#010x, status=%d, flags=%d)" % (
             self.bit, self.end_bit, self.out_off, self.out_len, self.crc, self.status, self.flags)
+
+
+REC_REPORT = C.CFUNCTYPE(C.c_int, C.c_void_p, C.POINTER(RecEntry), C.c_uint32)   # bz2b200_rec_report
 
 
 def load_library():
@@ -144,6 +148,9 @@ def load_library():
     L.bz2b200_dstream_close.argtypes = [vp, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]
     L.bz2b200_recover.argtypes = [vp, u8p, C.c_size_t, SINK, vp, C.POINTER(RecEntry), C.c_uint32,
                                   C.POINTER(C.c_uint32), C.POINTER(C.c_uint64)]
+    L.bz2b200_rstream_open.argtypes = [vp, SINK, REC_REPORT, vp, C.POINTER(vp)]
+    L.bz2b200_rstream_write.argtypes = [vp, u8p, C.c_size_t]
+    L.bz2b200_rstream_close.argtypes = [vp, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]
     _lib = L
     return L
 
@@ -555,6 +562,80 @@ class DStream:
         rc = self._L.bz2b200_dstream_close(self._h, C.byref(ti), C.byref(to))
         self._h = None
         self.total_in, self.total_out = ti.value, to.value
+        if self._err is not None or rc != OK:
+            self._raise(rc)
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+        return False
+
+
+class RStream:
+    """Streaming block recovery (bz2b200_rstream_*): write() a possibly damaged .bz2 input in pieces; the bytes of its
+    intact blocks go to `out.write` (out=None: report only, nothing is downloaded), its entries (RecEntry, as
+    Engine.recover lists them) to `on_entries(list)` or, when that is None, to `.entries`.  Both callbacks run on one
+    library thread, in input order; a batch's entries come after its bytes.  close() sets total_in, total_out and nent.
+
+        with RStream(engine, fileobj) as r:
+            for piece in pieces: r.write(piece)
+        r.entries
+    """
+
+    def __init__(self, engine, out=None, on_entries=None):
+        self._L = engine._L
+        self._eng = engine
+        self._err = None
+        self._h = None
+        self.entries = []
+        self.total_in = self.total_out = self.nent = 0
+        self._cb = SINK()                   # a NULL sink: report only
+        if out is not None:
+            def sink(_user, data, n):
+                try:
+                    out.write(C.string_at(data, n))
+                    return 0
+                except BaseException as e:  # an exception must not unwind through the C library
+                    self._err = self._err or e
+                    return 1
+            self._cb = SINK(sink)           # keep the callback objects alive as long as the stream
+        take = on_entries if on_entries is not None else self.entries.extend
+
+        def report(_user, p, n):
+            try:
+                arr = (RecEntry * n).from_buffer_copy(C.string_at(p, n * C.sizeof(RecEntry)))
+                take(list(arr))
+                return 0
+            except BaseException as e:
+                self._err = self._err or e
+                return 1
+        self._rep = REC_REPORT(report)
+        h = C.c_void_p()
+        rc = self._L.bz2b200_rstream_open(engine._h, self._cb, self._rep, None, C.byref(h))
+        if rc != OK:
+            raise Bz2B200Error(rc, "bz2b200_rstream_open")
+        self._h = h
+
+    def _raise(self, rc):
+        if self._err is not None:
+            raise self._err
+        raise Bz2B200Error(rc, self._L.bz2b200_last_error(self._eng._h).decode())
+
+    def write(self, data):
+        a = _np_u8(data)
+        rc = self._L.bz2b200_rstream_write(self._h, a.ctypes.data, a.size)
+        if rc != OK:
+            self._raise(rc)
+
+    def close(self):
+        if self._h is None:
+            return
+        ti, to, ne = C.c_uint64(), C.c_uint64(), C.c_uint64()
+        rc = self._L.bz2b200_rstream_close(self._h, C.byref(ti), C.byref(to), C.byref(ne))
+        self._h = None
+        self.total_in, self.total_out, self.nent = ti.value, to.value, ne.value
         if self._err is not None or rc != OK:
             self._raise(rc)
 

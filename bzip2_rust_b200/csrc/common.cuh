@@ -154,11 +154,11 @@ struct bz2b200_ctx {
     DevBuf d_len6, d_rfreq, d_sel, d_gbits, d_hdr, d_bitoff, d_out, d_outbits, d_hmisc;
     // ---- stream / rle1 / decode ----
     DevBuf d_in, d_runflag, d_misc, d_stream, d_dec1, d_dec2, d_dec3;
-    // ---- dstream (dstream.cu): window, batch outputs, staging and output pieces, kept for the next stream ----
+    // ---- dstream and rstream (pump.cuh): window, batch outputs, staging and output pieces, kept for the next stream ----
     DevBuf d_dwin, d_ddec[2];
     PinBuf h_dstage[2], h_dpiece[2];
     cudaEvent_t ev_dpiece[2] = {nullptr, nullptr};
-    bool dstream_open = false;       // one dstream at a time uses them
+    bool pump_open = false;          // one dstream or rstream at a time uses them
     // ---- recovery (recover.cu): page-locked pieces of intact bytes on their way to the sink ----
     PinBuf h_rec[2];
     cudaEvent_t ev_rec[2] = {nullptr, nullptr};

@@ -283,6 +283,38 @@ typedef struct {
 int bz2b200_recover(bz2b200_ctx *ctx, const uint8_t *in, size_t n, bz2b200_sink sink, void *user,
                     bz2b200_rec_entry *ent, uint32_t ent_cap, uint32_t *nent, uint64_t *total_out);
 
+/* ---- streaming block recovery: a damaged .bz2 input of any size, in pieces, in bounded memory ---------------------- */
+/* bz2b200_recover on an input that arrives in pieces, through the dstream's machinery: bz2b200_rstream_write copies the
+ * caller's bytes into page-locked staging; a worker thread judges the candidates of each window (64 MiB, or
+ * BZ2B200_RSTREAM_WINDOW bytes: at least 1024, at most 1 GiB) that start before its last 4 MiB, carrying those 4 MiB and
+ * the recovery state (where the last intact block ends, a pending lost-magic bit, the running stream fold) to the next
+ * window; a delivery thread downloads the intact bytes in pieces of 32 MiB, hands them to `sink`, then hands the batch's
+ * entries to `report`.
+ *   Result: for any input bz2b200_recover accepts (1 <= n <= its bound), written in any piece sizes and at any window
+ *   size, `report` receives the same entries bz2b200_recover lists (count, order, bit, end_bit, out_off, out_len, crc,
+ *   status, flags), `sink` the same bytes and *total_out is the same.  Larger inputs follow the same rules with 64-bit
+ *   offsets; there is no size limit.  *nent = the number of entries reported.
+ *   Threads and order: `sink` and `report` run on one library thread, never on the caller's thread and never at the
+ *   same time.  Entries are reported in input order, each once, after the sink has received the bytes of their batch:
+ *   when entry e is reported, its bytes [out_off, out_off + out_len) have been delivered.  sink == NULL is report-only
+ *   (nothing is downloaded); report may be NULL too.
+ *   Errors are sticky, as in the dstream: the next write or the close returns them.  A non-zero return from `sink` or
+ *   `report`, and a close with no bytes written, give BZ2B200_E_ARG.  Otherwise the only errors are BZ2B200_E_CUDA and
+ *   BZ2B200_E_NOMEM, however much damage the input holds: there is no E_CAP and no E_FORMAT.
+ *   bz2b200_rstream_close judges what is left, waits for the sink and the report to finish and frees the stream (also
+ *   after an error); on an error bz2b200_last_error(ctx) says "rstream: ...".
+ * Memory: the rstream uses the dstream's staging buffers, window, batch outputs and output pieces (host memory about
+ * 200 MB; device memory one window and its candidates, the decode workspaces of one batch and two batch outputs),
+ * whatever the input size.  A context has one dstream or one rstream open at a time (a second open returns E_ARG), and
+ * must not be used by other threads while it is open (calls are serialised, so they would only wait). */
+typedef struct bz2b200_rstream bz2b200_rstream;
+/* entries in input order, each reported once, when final; non-zero aborts */
+typedef int (*bz2b200_rec_report)(void *user, const bz2b200_rec_entry *ent, uint32_t n);
+int bz2b200_rstream_open(bz2b200_ctx *ctx, bz2b200_sink sink, bz2b200_rec_report report, void *user,
+                         bz2b200_rstream **out);
+int bz2b200_rstream_write(bz2b200_rstream *r, const uint8_t *data, size_t n);
+int bz2b200_rstream_close(bz2b200_rstream *r, uint64_t *total_in, uint64_t *total_out, uint64_t *nent);
+
 /* ---- measurement hooks ------------------------------------------------------------------- */
 /* Per-stage device time (ms, CUDA events on the context's stream) of the last compress call:
  * [0]=rle1+crc+split [1]=bwt [2]=mtf/rle2 [3]=huffman select+lengths [4]=bit pack [5]=total.

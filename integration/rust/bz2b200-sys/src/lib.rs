@@ -7,6 +7,7 @@ use std::os::raw::{c_char, c_int, c_void};
 #[repr(C)] pub struct bz2b200_mctx { _private: [u8; 0] }
 #[repr(C)] pub struct bz2b200_zstream { _private: [u8; 0] }
 #[repr(C)] pub struct bz2b200_dstream { _private: [u8; 0] }
+#[repr(C)] pub struct bz2b200_rstream { _private: [u8; 0] }
 pub type bz2b200_sink = Option<unsafe extern "C" fn(user: *mut c_void, data: *const u8, n: usize) -> c_int>;
 
 pub const BZ2B200_OK: c_int = 0;
@@ -34,6 +35,8 @@ pub struct bz2b200_rec_entry {
     pub status: i32,
     pub flags: u32,
 }
+/// Receives `n` entries of a streaming recovery, in input order, after the sink has their bytes; non-zero aborts.
+pub type bz2b200_rec_report = Option<unsafe extern "C" fn(user: *mut c_void, ent: *const bz2b200_rec_entry, n: u32) -> c_int>;
 
 extern "C" {
     // ---- context ----
@@ -112,6 +115,12 @@ extern "C" {
     // ---- block recovery: every intact block of a damaged input to a sink (None: report only) ----
     pub fn bz2b200_recover(ctx: *mut bz2b200_ctx, input: *const u8, n: usize, sink: bz2b200_sink, user: *mut c_void,
         ent: *mut bz2b200_rec_entry, ent_cap: u32, nent: *mut u32, total_out: *mut u64) -> c_int;
+    // ---- streaming block recovery: any input size, in pieces; entries to `report` after their bytes to `sink` ----
+    pub fn bz2b200_rstream_open(ctx: *mut bz2b200_ctx, sink: bz2b200_sink, report: bz2b200_rec_report,
+        user: *mut c_void, out: *mut *mut bz2b200_rstream) -> c_int;
+    pub fn bz2b200_rstream_write(r: *mut bz2b200_rstream, data: *const u8, n: usize) -> c_int;
+    pub fn bz2b200_rstream_close(r: *mut bz2b200_rstream, total_in: *mut u64, total_out: *mut u64,
+        nent: *mut u64) -> c_int;
     // ---- measurement hooks ----
     pub fn bz2b200_set_timing(ctx: *mut bz2b200_ctx, on: c_int);
     pub fn bz2b200_get_timing(ctx: *const bz2b200_ctx, ms: *mut f32) -> c_int;

@@ -1,6 +1,7 @@
 """Decode rate of the stream bench.py compresses in its `e2e` leg, so that compress and decompress rates compare.
 
     python tools/bench_decode.py --gpus 1 2 4 8 [--steps K] [--warmup W] [--size-mb 100] [--dstream] [--recover]
+                                 [--rstream]
 
 Workload for world N: corpus.text(size_mb * 10^6, seed 2 + r) for r < N, concatenated, compressed at -9.  Pinned host
 buffers; W warm-up calls, then K calls timed with a host clock around each call (a call returns when its output is in
@@ -23,6 +24,12 @@ compared with the input minus the input slices of the damaged blocks (Engine.str
 totals with the expected sizes.  When bzip2recover and bzip2 are installed, one more line times the CPU way on the damaged
 copy: bzip2recover, then bzip2 -dc of every piece, one after the other ("cpu_bzip2recover"); otherwise that line says
 "not measured".
+
+--rstream adds three bz2b200_rstream arms for world 1, timed in turn with "recover_report" and "recover_sink" (added
+too when --recover is not given) on the same bytes: "rstream_report" (NULL sink), "rstream_sink" (the dstream arm's
+pinned memmove sink) and "rstream_damaged" (that sink, on the damaged copy of --recover).  Each writes the pinned stream
+in pieces of 16 MiB and is timed with a host clock from open to close; its report callback counts the entries, which
+must match the count close returns.  Outputs and totals are verified as in the recovery arms.
 """
 import argparse
 import ctypes as C
@@ -72,8 +79,11 @@ def run(world, args, eng, info):
     arms = []
     if world == 1 and args.dstream:
         arms = dstream_arms(eng, h_in, len(s), data.size)
-    if world == 1 and args.recover:
-        arms += recover_arms(eng, h_in, len(s), data)
+    if world == 1 and (args.recover or args.rstream):
+        rarms = recover_arms(eng, h_in, len(s), data)
+        arms += rarms if args.recover else rarms[:2]
+        if args.rstream:
+            arms += rstream_arms(eng, h_in, len(s), data, rarms[-1])
     if world == 1:
         L, ln = eng._L, C.c_size_t()
 
@@ -120,12 +130,12 @@ def run(world, args, eng, info):
              "ms_per_call": ms, "ms_min": 1e3 * min(arm["times"]), "ms_max": 1e3 * max(arm["times"]), "steps": args.steps,
              "piece_bytes": PIECE, "compressed_bytes": len(s), "decompressed_bytes": int(data.size),
              "verified": bool(a_ok), "library": rec["library"]}
-        r.update({k: arm[k] for k in ("damaged_blocks", "blocks") if k in arm})
+        r.update({k: arm[k] for k in ("damaged_blocks", "blocks", "window_bytes") if k in arm})
         r.update(info)
         print(json.dumps(r), flush=True)
         ok = ok and a_ok
     if world == 1 and args.recover:
-        print(json.dumps(cpu_recover_reference(arms[-1]["input"], info)), flush=True)
+        print(json.dumps(cpu_recover_reference(rarms[-1]["input"], info)), flush=True)
     return ok
 
 
@@ -220,6 +230,63 @@ def recover_arms(eng, h_in, n_in, data):
     return [arm("recover_report", h_in, data, False), arm("recover_sink", h_in, data, True), dmg_report, damaged]
 
 
+def memmove_sink(n):
+    """A pinned output buffer of n bytes and a sink that memmoves into it at a running offset: (out, cb, pos)."""
+    out = pinned(n)
+    out_ptr, pos = out.ctypes.data, [0]
+
+    def put(_user, p, k):
+        if pos[0] + k > out.size:
+            return 1
+        C.memmove(out_ptr + pos[0], p, k)
+        pos[0] += k
+        return 0
+    return out, bz.SINK(put), pos
+
+
+def rstream_arms(eng, h_in, n_in, data, damaged):
+    """The streaming recovery arms (see the module doc), like recover_arms'."""
+    L = eng._L
+    h_dmg = pinned(n_in)
+    h_dmg[:n_in] = np.frombuffer(damaged["input"], dtype=np.uint8)
+
+    def arm(metric, buf, want, sink):
+        a = {"metric": metric, "times": [], "out": None, "n": 0, "want": want,
+             "window_bytes": int(os.environ.get("BZ2B200_RSTREAM_WINDOW", 64 << 20))}
+        cb, pos, counted = bz.SINK(), [0], [0]
+        if sink:
+            out, cb, pos = memmove_sink(want.size + 64)
+            a["out"] = out
+
+        def rep(_user, _p, k):
+            counted[0] += k
+            return 0
+        rcb = bz.REC_REPORT(rep)
+        a["cbs"] = (cb, rcb)                                # alive as long as the arm
+
+        def call():
+            pos[0] = counted[0] = 0
+            h, ti, to, ne = C.c_void_p(), C.c_uint64(), C.c_uint64(), C.c_uint64()
+            rc = L.bz2b200_rstream_open(eng._h, cb, rcb, None, C.byref(h))
+            if rc == bz.OK:
+                for off in range(0, n_in, PIECE):
+                    rc = L.bz2b200_rstream_write(h, buf.ctypes.data + off, min(PIECE, n_in - off))
+                    if rc != bz.OK:
+                        break
+                rc2 = L.bz2b200_rstream_close(h, C.byref(ti), C.byref(to), C.byref(ne))
+                rc = rc if rc != bz.OK else rc2
+            if rc != bz.OK:
+                raise bz.Bz2B200Error(rc, L.bz2b200_last_error(eng._h).decode())
+            if ne.value != counted[0] or ti.value != n_in:
+                return -1                                   # fails verification
+            return to.value
+        a["call"] = call
+        return a
+    dmg = arm("rstream_damaged", h_dmg, damaged["want"], True)
+    dmg.update(damaged_blocks=damaged["damaged_blocks"], blocks=damaged["blocks"])
+    return [arm("rstream_report", h_in, data, False), arm("rstream_sink", h_in, data, True), dmg]
+
+
 def cpu_recover_reference(damaged, info):
     """bzip2recover + bzip2 -dc of each piece on the damaged copy, timed once with a host clock (the CPU reference)."""
     import shutil
@@ -252,6 +319,7 @@ def main():
     ap.add_argument("--size-mb", type=int, default=100)
     ap.add_argument("--dstream", action="store_true", help="also time the streaming decoder and its test mode (world 1)")
     ap.add_argument("--recover", action="store_true", help="also time block recovery, intact and damaged (world 1)")
+    ap.add_argument("--rstream", action="store_true", help="also time streaming recovery against block recovery (world 1)")
     args = ap.parse_args()
     if args.steps < 1 or min(args.gpus) < 1:
         ap.error("--steps and --gpus must be at least 1")

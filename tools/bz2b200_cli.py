@@ -19,11 +19,11 @@ input bit range and the output offset where the lost bytes would have been; it e
 2 otherwise.
 """
 import argparse
-import mmap
 import os
 import sys
 
 GAP_BITS = 80 + 7 + 32          # a footer, its padding and the next stream's header lie between two streams' blocks
+PIECE = 16 << 20
 
 
 def recover(bz, eng, name, a):
@@ -33,34 +33,26 @@ def recover(bz, eng, name, a):
     if not to_stdout and os.path.exists(oname) and not a.force:
         sys.stderr.write("bz2b200: output file %s already exists (use -f)\n" % oname)
         return 1
-    import numpy as np
-    mm = None
-    if name == "-":
-        src = sys.stdin.buffer.read()
-    else:
-        with open(name, "rb") as f:
-            if os.fstat(f.fileno()).st_size:
-                mm = mmap.mmap(f.fileno(), 0, access=mmap.ACCESS_READ)     # the input is not copied into host memory
-        src = mm
-    size = len(src) if src is not None else 0
-    if size == 0:
-        sys.stderr.write("bz2b200: %s: empty file\n" % name)
-        return 2
-    view = np.frombuffer(src, dtype=np.uint8)
-    err = None
-    dst = sys.stdout.buffer if to_stdout else open(oname, "wb")
+    # in bounded memory: the input is read in pieces while earlier pieces are judged and their intact bytes written
+    src = sys.stdin.buffer if name == "-" else open(name, "rb")
     try:
-        total, ents = eng.recover(view, dst)                       # the sink writes as blocks decode
-    except BaseException as e:
-        err = e.with_traceback(None)        # its frames would hold views of the map, which must be closed first
+        piece = src.read(PIECE)
+        if not piece:
+            sys.stderr.write("bz2b200: %s: empty file\n" % name)
+            return 2
+        dst = sys.stdout.buffer if to_stdout else open(oname, "wb")
+        try:
+            with bz.RStream(eng, dst) as r:             # the sink writes as blocks decode
+                while piece:
+                    r.write(piece)
+                    piece = src.read(PIECE)
+        finally:
+            if dst is not sys.stdout.buffer:
+                dst.close()
     finally:
-        if dst is not sys.stdout.buffer:
-            dst.close()
-    del view
-    if mm is not None:
-        mm.close()
-    if err is not None:
-        raise err
+        if src is not sys.stdin.buffer:
+            src.close()
+    size, total, ents = r.total_in, r.total_out, r.entries
     nbits = size * 8
     lines, cursor = [], 0
     for i, e in enumerate(ents):
